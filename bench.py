@@ -5,6 +5,7 @@ catalog, buyer-tower pooling, and the device-resident /retrieve path.
     python bench.py --gpus N --steps K --warmup W                     # headline: 10M x 384, nq 4096, top-100
     python bench.py --workload c3|c4|c5 ...                           # the other BASELINE configs (see WORKLOADS)
     python bench.py --impl reference --gpus N --steps K --warmup W    # the reference's CPU path (rank 0 only)
+    python bench.py ... --dump-outputs DIR                            # + the last timed step's results as DIR/*.npy
 
 A "step" is one search of a batch of `--nq` queries (c5: one /retrieve batch).  Prints ONE JSON line (rank 0).
 Catalogs (>= 768 MB of bf16 per pass) are larger than L2, so no flush is needed between iterations.  Inputs
@@ -603,6 +604,27 @@ def make_roofline(peaks, clocks, scan_avg_ms, ms_step, n_local, dp, d, nq, world
     return r
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, scores, ids):
+    """Writes what a caller of the timed path receives for one batch: scores.npy (float32 [rows, k]) and ids.npy
+    (float64, exact for any row id below 2**53).  Above DUMP_MAX_BYTES a fixed, seeded sample of query rows is
+    kept and rows.npy (float64) lists which; the inputs are seeded too, so two builds can be compared file by file."""
+    scores = scores.cpu().numpy().astype(np.float32)
+    ids = ids.cpu().numpy().astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    nq, k = scores.shape
+    keep = max(1, (DUMP_MAX_BYTES - 4096) // (k * 12 + 8))      # 4096: room for the three .npy headers
+    if nq > keep:
+        rows = np.sort(np.random.default_rng(0).choice(nq, keep, replace=False))
+        scores, ids = scores[rows], ids[rows]
+        np.save(out / "rows.npy", rows.astype(np.float64))
+    np.save(out / "scores.npy", scores)
+    np.save(out / "ids.npy", ids)
+
+
 def run_pipelined(submit, first, last, depth=2):
     """Steps first..last-1 with `depth` batches in flight: step i+depth-1 is enqueued before step i's certificate is
     looked at, so the device never idles on the host (the sharded search runs a 3-stage pipeline and wants depth 3).
@@ -671,6 +693,9 @@ def run_search(args):
     dp = int(lib.tt_flat_pitch(d))
     scan_avg_ms = float(scan_ms[:n_rec].mean()) if n_rec > 0 else None
     roofline = make_roofline(peaks, clocks, scan_avg_ms, ms_step, n_local, dp, d, nq, world, n_total)
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0], last[1])
 
     # ---- parity of the last timed batch (outside the timed region, every rank) -------------------
     parity = parity_block(searcher, sharded, index, queries[total - 1], last[0], last[1], k, world)
@@ -749,7 +774,13 @@ def main():
     ap.add_argument("--dim", type=int, default=None)
     ap.add_argument("--topk", type=int, default=None)
     ap.add_argument("--no-secondary", action="store_true", help="skip pooling / cpu baseline extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's results (scores, ids) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     wl = WORKLOADS[args.workload]
     if args.nq is None:
         args.nq = int(os.environ.get("TT_BENCH_NQ", wl["nq"]))
@@ -817,6 +848,8 @@ def run_c5(args):
     scan_ms = torch.empty(args.steps, dtype=torch.float32)
     n_rec = lib.tt_profile_scan_read(scan_ms.data_ptr(), args.steps)
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0], last[1])
     dp = int(lib.tt_flat_pitch(d))
     roofline = make_roofline(peaks, clocks, float(scan_ms[:n_rec].mean()) if n_rec > 0 else None, ms_step, n_local, dp, d,
                              batch, world, n_total)

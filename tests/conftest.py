@@ -15,8 +15,29 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with `-m gpu`)")
 
 
+def infonce_inputs(B: int, M: int, D: int, seed: int, unit: bool = True):
+    """The seeded (buyer [B,D], pos [B,D], neg [B,M,D]) f32 inputs of the infonce_*.npz golden cases."""
+    rng = np.random.default_rng(seed)
+    b = rng.standard_normal((B, D)).astype(np.float32)
+    p = rng.standard_normal((B, D)).astype(np.float32)
+    n = rng.standard_normal((B, M, D)).astype(np.float32)
+    if unit:                          # the towers L2-normalise their outputs (buyer_tower.py:66,99; item tower likewise)
+        b /= np.linalg.norm(b, axis=1, keepdims=True)
+        p /= np.linalg.norm(p, axis=1, keepdims=True)
+        n /= np.maximum(np.linalg.norm(n, axis=2, keepdims=True), 1e-12)
+    return b, p, n
+
+
 def golden(name: str):
-    return dict(np.load(GOLDEN / name, allow_pickle=False))
+    g = dict(np.load(GOLDEN / name, allow_pickle=False))
+    if "input_seed" in g:
+        # buyer and pos are not stored (that keeps the file under 1 MB): they are regenerated from the seed, and
+        # neg, drawn after them from the same generator and stored, checks that the regeneration is exact
+        B, M, D = g["neg"].shape
+        b, p, n = infonce_inputs(B, M, D, int(g["input_seed"]), bool(g["input_unit"]))
+        assert np.array_equal(n, g["neg"]), f"{name}: the seeded generator no longer reproduces the stored inputs"
+        g.update(buyer=b, pos=p)
+    return g
 
 
 @pytest.fixture(scope="session")

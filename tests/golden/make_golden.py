@@ -23,12 +23,14 @@ import torch
 ROOT = Path(__file__).resolve().parents[2]
 OUT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.path.insert(0, str(ROOT / "tests"))
 sys.path.insert(0, str(ROOT / "oracle" / "faiss_shim"))
 sys.path.insert(0, "/root/reference")
 
 from src.models.buyer_tower import BuyerTower  # noqa: E402  (the reference)
 from src.inference.vector_db import VectorDatabase  # noqa: E402  (the reference, over the shim)
 from src.training.losses import InfoNCELoss  # noqa: E402  (the reference)
+from conftest import infonce_inputs  # noqa: E402
 
 EVENT_W = np.array([1.0, 5.0, 10.0], dtype=np.float32)
 
@@ -97,23 +99,19 @@ def vdb_case(name, N, D, nq, k, seed):
     print(name, out["batch_ids"].shape)
 
 
-def infonce_case(name, B, M, D, seed, temperature=0.07, unit=True):
-    """The real InfoNCELoss (losses.py:8-79) and its autograd gradients on seeded inputs."""
-    rng = np.random.default_rng(seed)
-    b = rng.standard_normal((B, D)).astype(np.float32)
-    p = rng.standard_normal((B, D)).astype(np.float32)
-    n = rng.standard_normal((B, M, D)).astype(np.float32)
-    if unit:                          # the towers L2-normalise their outputs (buyer_tower.py:66,99; item tower likewise)
-        b /= np.linalg.norm(b, axis=1, keepdims=True)
-        p /= np.linalg.norm(p, axis=1, keepdims=True)
-        n /= np.maximum(np.linalg.norm(n, axis=2, keepdims=True), 1e-12)
+def infonce_case(name, B, M, D, seed, temperature=0.07, unit=True, store_buyer_pos=True):
+    """The real InfoNCELoss (losses.py:8-79) and its autograd gradients on seeded inputs.  store_buyer_pos=False
+    stores the seed in place of buyer and pos (tests/conftest.py:golden regenerates them) for a case that would
+    otherwise exceed 1 MB."""
+    b, p, n = infonce_inputs(B, M, D, seed, unit)
     crit = InfoNCELoss(temperature)
     tb, tp, tn = (torch.from_numpy(a).requires_grad_(True) for a in (b, p, n))
     loss = crit(tb, tp, tn)
     loss.backward()
     with torch.no_grad():
         loss64 = crit(tb.double(), tp.double(), tn.double())
-    np.savez_compressed(OUT / f"infonce_{name}.npz", buyer=b, pos=p, neg=n, temperature=np.float64(temperature),
+    inputs = dict(buyer=b, pos=p) if store_buyer_pos else dict(input_seed=np.int64(seed), input_unit=np.bool_(unit))
+    np.savez_compressed(OUT / f"infonce_{name}.npz", **inputs, neg=n, temperature=np.float64(temperature),
                         loss=np.float32(loss.item()), loss_f64=np.float64(loss64.item()), d_buyer=tb.grad.numpy(),
                         d_pos=tp.grad.numpy(), d_neg=tn.grad.numpy())
     print(f"infonce_{name}: loss {loss.item():.6f}")
@@ -121,7 +119,7 @@ def infonce_case(name, B, M, D, seed, temperature=0.07, unit=True):
 
 if __name__ == "__main__":
     infonce_case("b16_m4_d384", 16, 4, 384, 21)                 # trainer defaults: 4 sampled negatives (losses.py:36-79)
-    infonce_case("b64_m4_d384", 64, 4, 384, 22)
+    infonce_case("b64_m4_d384", 64, 4, 384, 22, store_buyer_pos=False)
     infonce_case("b5_m0_d384", 5, 0, 384, 23)                   # no sampled negatives: in-batch only
     infonce_case("b9_m3_d100_raw", 9, 3, 100, 24, temperature=0.5, unit=False)   # unnormalised, D % 32 != 0
     infonce_case("b1_m2_d64", 1, 2, 64, 25)                     # batch of one: the in-batch block is all masked

@@ -5,6 +5,8 @@ import subprocess
 import sys
 from pathlib import Path
 
+import numpy as np
+import pytest
 import torch
 
 ROOT = Path(__file__).resolve().parents[1]
@@ -35,6 +37,57 @@ def test_product_arm_needs_cuda():
         return
     r = _run("--steps", "1", "--catalog-rows", "20000", "--nq", "16")
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
+
+
+def test_bad_steps_and_dump_of_the_cpu_arm_are_refused():
+    r = _run("--impl", "reference", "--steps", "0", "--warmup", "0", "--catalog-rows", "20000", "--nq", "16")
+    assert r.returncode != 0 and "--steps" in r.stderr
+    r = _run("--impl", "reference", "--steps", "1", "--catalog-rows", "20000", "--nq", "16", "--dump-outputs", "x")
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+
+
+def test_dump_outputs_dtypes_and_bounded_sample(tmp_path, monkeypatch):
+    """scores stay float32, ids become float64 (exact below 2**53); a result above the size cap is cut to a fixed
+    seeded sample of query rows, listed in rows.npy."""
+    sys.path.insert(0, str(ROOT))
+    import bench
+    s = torch.rand(50, 7)
+    i = torch.randint(0, 1 << 40, (50, 7))
+    bench.dump_outputs(tmp_path / "full", s, i)
+    assert sorted(p.name for p in (tmp_path / "full").iterdir()) == ["ids.npy", "scores.npy"]
+    gs, gi = np.load(tmp_path / "full" / "scores.npy"), np.load(tmp_path / "full" / "ids.npy")
+    assert gs.dtype == np.float32 and gi.dtype == np.float64
+    assert np.array_equal(gs, s.numpy()) and np.array_equal(gi.astype(np.int64), i.numpy())
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 4096 + 10 * (7 * 12 + 8))
+    for name in ("a", "b"):
+        bench.dump_outputs(tmp_path / name, s, i)
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.dtype == np.float64 and len(rows) == 10 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))
+    r = rows.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "scores.npy"), s.numpy()[r])
+    assert np.array_equal(np.load(tmp_path / "a" / "ids.npy").astype(np.int64), i.numpy()[r])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_batch_and_repeats(tmp_path):
+    """--dump-outputs writes the results of the last timed step (checked against the fp32 torch checker on the same
+    seeded catalog and queries), and a second run with the same arguments writes the same bytes."""
+    args = ["--steps", "2", "--warmup", "3", "--catalog-rows", "20000", "--nq", "16", "--topk", "10", "--no-secondary"]
+    for name in ("a", "b"):
+        r = _run(*args, "--dump-outputs", str(tmp_path / name))
+        assert r.returncode == 0, r.stderr[-2000:]
+    for f in ("scores.npy", "ids.npy"):
+        assert (tmp_path / "a" / f).read_bytes() == (tmp_path / "b" / f).read_bytes(), f
+    s, i = np.load(tmp_path / "a" / "scores.npy"), np.load(tmp_path / "a" / "ids.npy")
+    assert s.dtype == np.float32 and i.dtype == np.float64 and s.shape == i.shape == (16, 10)
+    sys.path.insert(0, str(ROOT))
+    import bench
+    index, _, _ = bench.make_shard(20000, 384, 1, 0)
+    q = torch.randn((5, 16, 384), device="cuda", generator=torch.Generator(device="cuda").manual_seed(4321))[4]
+    ts, ti = bench.torch_flat_topk(index.xn, q, 10)
+    rep = bench.compare_topk_device(torch.from_numpy(s).cuda(), torch.from_numpy(i).long().cuda(), ts, ti)
+    assert rep["ok"], rep
 
 
 def test_reference_arm_under_torchrun_uses_all_threads_and_is_bounded():

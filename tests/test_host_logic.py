@@ -41,7 +41,7 @@ def test_buyer_tower_has_no_cpu_fallback():
         m(torch.zeros(2, 3, 8), torch.ones(2, 4))
 
 
-def test_vector_database_errors_match_reference():
+def test_vector_database_errors_match_reference(tmp_path):
     db = pkg.VectorDatabase(embedding_dim=16)
     assert db.index is None and db.product_ids is None and db.id_to_index is None and db.index_to_id is None
     with pytest.raises(ValueError, match="Embedding dimension mismatch: expected 16, got 8"):
@@ -51,7 +51,8 @@ def test_vector_database_errors_match_reference():
     with pytest.raises(ValueError, match="Index not built"):
         db.retrieve_batch(np.zeros((2, 16), np.float32))
     with pytest.raises(ValueError, match="Index not built"):
-        db.save_index("/tmp/nope.faiss")
+        db.save_index(str(tmp_path / "nope.faiss"))
+    assert not (tmp_path / "nope.faiss").exists()
     assert db.get_embedding("x") is None
     if not torch.cuda.is_available():
         with pytest.raises(RuntimeError, match="CUDA"):
