@@ -200,6 +200,34 @@ int tt_flat_search_exact(const float* q, int nq, const int32_t* qsel, int nsel,
                          float* scores, int64_t* ids,
                          void* workspace, size_t workspace_bytes, void* stream);
 
+/* Exclusion lists: the exact top-K over the rows a query does NOT exclude (e.g. a buyer's own history).
+ *   excl    i64 [nq, E]   row-major; excl[q, j] is an id in the result id space (row + id_offset, a global id
+ *                         on a shard).  Entries below 0 are padding, ids outside the index (or this shard) are
+ *                         ignored, duplicates are allowed: the padded history idx of the pooling calls fits as is.
+ *   E       0 <= E <= TT_FLAT_MAX_EXCLUDE; excl may be NULL only when E == 0.  E == 0 is the plain call.
+ * Results are ordered as above; with fewer than K allowed rows the tail is score -inf / id -1.  An excluded row
+ * never appears in an output.  The certificate is read over the allowed rows: "every allowed row not rescored
+ * scores below the bound"; flags, bound and the merge keep their meaning.
+ * Excluded rows are typically a query's best ones, so the scan is planned for
+ *     K_plan = min(K + E, N, TT_FLAT_MAX_K)          (N = rows of this index, N_total on the global-threshold path)
+ * while K results are emitted and the K-th ALLOWED score is certified.  tt_flat_search_excl_workspace_bytes sizes the
+ * workspace for it.  The global-threshold calls that never see the list - tt_flat_shard_plan_ok,
+ * tt_flat_shard_workspace_bytes and tt_flat_shard_sample - are called with K_plan as their K (N = N_total), and
+ * tt_flat_shard_search_excl with K.  tt_flat_search_exact_excl reads the list row of the QUERY row qsel[i] (not of
+ * the slot i); an uncertified query is re-run there with the same list. */
+#define TT_FLAT_MAX_EXCLUDE 1024
+size_t tt_flat_search_excl_workspace_bytes(int64_t N, int D, int nq, int K, int E);
+int tt_flat_search_excl(const float* q, int nq,
+                        const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
+                        int K, int64_t id_offset,
+                        float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified,
+                        const int64_t* excl, int E,
+                        void* workspace, size_t workspace_bytes, void* stream);
+int tt_flat_search_exact_excl(const float* q, int nq, const int32_t* qsel, int nsel,
+                              const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                              float* scores, int64_t* ids, const int64_t* excl, int E,
+                              void* workspace, size_t workspace_bytes, void* stream);
+
 /* Merge G per-shard sorted top-K lists into one: scores_g f32 [G, nq, K], ids_g i64 [G, nq, K]
  * (the layout an all-gather of per-rank [nq,K] results produces) -> [nq, K], same ordering
  * (score descending, id ascending). */
@@ -245,6 +273,21 @@ int tt_flat_shard_search(int nq, const float* Xn, const void* Xh, int64_t N_loca
                          int K, int64_t id_offset, const float* topr_g, int G,
                          float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
                          void* workspace, size_t workspace_bytes, void* stream);
+/* The same two shard searches with per-query exclusion lists (see tt_flat_search_excl; ids are global).  On the
+ * global-threshold path call tt_flat_shard_plan_ok / tt_flat_shard_workspace_bytes / tt_flat_shard_sample with
+ * K_plan = min(K + E, N_total, TT_FLAT_MAX_K) and tt_flat_shard_search_excl with K.  A shard whose allowed rows
+ * are fewer than K pads its record with -inf / -1; its bound keeps its meaning over the allowed rows. */
+int tt_flat_search_shard_excl(const float* q, int nq,
+                              const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
+                              int K, int64_t id_offset,
+                              float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
+                              const int64_t* excl, int E,
+                              void* workspace, size_t workspace_bytes, void* stream);
+int tt_flat_shard_search_excl(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total, int D,
+                              int K, int64_t id_offset, const float* topr_g, int G,
+                              float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
+                              const int64_t* excl, int E,
+                              void* workspace, size_t workspace_bytes, void* stream);
 int tt_shard_merge(const void* gathered, size_t rank_stride, size_t off_scores, size_t off_ids,
                    size_t off_bound, size_t off_flags, int G, int nq, int K,
                    float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, void* stream);

@@ -16,7 +16,14 @@ LIB_PATH = _HERE / "lib" / "libtt_b200.so"
 
 TT_FLAT_MAX_K = 2048
 TT_SHARD_TOPR = 32
+TT_FLAT_MAX_EXCLUDE = 1024
 ABI_VERSION = 1
+
+
+def plan_k(k: int, n_excl: int, n: int) -> int:
+    """K_plan = min(K + E, N, TT_FLAT_MAX_K): the K a search with E exclusions per query plans its scan for
+    (include/tt_b200.h); the global-threshold calls of a sharded search take it with N = N_total."""
+    return min(int(k) + int(n_excl), int(n), TT_FLAT_MAX_K)
 
 # name -> (restype, argtypes); mirrors include/tt_b200.h one to one
 SIGNATURES = {
@@ -45,7 +52,18 @@ SIGNATURES = {
                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "tt_flat_search_shard": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
-    "tt_flat_shard_plan_ok": (c_int, [c_int64, c_int64, c_int, c_int, c_int]),
+    "tt_flat_search_excl_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int, c_int]),
+    "tt_flat_search_excl": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64,
+                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_search_shard_excl": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                          c_size_t, c_void_p]),
+    "tt_flat_shard_search_excl": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64, c_void_p,
+                                          c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                          c_void_p, c_size_t, c_void_p]),
+    "tt_flat_search_exact_excl": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int64,
+                                          c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_shard_plan_ok":(c_int, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_sample": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p,
                                      c_void_p, c_size_t, c_void_p]),

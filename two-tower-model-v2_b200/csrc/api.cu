@@ -1,6 +1,7 @@
 // C-ABI glue: error reporting and the tt_flat_search orchestration (include/tt_b200.h).
 #include "tt_common.cuh"
 #include "flat_internal.cuh"
+#include <algorithm>
 #include <atomic>
 #include <vector>
 
@@ -81,10 +82,24 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_workspac
   return search_ws_layout(pl, D, nq).total;
 }
 
+// The K a search with E exclusions per query plans its scan for: the excluded rows are typically the query's best
+// ones, so the candidate budget must cover them (include/tt_b200.h).
+static int plan_k(int64_t N, int K, int E) {
+  const int64_t k = (int64_t)K + (E > 0 ? E : 0);
+  return (int)std::min<int64_t>(std::min<int64_t>(k, N), TT_FLAT_MAX_K);
+}
+
+extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_excl_workspace_bytes(int64_t N, int D, int nq, int K, int E) {
+  if (E < 0 || E > TT_FLAT_MAX_EXCLUDE || N < 1 || K < 1) return 0;
+  return tt_flat_search_workspace_bytes(N, D, nq, plan_k(N, K, E));
+}
+
 static int flat_search_impl(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
                             int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
-                            int32_t* flags, int32_t* n_uncertified, float* bound, void* workspace,
-                            size_t workspace_bytes, void* stream) {
+                            int32_t* flags, int32_t* n_uncertified, float* bound, const int64_t* excl, int E,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
+  TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   TT_CHECK_ARG(q && Xn && Xh && stats && scores && ids && flags && n_uncertified, "null pointer");
   TT_CHECK_ARG(nq >= 0, "nq < 0");
   TT_CHECK_ARG(N >= 1 && N < (1LL << 31), "need 1 <= N < 2^31 rows per shard");
@@ -94,7 +109,7 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
   cudaStream_t st = (cudaStream_t)stream;
   if (nq == 0) { TT_CHECK_CUDA(cudaMemsetAsync(n_uncertified, 0, sizeof(int32_t), st)); return TT_OK; }
 
-  const ScanPlan pl = make_scan_plan(N, D, nq, K);
+  const ScanPlan pl = make_scan_plan(N, D, nq, plan_k(N, K, E));
   TT_CHECK_ARG(workspace != nullptr, "null workspace");
   TT_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "workspace must be 256-byte aligned");
   if (pl.route_exact || !pl.supported) {
@@ -107,8 +122,8 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
       fill_int_kernel<<<(nq + 255) / 256, 256, 0, st>>>(reinterpret_cast<int*>(bound), nq, (int)0xff800000);
       TT_CHECK_LAUNCH();
     }
-    return tt_flat_search_exact(q, nq, nullptr, nq, Xn, N, D, K, id_offset, scores, ids, workspace,
-                                workspace_bytes, stream);
+    return tt_flat_search_exact_excl(q, nq, nullptr, nq, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
+                                     workspace_bytes, stream);
   }
   const SearchWs w = search_ws_layout(pl, D, nq);
   if (workspace_bytes < w.total) { set_error("tt_flat_search: workspace too small"); return TT_ERR_WORKSPACE; }
@@ -125,7 +140,8 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
   if (int e = launch_prep_queries(q, nq, pl.nq_pad, D, pl.Dp, stats, qn, qh, eps, n_uncertified, st)) return e;
   if (int e = launch_scan(pl, qh, Xh, N, nq, thr, cnt, cand, sample, st)) return e;
   return launch_finalize(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, cnt, cand, scores,
-                         reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st);
+                         reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st,
+                         reinterpret_cast<const long long*>(excl), E);
 }
 
 extern "C" __attribute__((visibility("default"))) int tt_flat_search(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
@@ -133,7 +149,15 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search(const float
                               int32_t* flags, int32_t* n_uncertified, void* workspace, size_t workspace_bytes,
                               void* stream) {
   return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
-                          workspace, workspace_bytes, stream);
+                          nullptr, 0, workspace, workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_excl(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
+                                   int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
+                                   int32_t* flags, int32_t* n_uncertified, const int64_t* excl, int E,
+                                   void* workspace, size_t workspace_bytes, void* stream) {
+  return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
+                          excl, E, workspace, workspace_bytes, stream);
 }
 
 extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
@@ -142,7 +166,16 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard(const
                               size_t workspace_bytes, void* stream) {
   TT_CHECK_ARG(bound != nullptr, "null bound");
   return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, bound,
-                          workspace, workspace_bytes, stream);
+                          nullptr, 0, workspace, workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard_excl(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
+                                         int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
+                                         int32_t* flags, int32_t* n_uncertified, float* bound, const int64_t* excl,
+                                         int E, void* workspace, size_t workspace_bytes, void* stream) {
+  TT_CHECK_ARG(bound != nullptr, "null bound");
+  return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, bound,
+                          excl, E, workspace, workspace_bytes, stream);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -179,15 +212,18 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_shard_sample(const
   return launch_sample(pl, ws + w.qh, Xh, N_local, nq, nullptr, topr, reinterpret_cast<float*>(ws + w.sample), st);
 }
 
-extern "C" __attribute__((visibility("default"))) int tt_flat_shard_search(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total, int D,
-                                    int K, int64_t id_offset, const float* topr_g, int G, float* scores, int64_t* ids,
-                                    int32_t* flags, int32_t* n_uncertified, float* bound, void* workspace,
-                                    size_t workspace_bytes, void* stream) {
+static int flat_shard_search_impl(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total, int D,
+                                  int K, int64_t id_offset, const float* topr_g, int G, float* scores, int64_t* ids,
+                                  int32_t* flags, int32_t* n_uncertified, float* bound, const int64_t* excl, int E,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
+  TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
+  TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   TT_CHECK_ARG(Xn && Xh && topr_g && scores && ids && flags && n_uncertified && bound && workspace, "null pointer");
   TT_CHECK_ARG(nq >= 1 && G >= 1 && G <= 64 && N_local >= 1 && N_local < (1LL << 31) && N_total >= N_local, "bad sizes");
   TT_CHECK_ARG(K >= 1 && K <= N_local && K <= TT_FLAT_MAX_K, "need 1 <= K <= min(N_local, TT_FLAT_MAX_K)");
   bool ok = false;
-  const ScanPlan pl = make_shard_plan(N_local, N_total, D, nq, K, &ok);
+  // the sample pass and the plan checks were called with K_plan = min(K + E, N_total, TT_FLAT_MAX_K)
+  const ScanPlan pl = make_shard_plan(N_local, N_total, D, nq, plan_k(N_total, K, E), &ok);
   if (!ok) { set_error("tt_flat_shard_search: no global-threshold plan for these sizes"); return TT_ERR_UNSUPPORTED; }
   const SearchWs w = search_ws_layout(pl, D, nq);
   if (workspace_bytes < w.total) { set_error("tt_flat_shard_search: workspace too small"); return TT_ERR_WORKSPACE; }
@@ -200,7 +236,25 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_shard_search(int n
   if (int e = launch_select_gathered(topr_g, G, nq, pl.sample_rank, thr, n_uncertified, st)) return e;
   if (int e = launch_main_scan(pl, ws + w.qh, Xh, N_local, nq, thr, cnt, ws + w.cand, st)) return e;
   return launch_finalize(pl, qn, Xn, N_local, D, nq, K, id_offset, thr, eps, cnt, ws + w.cand, scores,
-                         reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st);
+                         reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st,
+                         reinterpret_cast<const long long*>(excl), E);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_shard_search(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total, int D,
+                                    int K, int64_t id_offset, const float* topr_g, int G, float* scores, int64_t* ids,
+                                    int32_t* flags, int32_t* n_uncertified, float* bound, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  return flat_shard_search_impl(nq, Xn, Xh, N_local, N_total, D, K, id_offset, topr_g, G, scores, ids, flags,
+                                n_uncertified, bound, nullptr, 0, workspace, workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_shard_search_excl(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total,
+                                         int D, int K, int64_t id_offset, const float* topr_g, int G, float* scores,
+                                         int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
+                                         const int64_t* excl, int E, void* workspace, size_t workspace_bytes,
+                                         void* stream) {
+  return flat_shard_search_impl(nq, Xn, Xh, N_local, N_total, D, K, id_offset, topr_g, G, scores, ids, flags,
+                                n_uncertified, bound, excl, E, workspace, workspace_bytes, stream);
 }
 
 // ------------------------------------------------------------------------------------------

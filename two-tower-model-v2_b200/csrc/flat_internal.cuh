@@ -48,11 +48,11 @@ int launch_select_gathered(const float* topr_g, int G, int nq, int r, float* thr
 int launch_main_scan(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr,
                      unsigned int* seg_cnt, void* cand, cudaStream_t st, const float* sel_sample = nullptr);
 
-// fp32 rescoring of every candidate, exact sort, certificate
+// fp32 rescoring of every candidate, exact sort, certificate; excl i64 [nq, E] (E > 0) drops the listed rows
 int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,
                     long long id_offset, const float* thr, const float* eps, const unsigned int* seg_cnt,
                     const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
-                    float* bound_out, cudaStream_t st);
+                    float* bound_out, cudaStream_t st, const long long* excl = nullptr, int E = 0);
 
 // shared TMA descriptor helper (flat_scan.cu) and the tensor-core attention-logits launcher (attn_logits_tc.cu)
 int make_tmap_f32(void* tensor_map /* CUtensorMap* */, const void* base, long long rows, int cols, int box_rows, int box_cols);

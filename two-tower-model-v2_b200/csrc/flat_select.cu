@@ -11,14 +11,15 @@
 
 namespace tt {
 
-// In-place bitonic sort of P (power of two) 64-bit keys in shared memory, descending.
-__device__ __forceinline__ void bitonic_sort_desc(unsigned long long* key, int P) {
+// In-place bitonic sort of P (power of two) keys in shared memory, descending.
+template <typename T>
+__device__ __forceinline__ void bitonic_sort_desc(T* key, int P) {
   for (int k = 2; k <= P; k <<= 1) {
     for (int j = k >> 1; j > 0; j >>= 1) {
       for (int i = threadIdx.x; i < P; i += blockDim.x) {
         const int ixj = i ^ j;
         if (ixj > i) {
-          const unsigned long long a = key[i], b = key[ixj];
+          const T a = key[i], b = key[ixj];
           const bool up = (i & k) == 0;          // "up" blocks are sorted descending
           if (up ? (a < b) : (a > b)) { key[i] = b; key[ixj] = a; }
         }
@@ -53,6 +54,58 @@ __device__ __forceinline__ float warp_dot(const float* __restrict__ qs, const fl
 }
 
 // ------------------------------------------------------------------------------------------
+// Per-query exclusion lists (tt_flat_search_excl & co.): excl i64 [nq, E], entry = local row + id_offset; entries
+// below 0 are padding, ids outside [id_offset, id_offset + N) are ignored, duplicates are harmless.  A CTA stages
+// its query's list in shared memory as local rows sorted descending; EXCL_NONE fills the unused slots (rows are
+// < 2^31, so it never matches one).  Membership is then a binary search.
+constexpr unsigned int EXCL_NONE = 0xffffffffu;
+
+// ex[j] for j < P (P = next_pow2(E)); returns true if the query excludes a row of this shard.  No barrier.
+__device__ __forceinline__ bool stage_exclusions(const long long* __restrict__ excl, int E, int q, long long id_offset,
+                                                 long long N, unsigned int* ex, int P) {
+  bool any = false;
+  for (int j = threadIdx.x; j < P; j += blockDim.x) {
+    unsigned int v = EXCL_NONE;
+    if (j < E) {
+      const long long id = excl[(long long)q * E + j];
+      const long long r = id - id_offset;
+      if (id >= 0 && r >= 0 && r < N) { v = (unsigned int)r; any = true; }
+    }
+    ex[j] = v;
+  }
+  return any;
+}
+
+__device__ __forceinline__ bool is_excluded(const unsigned int* ex, int P, unsigned int row) {
+  int lo = 0, hi = P;   // first position whose entry is <= row (the list is descending)
+  while (lo < hi) { const int mid = (lo + hi) >> 1; if (ex[mid] > row) lo = mid + 1; else hi = mid; }
+  return lo < P && ex[lo] == row;
+}
+
+// In-place, order-keeping compaction of key[0, n) to the keys `keep(key)` accepts; returns the new count.  Chunks of
+// NT keys move left only, so a chunk never overwrites keys not yet read.  n must be the same in every thread.
+template <int NT, typename Keep>
+__device__ __forceinline__ int compact_keys(unsigned long long* key, int n, int* s_wsum, Keep keep_fn) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int out = 0;
+  for (int base = 0; base < n; base += NT) {
+    const int i = base + (int)threadIdx.x;
+    const unsigned long long kk64 = (i < n) ? key[i] : 0ull;
+    const bool keep = (i < n) && keep_fn(kk64);
+    const unsigned int bal = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) s_wsum[warp] = __popc(bal);
+    __syncthreads();                       // also orders every read of this chunk before the writes below
+    int wbase = 0, tot = 0;
+#pragma unroll
+    for (int w = 0; w < NT / 32; ++w) { const int c = s_wsum[w]; if (w < warp) wbase += c; tot += c; }
+    if (keep) key[out + wbase + __popc(bal & ((1u << lane) - 1u))] = kk64;
+    out += tot;
+    __syncthreads();
+  }
+  return out;
+}
+
+// ------------------------------------------------------------------------------------------
 // finalize: one CTA per query.
 //   1. gather the query's per-slice candidate segments (bf16 tensor-core score, row);
 //   2. b_K = K-th largest bf16 score by a 4-pass radix select (no sort of the over-fetched list);
@@ -63,36 +116,43 @@ __device__ __forceinline__ float warp_dot(const float* __restrict__ qs, const fl
 //      c = max(scan threshold, cutoff), hence an fp32 score below c + eps.  If the K-th best rescored
 //      fp32 score f_K >= c + eps, no such row can enter the top-K: the result is exact.  Otherwise the
 //      query is flagged and the host re-runs it through the exact path.
+// EXCL (exclusion lists): right after the gather, candidates whose row the query excludes are dropped, so n, b_K,
+// the cutoff and m all count allowed rows only, and the certificate reads "every ALLOWED row not rescored has a
+// bf16 score < c".  Excluded rows are typically a query's best ones: the caller plans the scan for
+// K_plan = min(K + E, N, TT_FLAT_MAX_K) so that the candidate budget covers them.
 constexpr int FIN_THREADS = 256;          // large batches: one 256-thread CTA per query, several CTAs per SM
 constexpr int FIN_THREADS_WIDE = 1024;    // small batches (fewer queries than SMs): the latency-bound phases of the
                                           // single query (gather, fp32 rescoring of ~200 scattered rows) get 4x the warps
 constexpr float PRUNE_MARGIN = 1.5f;       // in units of eps; typical |bf16 - fp32| is ~eps/25
 constexpr int RANK_BY_COUNT_MAX = 1024;    // survivors up to this many are ranked by counting, else bitonic sort
 
-template <int FIN_THREADS>
+template <int FIN_THREADS, bool EXCL>
 __global__ void __launch_bounds__(FIN_THREADS)
 flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn, long long N, int D, int K,
                      long long id_offset, const float* __restrict__ thr, const float* __restrict__ eps,
                      const unsigned int* __restrict__ seg_cnt, const uint2* __restrict__ cand, int nslices,
                      int seg_cap, int cand_cap,
                      float* __restrict__ scores, long long* __restrict__ ids, int* __restrict__ flags,
-                     int* __restrict__ n_uncertified, float* __restrict__ bound_out) {
+                     int* __restrict__ n_uncertified, float* __restrict__ bound_out,
+                     const long long* __restrict__ excl, int E) {
   pdl_trigger();
   pdl_wait();
   extern __shared__ __align__(16) unsigned char fsm[];
   unsigned long long* key = reinterpret_cast<unsigned long long*>(fsm);
   float* qs = reinterpret_cast<float*>(key + cand_cap);
+  unsigned int* ex = reinterpret_cast<unsigned int*>(qs + D);   // EXCL: the query's sorted exclusion list
   __shared__ int s_off[FINALIZE_MAX_SLICES + 1];
   __shared__ unsigned int s_hist[256];
   __shared__ int s_wsum[FIN_THREADS / 32];
-  __shared__ int s_over, s_bad, s_digit, s_kk;
+  __shared__ int s_over, s_bad, s_digit, s_kk, s_any_ex;
   __shared__ float s_fk;
   const int q = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int NWARPS = FIN_THREADS / 32;
+  const int EP = EXCL ? next_pow2(E) : 0;
 
   // ---- 1. segment sizes -> offsets (parallel loads, warp-0 scan) --------------------------------
-  if (tid == 0) { s_over = 0; s_bad = 0; s_fk = -INFINITY; s_off[0] = 0; }
+  if (tid == 0) { s_over = 0; s_bad = 0; s_fk = -INFINITY; s_off[0] = 0; s_any_ex = 0; }
   __syncthreads();
   for (int sl = tid; sl < nslices; sl += FIN_THREADS) {
     unsigned int c = seg_cnt[(size_t)q * nslices + sl];
@@ -100,7 +160,13 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
     s_off[sl + 1] = (int)c;
   }
   for (int d = tid; d < D; d += FIN_THREADS) qs[d] = qn[(long long)q * D + d];
+  if constexpr (EXCL) {
+    if (stage_exclusions(excl, E, q, id_offset, N, ex, EP)) s_any_ex = 1;
+  }
   __syncthreads();
+  if constexpr (EXCL) {
+    if (s_any_ex) bitonic_sort_desc(ex, EP);   // ends with a barrier
+  }
   if (warp == 0) {
     int carry = 0;
     for (int base = 0; base < nslices; base += 32) {
@@ -116,7 +182,7 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
   }
   __syncthreads();
   const bool overflow = s_over != 0;
-  const int n = s_off[nslices];
+  int n = s_off[nslices];
   const float my_eps = eps[q];
   const float t = thr[q];
 
@@ -128,6 +194,11 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
     key[i] = make_key(__uint_as_float(e.x), e.y);
   }
   __syncthreads();
+  if constexpr (EXCL) {
+    if (s_any_ex)   // from here on: allowed rows only
+      n = compact_keys<FIN_THREADS>(key, n, s_wsum,
+                                    [&](unsigned long long k) { return !is_excluded(ex, EP, key_row(k)); });
+  }
 
   // ---- 2. b_K by radix select on the ordered score bits (8 bits per pass, MSB first) --------------
   float cutoff = -INFINITY;
@@ -174,24 +245,8 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
 
   // ---- 3. prune: in-place compaction of the survivors (chunks of FIN_THREADS, left-moving) ---------
   int m = n;
-  if (cutoff > -INFINITY) {
-    int out = 0;
-    for (int base = 0; base < n; base += FIN_THREADS) {
-      const int i = base + tid;
-      const unsigned long long kk64 = (i < n) ? key[i] : 0ull;
-      const bool keep = (i < n) && (key_score(kk64) >= cutoff);
-      const unsigned int bal = __ballot_sync(0xffffffffu, keep);
-      if (lane == 0) s_wsum[warp] = __popc(bal);
-      __syncthreads();                       // also orders every read of this chunk before the writes below
-      int wbase = 0, tot = 0;
-#pragma unroll
-      for (int w = 0; w < NWARPS; ++w) { const int c = s_wsum[w]; if (w < warp) wbase += c; tot += c; }
-      if (keep) key[out + wbase + __popc(bal & ((1u << lane) - 1u))] = kk64;
-      out += tot;
-      __syncthreads();
-    }
-    m = out;
-  }
+  if (cutoff > -INFINITY)
+    m = compact_keys<FIN_THREADS>(key, n, s_wsum, [&](unsigned long long k) { return key_score(k) >= cutoff; });
 
   // ---- 4. fp32 rescoring of the m survivors (in place) --------------------------------------------
   const bool vec = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(Xn) & 15) == 0);
@@ -335,25 +390,41 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
   }
 }
 
+template <int NT, bool EXCL>
+static int launch_finalize_t(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,
+                             long long id_offset, const float* thr, const float* eps, const unsigned int* seg_cnt,
+                             const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
+                             float* bound_out, const long long* excl, int E, size_t smem, cudaStream_t st) {
+  TT_CHECK_CUDA(cudaFuncSetAttribute(flat_finalize_kernel<NT, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  TT_CHECK_CUDA(launch_pdl(flat_finalize_kernel<NT, EXCL>, dim3(nq), dim3(NT), smem, st, qn, Xn, N, D, K, id_offset, thr, eps,
+                           seg_cnt, reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap, pl.cand_cap, scores,
+                           ids, flags, n_uncertified, bound_out, excl, E));
+  return TT_OK;
+}
+
 int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,
                     long long id_offset, const float* thr, const float* eps, const unsigned int* seg_cnt,
                     const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
-                    float* bound_out, cudaStream_t st) {
+                    float* bound_out, cudaStream_t st, const long long* excl, int E) {
   TT_CHECK_ARG(pl.main_slices <= FINALIZE_MAX_SLICES, "too many catalog slices");
-  const size_t smem = (size_t)pl.cand_cap * 8 + (size_t)D * 4 + 16;
-  count_launch();
-  if (nq <= 16) {                 // measured (1M x 384): nq = 1 wide 20 us vs 31 us; nq = 128 wide 57 us vs 23 us
-    TT_CHECK_CUDA(cudaFuncSetAttribute(flat_finalize_kernel<FIN_THREADS_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    TT_CHECK_CUDA(launch_pdl(flat_finalize_kernel<FIN_THREADS_WIDE>, dim3(nq), dim3(FIN_THREADS_WIDE), smem, st, qn, Xn, N, D, K,
-                             id_offset, thr, eps, seg_cnt, reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap,
-                             pl.cand_cap, scores, ids, flags, n_uncertified, bound_out));
-  } else {
-    TT_CHECK_CUDA(cudaFuncSetAttribute(flat_finalize_kernel<FIN_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    TT_CHECK_CUDA(launch_pdl(flat_finalize_kernel<FIN_THREADS>, dim3(nq), dim3(FIN_THREADS), smem, st, qn, Xn, N, D, K, id_offset,
-                             thr, eps, seg_cnt, reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap, pl.cand_cap,
-                             scores, ids, flags, n_uncertified, bound_out));
+  const bool with_excl = excl != nullptr && E > 0;
+  size_t smem = (size_t)pl.cand_cap * 8 + (size_t)D * 4 + 16;
+  if (with_excl) {
+    int P = 1;
+    while (P < E) P <<= 1;
+    smem += (size_t)P * 4;
   }
-  return TT_OK;
+  count_launch();
+  // wide CTAs for small batches, measured (1M x 384): nq = 1 wide 20 us vs 31 us; nq = 128 wide 57 us vs 23 us
+  if (nq <= 16)
+    return with_excl ? launch_finalize_t<FIN_THREADS_WIDE, true>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand,
+                                                                scores, ids, flags, n_uncertified, bound_out, excl, E, smem, st)
+                     : launch_finalize_t<FIN_THREADS_WIDE, false>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand,
+                                                                 scores, ids, flags, n_uncertified, bound_out, nullptr, 0, smem, st);
+  return with_excl ? launch_finalize_t<FIN_THREADS, true>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand, scores,
+                                                         ids, flags, n_uncertified, bound_out, excl, E, smem, st)
+                   : launch_finalize_t<FIN_THREADS, false>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand, scores,
+                                                          ids, flags, n_uncertified, bound_out, nullptr, 0, smem, st);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -535,6 +606,23 @@ exact_scores_kernel(const float* __restrict__ q, const int* __restrict__ qsel, i
   }
 }
 
+// Exclusion lists on the exact path: the score of every excluded row becomes EXCL_SCORE_BITS, whose ordered key has
+// zero high bits, below the key of any real score (-inf included).  O(E) per query; select, collect and sort then
+// see these rows as the smallest keys and the sort writes them as (-inf, -1).  The list row is the QUERY row qsel[i].
+constexpr unsigned int EXCL_SCORE_BITS = 0xffffffffu;   // a negative NaN: float_to_ordered() maps it to 0
+
+__global__ void __launch_bounds__(256)
+exact_exclude_kernel(const long long* __restrict__ excl, int E, const int* __restrict__ qsel, int slot0,
+                     long long id_offset, long long N, float* __restrict__ scores_ws) {
+  const int s = blockIdx.x;
+  const int qi = qsel ? qsel[slot0 + s] : (slot0 + s);
+  for (int j = threadIdx.x; j < E; j += blockDim.x) {
+    const long long id = excl[(long long)qi * E + j];
+    const long long r = id - id_offset;
+    if (id >= 0 && r >= 0 && r < N) scores_ws[(long long)s * N + r] = __uint_as_float(EXCL_SCORE_BITS);
+  }
+}
+
 __global__ void exact_init_kernel(SelState* st, unsigned int* hist, int nslot, int K) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < nslot) { st[i].prefix = 0ull; st[i].kremain = K; st[i].count = 0u; }
@@ -595,7 +683,7 @@ exact_collect_kernel(const float* __restrict__ scores_ws, long long N, SelState*
 
 __global__ void __launch_bounds__(256)
 exact_sort_kernel(const unsigned long long* __restrict__ keys_in, const int* __restrict__ qsel, int slot0, int K,
-                  long long id_offset, float* __restrict__ scores, long long* __restrict__ ids) {
+                  long long id_offset, float* __restrict__ scores, long long* __restrict__ ids, bool excl) {
   extern __shared__ __align__(16) unsigned char ssm[];
   unsigned long long* key = reinterpret_cast<unsigned long long*>(ssm);
   const int s = blockIdx.x;
@@ -605,8 +693,13 @@ exact_sort_kernel(const unsigned long long* __restrict__ keys_in, const int* __r
   __syncthreads();
   bitonic_sort_desc(key, P);
   for (int i = threadIdx.x; i < K; i += blockDim.x) {
-    scores[(long long)qi * K + i] = key_score(key[i]);
-    ids[(long long)qi * K + i] = (long long)key_row(key[i]) + id_offset;
+    if (excl && (key[i] >> 32) == 0ull) {   // an excluded row (fewer than K allowed rows): the tail is padding
+      scores[(long long)qi * K + i] = -INFINITY;
+      ids[(long long)qi * K + i] = -1;
+    } else {
+      scores[(long long)qi * K + i] = key_score(key[i]);
+      ids[(long long)qi * K + i] = (long long)key_row(key[i]) + id_offset;
+    }
   }
 }
 
@@ -665,10 +758,9 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_exact_wo
   return exact_ws_layout(N, K, &a, &b, &c);
 }
 
-extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact(const float* q, int nq, const int32_t* qsel, int nsel,
-                                    const float* Xn, int64_t N, int D, int K, int64_t id_offset,
-                                    float* scores, int64_t* ids, void* workspace, size_t workspace_bytes,
-                                    void* stream) {
+static int flat_search_exact_impl(const float* q, int nq, const int32_t* qsel, int nsel, const float* Xn, int64_t N,
+                                  int D, int K, int64_t id_offset, float* scores, int64_t* ids, const int64_t* excl,
+                                  int E, void* workspace, size_t workspace_bytes, void* stream) {
   TT_CHECK_ARG(q && Xn && scores && ids && workspace, "null pointer");
   TT_CHECK_ARG(N >= 1 && N < (1LL << 32) && D >= 1, "need 1 <= N < 2^32, D >= 1");
   TT_CHECK_ARG(K >= 1 && K <= N && K <= TT_FLAT_MAX_K, "need 1 <= K <= min(N, TT_FLAT_MAX_K)");
@@ -698,6 +790,11 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact(const
     if (gw > (long long)sms * 4) gw = (long long)sms * 4;
     exact_scores_kernel<<<(unsigned)gw, 256, smem_q, st>>>(q, qsel, slot0, nslot, Xn, N, D, scores_ws);
     TT_CHECK_LAUNCH();
+    if (E > 0) {
+      exact_exclude_kernel<<<nslot, 256, 0, st>>>(reinterpret_cast<const long long*>(excl), E, qsel, slot0, id_offset, N,
+                                                  scores_ws);
+      TT_CHECK_LAUNCH();
+    }
     exact_init_kernel<<<(nslot * 256 + 255) / 256, 256, 0, st>>>(state, hist, nslot, K);
     TT_CHECK_LAUNCH();
     for (int shift = 56; shift >= 0; shift -= 8) {
@@ -709,8 +806,26 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact(const
     exact_collect_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(scores_ws, N, state, keys, K);
     TT_CHECK_LAUNCH();
     exact_sort_kernel<<<nslot, 256, (size_t)P * 8, st>>>(keys, qsel, slot0, K, id_offset, scores,
-                                                         reinterpret_cast<long long*>(ids));
+                                                         reinterpret_cast<long long*>(ids), E > 0);
     TT_CHECK_LAUNCH();
   }
   return TT_OK;
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact(const float* q, int nq, const int32_t* qsel, int nsel,
+                                    const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                                    float* scores, int64_t* ids, void* workspace, size_t workspace_bytes,
+                                    void* stream) {
+  return flat_search_exact_impl(q, nq, qsel, nsel, Xn, N, D, K, id_offset, scores, ids, nullptr, 0, workspace,
+                                workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact_excl(const float* q, int nq, const int32_t* qsel, int nsel,
+                                         const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                                         float* scores, int64_t* ids, const int64_t* excl, int E,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+  TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
+  TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
+  return flat_search_exact_impl(q, nq, qsel, nsel, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
+                                workspace_bytes, stream);
 }

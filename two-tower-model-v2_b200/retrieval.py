@@ -64,12 +64,22 @@ class RetrievalPipeline:
         """history rows i64 [B,S] + weights f32 [B,S] (device) -> buyer embeddings [B,D] (device)."""
         return self.tower.forward_gather(self.table, indices, weights, self.item_logits)
 
-    def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int) -> PendingSearch:
+    def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int, *,
+                              exclude_history: bool = False) -> PendingSearch:
+        """exclude_history: the pooled history rows `indices` (-1 padded; the last `max_interaction_history`
+        interactions when they come from encode_histories) are also the exclusion list of the search, so no buyer
+        is shown the items they have just viewed, carted or bought.  No extra host-to-device copy."""
         k = min(k, self.index.ntotal)                                                  # vector_db.py:159
-        return self.index.search_async(self.encode_device(indices, weights), k)
+        emb = self.encode_device(indices, weights)
+        if not exclude_history:
+            return self.index.search_async(emb, k)
+        excl = indices.to(device=self.index.device, dtype=torch.int64).contiguous()
+        return self.index.search_async(emb, k, exclude=excl)
 
-    def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10):
-        """-> (scores f32 [B,k'], row indices i64 [B,k']) numpy; one H2D of the padded history, one D2H."""
+    def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *, exclude_history: bool = False):
+        """-> (scores f32 [B,k'], row indices i64 [B,k']) numpy; one H2D of the padded history, one D2H.
+        exclude_history: leave out the buyer's last `max_interaction_history` interacted items (see
+        retrieve_device_async); a buyer with fewer than k' other items gets (-inf, -1) at the tail."""
         idx, w, _ = self.encode_histories(batch)
         key = idx.shape
         pins = self._pins.get(key)
@@ -81,18 +91,26 @@ class RetrievalPipeline:
         pins[0].copy_(torch.from_numpy(idx))
         pins[1].copy_(torch.from_numpy(w))
         dev = self.index.device
-        scores, ids, _ = self.retrieve_device_async(pins[0].to(dev, non_blocking=True), pins[1].to(dev, non_blocking=True),
-                                                    k).result()
+        idx_dev, w_dev = pins[0].to(dev, non_blocking=True), pins[1].to(dev, non_blocking=True)
+        if exclude_history:
+            pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=True)
+        else:
+            pending = self.retrieve_device_async(idx_dev, w_dev, k)
+        scores, ids, _ = pending.result()
         return scores.cpu().numpy(), ids.cpu().numpy()
 
-    def retrieve(self, interactions: Sequence[Dict[str, Any]], k: int = 10) -> List[Tuple[str, float]]:
-        """One request, the shape of server.py:241-244 -> [(product_id, score)] in descending score."""
-        scores, ids = self.retrieve_arrays([interactions], k)
+    def retrieve(self, interactions: Sequence[Dict[str, Any]], k: int = 10, *,
+                 exclude_history: bool = False) -> List[Tuple[str, float]]:
+        """One request, the shape of server.py:241-244 -> [(product_id, score)] in descending score.
+        exclude_history: never return the items of the buyer's last `max_interaction_history` interactions."""
+        scores, ids = self.retrieve_arrays([interactions], k, exclude_history=exclude_history)
         pids = self.db.product_ids
         return [(pids[i], float(s)) for i, s in zip(ids[0].tolist(), scores[0].tolist()) if 0 <= i < len(pids)]
 
-    def retrieve_batch(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10) -> List[List[Tuple[str, float]]]:
-        scores, ids = self.retrieve_arrays(batch, k)
+    def retrieve_batch(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *,
+                       exclude_history: bool = False) -> List[List[Tuple[str, float]]]:
+        """exclude_history: as in retrieve, per buyer."""
+        scores, ids = self.retrieve_arrays(batch, k, exclude_history=exclude_history)
         pids = self.db.product_ids
         n = len(pids)
         return [[(pids[i], s) for i, s in zip(ri, rs) if 0 <= i < n] for rs, ri in zip(scores.tolist(), ids.tolist())]
@@ -162,14 +180,27 @@ class ShardedRetrievalPipeline:
                 dist.all_gather_into_tensor(gathered.view(-1), partial.view(-1), group=self.group)
         return ops.pool_partial_merge(gathered, self.attention)
 
-    def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int) -> PendingSearch:
+    def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int, *,
+                              exclude_history: bool = False) -> PendingSearch:
+        """exclude_history: the pooled history rows (global ids, -1 padded; the last `max_interaction_history`
+        interactions when built by RetrievalPipeline.encode_histories) are the exclusion list of the search."""
         k = min(k, self.n_total)                                                       # vector_db.py:159
-        return self.sharded.search_async(self.encode_device(indices, weights, k), k)
+        emb = self.encode_device(indices, weights, k)
+        if not exclude_history:
+            return self.sharded.search_async(emb, k)
+        excl = indices.to(device=self.table.device, dtype=torch.int64).contiguous()
+        return self.sharded.search_async(emb, k, exclude=excl)
 
-    def retrieve_host_async(self, idx_host: torch.Tensor, w_host: torch.Tensor, k: int) -> PendingSearch:
-        """Pinned host tensors in (history rows / weights of the WHOLE batch, the same on every rank), numpy out."""
+    def retrieve_host_async(self, idx_host: torch.Tensor, w_host: torch.Tensor, k: int, *,
+                            exclude_history: bool = False) -> PendingSearch:
+        """Pinned host tensors in (history rows / weights of the WHOLE batch, the same on every rank), numpy out.
+        exclude_history: as in retrieve_device_async (the copied history rows are the list)."""
         dev = self.table.device
-        pending = self.retrieve_device_async(idx_host.to(dev, non_blocking=True), w_host.to(dev, non_blocking=True), k)
+        idx_dev, w_dev = idx_host.to(dev, non_blocking=True), w_host.to(dev, non_blocking=True)
+        if exclude_history:
+            pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=True)
+        else:
+            pending = self.retrieve_device_async(idx_dev, w_dev, k)
 
         def finish():
             s, i, n_bad = pending.result()

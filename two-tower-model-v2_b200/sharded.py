@@ -347,16 +347,32 @@ class ShardedFlatIPIndex:
             raise ValueError(f"shards hold {total} rows in total but n_total = {self.n_total}")
         self._n_local_min, self._n_local_max = n_min, n_max
 
-    def _local_search(self, q: torch.Tensor, k: int, k_local: int, world: int, views, p2p=None, status=None) -> None:
+    def _global_threshold(self, world: int, nq: int, k: int, exclude) -> bool:
+        """Whether all ranks take the one-threshold plan.  A function of replicated values only (n_total, the
+        smallest shard, nq, k and the exclusion list width), so every rank decides alike.  With E exclusions per
+        query the plan is made for K_plan = min(k + E, n_total, TT_FLAT_MAX_K)."""
+        n_local_min = self._n_local_min if self._n_local_min is not None else self.local.ntotal
+        plan_ok = getattr(self.local, "shard_plan_ok", None)
+        if exclude is not None:
+            from ._native import plan_k
+            k = plan_k(k, exclude.shape[1], self.n_total)
+        return world > 1 and n_local_min >= k and plan_ok is not None and plan_ok(self.n_total, nq, k, max(n_local_min, 0))
+
+    @staticmethod
+    def _kw(exclude):
+        """Keyword arguments of the local calls: none without a list, so stand-ins that predate it keep working."""
+        return {} if exclude is None else {"exclude": exclude}
+
+    def _local_search(self, q: torch.Tensor, k: int, k_local: int, world: int, views, p2p=None, status=None,
+                      exclude=None) -> None:
         """Fills this rank's record.  With every shard holding >= k rows and a plan for it, all ranks use ONE
         threshold estimated from a sample of the whole catalog (a small all-gather of per-rank top-r sampled
         scores): candidates per rank drop to ~1/G of the single-device count.  Otherwise each shard picks its
         own threshold."""
         scores, ids, bound, flags = views
         nq = q.shape[0]
-        n_local_min = self._n_local_min if self._n_local_min is not None else self.local.ntotal
-        plan_ok = getattr(self.local, "shard_plan_ok", None)
-        if world > 1 and n_local_min >= k and plan_ok is not None and plan_ok(self.n_total, nq, k, max(n_local_min, 0)):
+        kw = self._kw(exclude)
+        if self._global_threshold(world, nq, k, exclude):
             from ._native import TT_SHARD_TOPR
             key = ("topr", nq, world)
             bufs = self._bufs.get(key)
@@ -364,16 +380,16 @@ class ShardedFlatIPIndex:
                 bufs = self._bufs[key] = (torch.empty((nq, TT_SHARD_TOPR), device=q.device, dtype=torch.float32),
                                           torch.empty((world, nq, TT_SHARD_TOPR), device=q.device, dtype=torch.float32))
             topr, topr_g = bufs
-            self.local.shard_sample(q, k, self.n_total, topr)
+            self.local.shard_sample(q, k, self.n_total, topr, **kw)
             if p2p is not None:
                 topr_g = p2p.all_gather(0, topr.view(torch.uint8).view(-1), status).view(torch.float32).view(world, nq, TT_SHARD_TOPR)
             else:
                 dist.all_gather_into_tensor(topr_g.view(-1), topr.view(-1), group=self.group)
-            self.local.shard_search_into(nq, k, self.n_total, topr_g, scores, ids, bound, flags)
+            self.local.shard_search_into(nq, k, self.n_total, topr_g, scores, ids, bound, flags, **kw)
         else:
-            self.local.search_shard_into(q, k_local, scores, ids, bound, flags)
+            self.local.search_shard_into(q, k_local, scores, ids, bound, flags, **kw)
 
-    def search_async(self, q: torch.Tensor, k: int):
+    def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
         """Enqueues the sharded search of one batch and returns a PendingSearch; `.result()` looks at the global
         certificate later (no host sync between consecutive batches).
 
@@ -384,20 +400,22 @@ class ShardedFlatIPIndex:
                       C(j-2) wait for the peers' records of j-2, merge + global certificate
         `.result()` of a batch first enqueues whatever stages it (and every older batch) still misses.  Every rank
         issues the same calls in the same order, so the exchanges pair up.  A caller that keeps three batches in
-        flight gets the full overlap; with fewer the stages simply run back to back."""
+        flight gets the full overlap; with fewer the stages simply run back to back.
+
+        `exclude` (i64 [nq, E], GLOBAL ids, -1 = padding, replicated on every rank like q): the exact top-k over the
+        rows query i does not list; with fewer than k allowed rows the tail is (-inf, -1)."""
         from .vector_db import PendingSearch
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         nq = q.shape[0]
+        if exclude is not None and exclude.shape[1] == 0:
+            exclude = None
         self._validate(world, q.device)
         lay, rec, gathered = self._buffers(nq, k, q.device, world)
         k_local = min(k, self.local.ntotal)
         p2p = self._p2p_for(nq, k, q.device, world, lay)
-        n_local_min = self._n_local_min if self._n_local_min is not None else self.local.ntotal
-        plan_ok = getattr(self.local, "shard_plan_ok", None)
-        global_thr = (world > 1 and n_local_min >= k and plan_ok is not None
-                      and plan_ok(self.n_total, nq, k, max(n_local_min, 0)))
+        global_thr = self._global_threshold(world, nq, k, exclude)
         if p2p is not None and global_thr and self.pipelined:
-            return self._search_pipelined(q, k, nq, world, lay, rec, p2p)
+            return self._search_pipelined(q, k, nq, world, lay, rec, p2p, exclude)
         self.flush()          # never interleave the two schedules
         views = record_views(rec, lay, nq, k)
         scores, ids, bound, flags = views
@@ -406,19 +424,19 @@ class ShardedFlatIPIndex:
             ids.fill_(-1)
         if p2p is not None:
             status = self._bufs.setdefault(("status", nq, k, world), torch.zeros(2, dtype=torch.int32, device=q.device))
-            self._local_search(q, k, k_local, world, views, p2p, status)
+            self._local_search(q, k, k_local, world, views, p2p, status, exclude)
             gathered = p2p.all_gather(1, rec, status)
             s, i, fl, n_unc = self._merge(gathered, lay, nq, k, status[0:1])
             n_unc = status
         else:
-            self._local_search(q, k, k_local, world, views)
+            self._local_search(q, k, k_local, world, views, exclude=exclude)
             self._exchange(rec, gathered, world)
             s, i, fl, n_unc = self._merge(gathered, lay, nq, k)
         post = getattr(self.local, "post_flag", None)
         token = post(n_unc) if post is not None else None
-        return PendingSearch(lambda: self._finish(q, k, s, i, fl, n_unc, token))
+        return PendingSearch(lambda: self._finish(q, k, s, i, fl, n_unc, token, exclude))
 
-    def _finish(self, q, k, s, i, fl, n_unc, token):
+    def _finish(self, q, k, s, i, fl, n_unc, token, exclude=None):
         # identical on every rank: all ranks merged the same records
         st = self.local.read_flag(token) if token is not None else int(n_unc)
         if isinstance(st, list):
@@ -431,7 +449,8 @@ class ShardedFlatIPIndex:
         # Re-run the flagged queries alone (this rank's record buffer may already hold a later batch):
         # exact fp32 search of every shard, a small exchange, merge, scatter into the result.
         rows = torch.nonzero(fl != 1).flatten()
-        s2, i2 = self.search_exact_device(q[rows].contiguous(), k)
+        kw = {} if exclude is None else {"exclude": exclude[rows].contiguous()}
+        s2, i2 = self.search_exact_device(q[rows].contiguous(), k, **kw)
         s[rows] = s2
         i[rows] = i2
         return s, i, n_bad
@@ -439,7 +458,7 @@ class ShardedFlatIPIndex:
     # -- 3-stage pipeline -----------------------------------------------------------------------------------------
     NSLOT = 3      # batches in flight: workspaces / status words are per slot
 
-    def _search_pipelined(self, q, k, nq, world, lay, rec, p2p):
+    def _search_pipelined(self, q, k, nq, world, lay, rec, p2p, exclude=None):
         from ._native import TT_SHARD_TOPR
         from .vector_db import PendingSearch
         self._pipe_seq = getattr(self, "_pipe_seq", 0) + 1
@@ -448,9 +467,9 @@ class ShardedFlatIPIndex:
         topr = self._bufs.setdefault(("topr1", nq, world), torch.empty((nq, TT_SHARD_TOPR), device=dev, dtype=torch.float32))
         status = self._bufs.setdefault(("status", nq, k, world, slot), torch.zeros(2, dtype=torch.int32, device=dev))
         b = {"q": q, "k": k, "nq": nq, "world": world, "lay": lay, "rec": rec, "p2p": p2p, "slot": slot, "status": status,
-             "stage": 0, "out": None}
+             "stage": 0, "out": None, "exclude": exclude}
         # stage A: sample pass + push of the top-r lists (no wait)
-        self.local.shard_sample(q, k, self.n_total, topr, slot)
+        self.local.shard_sample(q, k, self.n_total, topr, slot, **self._kw(exclude))
         b["seq0"] = p2p.push(0, topr.view(torch.uint8).view(-1))
         b["stage"] = 1
         self._inflight.append(b)
@@ -467,7 +486,8 @@ class ShardedFlatIPIndex:
         if b["stage"] < 2 <= to_stage:          # stage B
             topr_g = p2p.wait(0, b["seq0"], b["status"]).view(torch.float32).view(world, nq, TT_SHARD_TOPR)
             scores, ids, bound, flags = record_views(b["rec"], lay, nq, k)
-            self.local.shard_search_into(nq, k, self.n_total, topr_g, scores, ids, bound, flags, b["slot"])
+            self.local.shard_search_into(nq, k, self.n_total, topr_g, scores, ids, bound, flags, b["slot"],
+                                         **self._kw(b["exclude"]))
             b["seq1"] = p2p.push(1, b["rec"])
             b["stage"] = 2
         if b["stage"] < 3 <= to_stage:          # stage C
@@ -491,12 +511,15 @@ class ShardedFlatIPIndex:
                     break
         self._inflight = [x for x in self._inflight if x["stage"] < 3]
         s, i, fl, token = b["out"]
-        return self._finish(b["q"], b["k"], s, i, fl, b["status"], token)
+        return self._finish(b["q"], b["k"], s, i, fl, b["status"], token, b["exclude"])
 
-    def search_exact_device(self, q: torch.Tensor, k: int):
+    def search_exact_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
         """Always-exact fp32 path over the sharded catalog (collective: every rank calls it with the same q):
         fp32 exact search of every shard, one exchange of the records (NCCL / plain copy), merge.  Serves the
-        queries the global certificate rejects and the parity checks of bench.py / tests."""
+        queries the global certificate rejects and the parity checks of bench.py / tests.  With `exclude` a query
+        may have fewer than k allowed rows: its merged list then ends in (-inf, -1), which is exact here."""
+        if exclude is not None and exclude.shape[1] == 0:
+            exclude = None
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         nsel = q.shape[0]
         k_local = min(k, self.local.ntotal)
@@ -509,22 +532,27 @@ class ShardedFlatIPIndex:
         b_l.fill_(float("-inf"))
         f_l.fill_(1)
         if k_local > 0:
-            self.local.search_exact_into(q, k_local, s_l, i_l, torch.arange(nsel, device=q.device, dtype=torch.int32))
+            self.local.search_exact_into(q, k_local, s_l, i_l, torch.arange(nsel, device=q.device, dtype=torch.int32),
+                                         **self._kw(exclude))
         self._exchange(rec2, gathered2, world)
         s2, i2, fl2, n_unc2 = self._merge(gathered2, lay2, nsel, k)
-        if int(n_unc2):
+        if exclude is None:
+            if int(n_unc2):
+                raise RuntimeError("sharded search: queries still uncertified after the exact re-run")
+        elif bool(((fl2 != 1) & (fl2 != -2)).any()):     # -2 alone: fewer than k allowed rows, exact as padded
             raise RuntimeError("sharded search: queries still uncertified after the exact re-run")
         return s2, i2
 
-    def search_device(self, q: torch.Tensor, k: int):
+    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
         """q replicated on every rank -> global (scores, ids) [nq,k] on every rank, and the number of
         queries that failed the global certificate and were re-run through the exact path."""
-        return self.search_async(q, k).result()
+        return self.search_async(q, k, **self._kw(exclude)).result()
 
-    def search_host_async(self, q, k: int):
-        """numpy in / numpy out round trip (pinned staging), asynchronous; `.result()` -> (scores, ids, n_rerun)."""
+    def search_host_async(self, q, k: int, *, exclude=None):
+        """numpy in / numpy out round trip (pinned staging), asynchronous; `.result()` -> (scores, ids, n_rerun).
+        `exclude`: numpy int64 [nq, E] global ids (see search_async)."""
         from .vector_db import host_search_async
-        return host_search_async(self, self.search_async, self.local.device, self.local.d, q, k)
+        return host_search_async(self, self.search_async, self.local.device, self.local.d, q, k, exclude=exclude)
 
     def search_host_sliced_async(self, q_local, k: int):
         """Serving layout for G ranks fronting one sharded catalog: every rank submits ITS share of the batch

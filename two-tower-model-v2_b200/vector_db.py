@@ -288,23 +288,42 @@ class FlatIPIndex:
         return self.xn.cpu().numpy()
 
     # -- search ----------------------------------------------------------------------------
-    def _workspace(self, nq: int, k: int) -> torch.Tensor:
-        key = (nq, k)
+    def _exclusions(self, exclude, nq: int) -> Optional[torch.Tensor]:
+        """Validates an exclusion list (CUDA i64 [nq, E], ids in this index's result id space, -1 padded) -> the
+        contiguous tensor, or None when there is nothing to exclude (E == 0 runs the plain search)."""
+        if exclude is None:
+            return None
+        if not (isinstance(exclude, torch.Tensor) and exclude.is_cuda and exclude.dtype == torch.int64
+                and exclude.dim() == 2 and exclude.shape[0] == nq):
+            raise ValueError(f"exclude must be a CUDA int64 tensor [nq={nq}, E], got "
+                             f"{getattr(exclude, 'dtype', type(exclude))} {tuple(getattr(exclude, 'shape', ()))}")
+        if exclude.shape[1] > _native.TT_FLAT_MAX_EXCLUDE:
+            raise ValueError(f"at most {_native.TT_FLAT_MAX_EXCLUDE} exclusions per query, got {exclude.shape[1]}")
+        if exclude.shape[1] == 0:
+            return None
+        return exclude.to(self.device).contiguous()
+
+    def _workspace(self, nq: int, k: int, n_excl: int = 0) -> torch.Tensor:
+        key = (nq, k) if n_excl == 0 else (nq, k, "excl", n_excl)
         ws = self._ws.get(key)
         if ws is None:
-            nbytes = int(_native.load().tt_flat_search_workspace_bytes(self.ntotal, self.d, nq, k))
+            lib = _native.load()
+            nbytes = int(lib.tt_flat_search_workspace_bytes(self.ntotal, self.d, nq, k) if n_excl == 0 else
+                         lib.tt_flat_search_excl_workspace_bytes(self.ntotal, self.d, nq, k, n_excl))
             ws = torch.empty(max(nbytes, 256), device=self.device, dtype=torch.uint8)
             if len(self._ws) > 8:
                 self._ws.clear()
             self._ws[key] = ws
         return ws
 
-    def search_device(self, q: torch.Tensor, k: int):
+    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
         """Asynchronous search of CUDA f32 queries [nq,D] on the current stream.
 
         Returns (scores [nq,k] f32, ids [nq,k] i64, flags [nq] i32, n_uncertified [1] i32) device
         tensors; rows with flags != 1 (1 = certified exact, <= 0 = -(reason bits), see include/tt_b200.h) must be
         passed to `search_exact_device` (`search_checked_device` / `search_async` do both).
+        `exclude` (CUDA i64 [nq, E], E <= 1024, ids as returned, -1 = padding): the top-k over the rows query i does
+        not list in exclude[i]; with fewer than k allowed rows the tail is (-inf, -1).
         """
         if self.ntotal == 0:
             raise ValueError("empty index")
@@ -314,23 +333,36 @@ class FlatIPIndex:
             raise ValueError(f"k must be in [1, min(ntotal, {_native.TT_FLAT_MAX_K})], got {k}")
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
+        excl = self._exclusions(exclude, nq)
         scores = torch.empty((nq, k), device=self.device, dtype=torch.float32)
         ids = torch.empty((nq, k), device=self.device, dtype=torch.int64)
         flags = torch.empty((max(nq, 1),), device=self.device, dtype=torch.int32)
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
-        ws = self._workspace(max(nq, 1), k)
+        lib = _native.load()
         with torch.cuda.device(self.device):
-            _native.check(_native.load().tt_flat_search(
-                q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
-                k, self.id_offset, scores.data_ptr(), ids.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
-                ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_search")
+            if excl is None:
+                ws = self._workspace(max(nq, 1), k)
+                _native.check(lib.tt_flat_search(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, scores.data_ptr(), ids.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_search")
+            else:
+                E = excl.shape[1]
+                ws = self._workspace(max(nq, 1), k, E)
+                _native.check(lib.tt_flat_search_excl(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, scores.data_ptr(), ids.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    excl.data_ptr(), E, ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_search_excl")
         return scores, ids, flags[:nq], nunc
 
     def search_exact_device(self, q: torch.Tensor, k: int, scores: Optional[torch.Tensor] = None,
-                            ids: Optional[torch.Tensor] = None, qsel: Optional[torch.Tensor] = None):
-        """Always-exact fp32 path; with `qsel` (i32 query rows) only those rows of scores/ids are rewritten."""
+                            ids: Optional[torch.Tensor] = None, qsel: Optional[torch.Tensor] = None, *,
+                            exclude: Optional[torch.Tensor] = None):
+        """Always-exact fp32 path; with `qsel` (i32 query rows) only those rows of scores/ids are rewritten.
+        `exclude` [nq, E] is indexed by query row (qsel[i]), as in search_device."""
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
+        excl = self._exclusions(exclude, nq)
         if scores is None:
             scores = torch.empty((nq, k), device=self.device, dtype=torch.float32)
             ids = torch.empty((nq, k), device=self.device, dtype=torch.int64)
@@ -340,39 +372,57 @@ class FlatIPIndex:
         if self._exact_ws is None or self._exact_ws.numel() < need:
             self._exact_ws = torch.empty(need, device=self.device, dtype=torch.uint8)
         with torch.cuda.device(self.device):
-            _native.check(lib.tt_flat_search_exact(
-                q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
-                self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(), self._exact_ws.data_ptr(),
-                self._exact_ws.numel(), ops._stream()), "tt_flat_search_exact")
+            if excl is None:
+                _native.check(lib.tt_flat_search_exact(
+                    q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
+                    self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(), self._exact_ws.data_ptr(),
+                    self._exact_ws.numel(), ops._stream()), "tt_flat_search_exact")
+            else:
+                _native.check(lib.tt_flat_search_exact_excl(
+                    q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
+                    self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(), excl.data_ptr(), excl.shape[1],
+                    self._exact_ws.data_ptr(), self._exact_ws.numel(), ops._stream()), "tt_flat_search_exact_excl")
         return scores, ids
 
     def search_shard_into(self, q: torch.Tensor, k: int, scores: torch.Tensor, ids: torch.Tensor,
-                          bound: torch.Tensor, flags: torch.Tensor) -> None:
+                          bound: torch.Tensor, flags: torch.Tensor, *, exclude: Optional[torch.Tensor] = None) -> None:
         """Shard-local search for ShardedFlatIPIndex (tt_flat_search_shard): fills the caller's record views.
-        scores/ids are [nq, k_record] with k_record >= k; only the first k columns of each row are written."""
+        scores/ids are [nq, k_record] with k_record >= k; only the first k columns of each row are written.
+        `exclude` holds GLOBAL ids (ids of other shards are ignored here)."""
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
+        excl = self._exclusions(exclude, nq)
         direct = scores.shape[1] == k and scores.is_contiguous() and ids.is_contiguous()
         s_out = scores if direct else torch.empty((nq, k), device=self.device, dtype=torch.float32)
         i_out = ids if direct else torch.empty((nq, k), device=self.device, dtype=torch.int64)
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
-        ws = self._workspace(max(nq, 1), k)
+        lib = _native.load()
         with torch.cuda.device(self.device):
-            _native.check(_native.load().tt_flat_search_shard(
-                q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
-                k, self.id_offset, s_out.data_ptr(), i_out.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
-                bound.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_search_shard")
+            if excl is None:
+                ws = self._workspace(max(nq, 1), k)
+                _native.check(lib.tt_flat_search_shard(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, s_out.data_ptr(), i_out.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    bound.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_search_shard")
+            else:
+                ws = self._workspace(max(nq, 1), k, excl.shape[1])
+                _native.check(lib.tt_flat_search_shard_excl(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, s_out.data_ptr(), i_out.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    bound.data_ptr(), excl.data_ptr(), excl.shape[1], ws.data_ptr(), ws.numel(), ops._stream()),
+                    "tt_flat_search_shard_excl")
         if not direct:
             scores[:, :k].copy_(s_out)
             ids[:, :k].copy_(i_out)
 
     def search_exact_into(self, q: torch.Tensor, k: int, scores: torch.Tensor, ids: torch.Tensor,
-                          qsel: torch.Tensor) -> None:
+                          qsel: torch.Tensor, *, exclude: Optional[torch.Tensor] = None) -> None:
         """Exact fp32 re-run of the query rows `qsel`, written into [nq, k_record] record views."""
+        kw = {} if exclude is None else {"exclude": exclude}
         if scores.shape[1] == k and scores.is_contiguous() and ids.is_contiguous():
-            self.search_exact_device(q, k, scores, ids, qsel)
+            self.search_exact_device(q, k, scores, ids, qsel, **kw)
             return
-        s_tmp, i_tmp = self.search_exact_device(q, k)
+        s_tmp, i_tmp = self.search_exact_device(q, k, **kw)
         rows = qsel.long()
         scores[rows, :k] = s_tmp[rows]
         ids[rows, :k] = i_tmp[rows]
@@ -392,10 +442,12 @@ class FlatIPIndex:
                                                   ops._stream()), "tt_flat_scan_scores")
         return out
 
-    def search_async(self, q: torch.Tensor, k: int) -> PendingSearch:
+    def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None) -> PendingSearch:
         """Enqueues a search and returns at once; `.result()` checks the certificate later, so a caller can
-        keep the next batch's kernels queued behind this one (no idle GPU between batches)."""
-        scores, ids, flags, nunc = self.search_device(q, k)
+        keep the next batch's kernels queued behind this one (no idle GPU between batches).  `exclude`: see
+        search_device; uncertified queries are re-run exactly with the same lists."""
+        kw = {} if exclude is None else {"exclude": exclude}
+        scores, ids, flags, nunc = self.search_device(q, k, **kw)
         if self._ring is None:
             self._ring = _FlagRing()
         token = self._ring.post(nunc)
@@ -404,13 +456,13 @@ class FlatIPIndex:
             n_bad = self._ring.read(*token)
             if n_bad:
                 qsel = torch.nonzero(flags != 1).flatten().to(torch.int32)
-                self.search_exact_device(q, k, scores, ids, qsel)
+                self.search_exact_device(q, k, scores, ids, qsel, **kw)
             return scores, ids, n_bad
         return PendingSearch(finish)
 
-    def search_checked_device(self, q: torch.Tensor, k: int):
+    def search_checked_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
         """search_device + re-run of uncertified queries through the exact path (one host sync)."""
-        return self.search_async(q, k).result()
+        return self.search_async(q, k, **({} if exclude is None else {"exclude": exclude})).result()
 
     def post_flag(self, nunc_dev: torch.Tensor):
         if self._ring is None:
@@ -435,10 +487,14 @@ class FlatIPIndex:
             self._ws[key] = ws
         return ws
 
-    def shard_sample(self, q: torch.Tensor, k: int, n_total: int, topr: torch.Tensor, slot: int = 0) -> None:
+    def shard_sample(self, q: torch.Tensor, k: int, n_total: int, topr: torch.Tensor, slot: int = 0, *,
+                     exclude: Optional[torch.Tensor] = None) -> None:
         """Phase 1 of the sharded search: fills topr f32 [nq, TT_SHARD_TOPR] (this shard's largest sampled scores).
         `slot` selects the workspace (phase 2 of the same batch must use the same slot; batches in flight at the same
-        time need different slots)."""
+        time need different slots).  With `exclude` [nq, E] the sample is planned for K_plan = min(k + E, n_total,
+        TT_FLAT_MAX_K); phase 2 must get the same list."""
+        if exclude is not None and exclude.shape[1] > 0:
+            k = _native.plan_k(k, exclude.shape[1], n_total)
         q = ops._f32c(q, "queries")
         ws = self._shard_workspace(n_total, q.shape[0], k, slot)
         with torch.cuda.device(self.device):
@@ -447,36 +503,55 @@ class FlatIPIndex:
                 topr.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_shard_sample")
 
     def shard_search_into(self, nq: int, k: int, n_total: int, topr_g: torch.Tensor, scores: torch.Tensor,
-                          ids: torch.Tensor, bound: torch.Tensor, flags: torch.Tensor, slot: int = 0) -> None:
+                          ids: torch.Tensor, bound: torch.Tensor, flags: torch.Tensor, slot: int = 0, *,
+                          exclude: Optional[torch.Tensor] = None) -> None:
         """Phase 2: global threshold from the gathered lists [G, nq, TT_SHARD_TOPR], main scan, finalize into
-        the record views (scores/ids must be contiguous [nq,k])."""
-        ws = self._shard_workspace(n_total, nq, k, slot)
+        the record views (scores/ids must be contiguous [nq,k]).  `exclude`: the list phase 1 was given."""
+        excl = self._exclusions(exclude, nq)
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
+        lib = _native.load()
         with torch.cuda.device(self.device):
-            _native.check(_native.load().tt_flat_shard_search(
-                nq, self.xn.data_ptr(), self.xh.data_ptr(), self.ntotal, n_total, self.d, k, self.id_offset,
-                topr_g.data_ptr(), topr_g.shape[0], scores.data_ptr(), ids.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
-                bound.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_shard_search")
+            if excl is None:
+                ws = self._shard_workspace(n_total, nq, k, slot)
+                _native.check(lib.tt_flat_shard_search(
+                    nq, self.xn.data_ptr(), self.xh.data_ptr(), self.ntotal, n_total, self.d, k, self.id_offset,
+                    topr_g.data_ptr(), topr_g.shape[0], scores.data_ptr(), ids.data_ptr(), flags.data_ptr(),
+                    nunc.data_ptr(), bound.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_shard_search")
+            else:
+                ws = self._shard_workspace(n_total, nq, _native.plan_k(k, excl.shape[1], n_total), slot)
+                _native.check(lib.tt_flat_shard_search_excl(
+                    nq, self.xn.data_ptr(), self.xh.data_ptr(), self.ntotal, n_total, self.d, k, self.id_offset,
+                    topr_g.data_ptr(), topr_g.shape[0], scores.data_ptr(), ids.data_ptr(), flags.data_ptr(),
+                    nunc.data_ptr(), bound.data_ptr(), excl.data_ptr(), excl.shape[1], ws.data_ptr(), ws.numel(),
+                    ops._stream()), "tt_flat_shard_search_excl")
 
-    def search_host_async(self, q: np.ndarray, k: int) -> PendingSearch:
+    def search_host_async(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None) -> PendingSearch:
         """Host-to-host search, asynchronous: stages q through pinned memory, enqueues H2D + search + D2H and
-        returns; `.result()` -> (scores, ids, n_rerun) numpy arrays.  Up to 3 calls may be in flight."""
-        return host_search_async(self, self.search_async, self.device, self.d, q, k)
+        returns; `.result()` -> (scores, ids, n_rerun) numpy arrays.  Up to 3 calls may be in flight.
+        `exclude`: numpy int64 [nq, E] (see search_device)."""
+        return host_search_async(self, self.search_async, self.device, self.d, q, k, exclude=exclude)
 
-    def search(self, q: np.ndarray, k: int) -> Tuple[np.ndarray, np.ndarray]:
+    def search(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
         """Host-to-host search, the shape of faiss `index.search(q, k)`: q f32 [nq,d] (un-normalised:
-        the device op applies q/(||q||+1e-8)) -> (scores f32 [nq,k], ids i64 [nq,k])."""
-        scores, ids, _ = self.search_host_async(q, k).result()
+        the device op applies q/(||q||+1e-8)) -> (scores f32 [nq,k], ids i64 [nq,k]).  `exclude`: numpy int64
+        [nq, E] ids to leave out per query (-1 = padding); short results end in (-inf, -1)."""
+        scores, ids, _ = self.search_host_async(q, k, exclude=exclude).result()
         return scores, ids
 
 
-def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int, depth: int = 3) -> PendingSearch:
+def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int, depth: int = 3, *,
+                      exclude: Optional[np.ndarray] = None) -> PendingSearch:
     """Shared host round trip of FlatIPIndex / ShardedFlatIPIndex: pinned staging buffers in a ring of `depth`
-    sets per (nq, k) so that consecutive batches overlap their copies with the previous batch's kernels."""
+    sets per (nq, k) so that consecutive batches overlap their copies with the previous batch's kernels.
+    `exclude` (numpy int64 [nq, E]) is copied to the device with the queries and passed on as `exclude=`."""
     q = np.ascontiguousarray(q, dtype=np.float32)
     if q.ndim != 2 or q.shape[1] != d:
         raise ValueError(f"expected queries [nq, {d}], got {q.shape}")
     nq = q.shape[0]
+    if exclude is not None:
+        exclude = np.ascontiguousarray(exclude, dtype=np.int64)
+        if exclude.ndim != 2 or exclude.shape[0] != nq:
+            raise ValueError(f"expected exclusions [nq={nq}, E], got {exclude.shape}")
     if nq == 0:
         empty = (np.empty((0, k), np.float32), np.empty((0, k), np.int64), 0)
         return PendingSearch(lambda: empty)
@@ -501,7 +576,10 @@ def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int
         dq = hq.to(device, non_blocking=True)
         evs[slot] = torch.cuda.Event()
         evs[slot].record(stream)
-        pending = search_async(dq, k)
+        if exclude is None:
+            pending = search_async(dq, k)
+        else:
+            pending = search_async(dq, k, exclude=torch.from_numpy(exclude).to(device))
 
     def finish():
         scores, ids, n_bad = pending.result()        # exact re-run (if any) is enqueued before the copies below
@@ -584,32 +662,62 @@ class VectorDatabase:
         print(f"Saved FAISS index to {index_path}")
 
     # -- search --------------------------------------------------------------------------------
-    def search_batch(self, query_embeddings: np.ndarray, k: int = 10) -> Tuple[np.ndarray, np.ndarray]:
-        """Array-returning retrieval: (scores f32 [nq,k'], row indices i64 [nq,k']) with k' = min(k, ntotal)."""
+    def search_batch(self, query_embeddings: np.ndarray, k: int = 10, *,
+                     exclude_rows: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """Array-returning retrieval: (scores f32 [nq,k'], row indices i64 [nq,k']) with k' = min(k, ntotal).
+        `exclude_rows` int64 [nq, E] (-1 = padding): row indices query i must not return; with fewer than k' allowed
+        rows the tail is (-inf, -1)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         k = min(k, self.index.ntotal)   # vector_db.py:159
-        return self.index.search(np.asarray(query_embeddings), k)
+        if exclude_rows is None:
+            return self.index.search(np.asarray(query_embeddings), k)
+        return self.index.search(np.asarray(query_embeddings), k, exclude=exclude_rows)
 
-    def retrieve(self, query_embedding: np.ndarray, k: int = 10) -> List[Tuple[str, float]]:
-        """vector_db.py:130-169 — descending score; only query row 0 is returned, as in the reference."""
+    def _exclude_rows(self, lists, nq: int) -> Optional[np.ndarray]:
+        """Product-id lists (one per query) -> row indices int64 [nq, E], -1 padded; unknown ids are dropped.
+        None when nothing is left to exclude."""
+        rows = [[r for r in (self.id_to_index.get(pid) for pid in ids) if r is not None and r >= 0] for ids in lists]
+        E = max((len(r) for r in rows), default=0)
+        if E == 0:
+            return None
+        out = np.full((nq, E), -1, np.int64)
+        for i, r in enumerate(rows):
+            out[i, :len(r)] = r
+        return out
+
+    def retrieve(self, query_embedding: np.ndarray, k: int = 10, *,
+                 exclude: Optional[List[str]] = None) -> List[Tuple[str, float]]:
+        """vector_db.py:130-169 — descending score; only query row 0 is returned, as in the reference.
+        `exclude`: product ids that must not be returned (e.g. the buyer's own history); unknown ids are ignored."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         query_embedding = np.asarray(query_embedding)
         if query_embedding.ndim == 1:
             query_embedding = query_embedding.reshape(1, -1)
-        scores, indices = self.search_batch(query_embedding, k)
+        if exclude is not None:
+            rows = self._exclude_rows([exclude] * query_embedding.shape[0], query_embedding.shape[0])
+            scores, indices = self.search_batch(query_embedding, k, exclude_rows=rows)
+        else:
+            scores, indices = self.search_batch(query_embedding, k)
         results = []
         for idx, score in zip(indices[0], scores[0]):
             if 0 <= idx < len(self.product_ids):
                 results.append((self.product_ids[idx], float(score)))
         return results
 
-    def retrieve_batch(self, query_embeddings: np.ndarray, k: int = 10) -> List[List[Tuple[str, float]]]:
-        """vector_db.py:171-209."""
+    def retrieve_batch(self, query_embeddings: np.ndarray, k: int = 10, *,
+                       exclude: Optional[List[List[str]]] = None) -> List[List[Tuple[str, float]]]:
+        """vector_db.py:171-209.  `exclude`: one list of product ids per query that it must not return."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
-        scores, indices = self.search_batch(query_embeddings, k)
+        if exclude is not None:
+            nq = np.asarray(query_embeddings).shape[0]
+            if len(exclude) != nq:
+                raise ValueError(f"exclude needs one list per query ({nq}), got {len(exclude)}")
+            scores, indices = self.search_batch(query_embeddings, k, exclude_rows=self._exclude_rows(exclude, nq))
+        else:
+            scores, indices = self.search_batch(query_embeddings, k)
         pids = self.product_ids
         n = len(pids)
         all_results = []
