@@ -71,10 +71,11 @@ int tt_pool_weighted(const float* x, const float* w, float* out,
 int tt_pool_weighted_gather(const float* table, int64_t N, const int64_t* idx, const float* w,
                             float* out, int B, int S, int D, void* stream);
 
-/* logits[r] = W2 . relu(W1 x_r + b1) + b2 for R rows of x at fp32 accuracy: the hidden layer runs on the tensor
- * cores as a 3xTF32 split (tcgen05 kind::tf32, error ~1e-7 absolute on O(0.1) logits) when D % 4 == 0, H <= 256,
- * R >= 128 and the pointers are 16-byte aligned, otherwise (or with TT_B200_ATTN_LOGITS=fma in the environment)
- * as fp32 FMA arithmetic on the CUDA cores.
+/* logits[r] = W2 . relu(W1 x_r + b1) + b2 for R rows of x at fp32 accuracy.  With 16-byte aligned pointers the
+ * hidden layer runs on the tensor cores: as an fp16 two-piece split (the fused pooling kernel without its pooling)
+ * when D % 64 == 0, D <= 384, H <= 128 and R >= 64, else as a 3xTF32 split (tcgen05 kind::tf32, error ~1e-7
+ * absolute on O(0.1) logits) when D % 4 == 0, H <= 256 and R >= 128.  Every other shape runs fp32 FMA arithmetic
+ * on the CUDA cores.
  * x f32 [R,D], W1 f32 [H,D], b1 f32 [H], W2 f32 [H], b2 f32 [1], logits f32 [R].
  * (buyer_tower.py:32-36 and :85-86).  For the gather path call it once over the item table
  * (R = N) and keep the result: the logit depends on the item row only. */

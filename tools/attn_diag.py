@@ -1,5 +1,4 @@
-"""Attention pooling at C2: the fused kernel vs its logits-only mode (MMA side alone) vs plain weighted pooling.
-TT_B200_ATTN_MODE selects the L2 policy of the fused kernel (bit 0 evict_last TMA loads, bit 1 bulk L2 prefetch)."""
+"""Attention pooling at C2: the fused kernel vs its logits-only mode (MMA side alone) vs plain weighted pooling."""
 import json
 import sys
 from pathlib import Path

@@ -19,4 +19,3 @@ for (R, D, H) in [(1000, 384, 128), (4096 * 50, 384, 128), (777, 100, 24), (300,
 PY
 timeout 600 python -m pytest tests/test_gpu_pool.py -q -x 2>&1 | tail -4
 timeout 300 python tools/pool_only.py 2>&1 | tail -1 | cut -c1-600
-TT_B200_ATTN_LOGITS=fma timeout 300 python tools/pool_only.py 2>&1 | tail -1 | cut -c1-600

@@ -23,10 +23,5 @@ except Exception as e:
     print("$W bench parse failed", e)
 PY
 done
-TT_B200_SHARD_PIPELINE=0 timeout 300 $TR --master-port 29531 bench.py --gpus $N --steps 20 --warmup 4 2>/dev/null | python -c "
-import sys,json
-for l in sys.stdin:
-    if l.startswith('{'):
-        r=json.loads(l); print('pipeline off: value', round(r['value']), 'e2e', round(r['e2e']['value']), 'share', round(r['roofline']['kernel_share_of_step'],3))"
 timeout 200 $TR --master-port 29541 tools/phase_times.py 2>&1 | grep -v "^W\|^\*\*\*" | tail -12 | tee $O/r02j_phase_times_n$N.log
 timeout 300 $TR --master-port 29551 bench.py --impl reference --gpus $N --steps 3 --warmup 1 2>/dev/null | tail -1 | cut -c1-600 | tee $O/r02j_reference_n$N.log

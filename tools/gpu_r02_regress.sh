@@ -11,5 +11,3 @@ for rep in 1 2; do
 (cd _r01 && timeout 300 $TR --master-port $((29560 + RANDOM % 300)) bench.py --gpus $N --steps 40 --warmup 5 2>/dev/null | python -c "$P" r01)
 timeout 300 $TR --master-port $((29560 + RANDOM % 300)) bench.py --gpus $N --steps 40 --warmup 5 2>/dev/null | python -c "$P" HEAD
 done
-TT_B200_PDL=0 timeout 300 $TR --master-port $((29560 + RANDOM % 300)) bench.py --gpus $N --steps 40 --warmup 5 2>/dev/null | python -c "$P" HEAD_nopdl
-TT_B200_SHARD_PIPELINE=0 timeout 300 $TR --master-port $((29560 + RANDOM % 300)) bench.py --gpus $N --steps 40 --warmup 5 2>/dev/null | python -c "$P" HEAD_nopipe

@@ -8,8 +8,6 @@
 // (fma.rn.f32x2, two k-partial sums per 64-bit accumulator): half the issue slots per FMA, which is
 // what the unpacked version was short of (ncu: 70 % issue utilisation, 24 % dispatch stalls at 52 % of
 // the FMA peak).
-#include <stdlib.h>
-#include <string.h>
 #include "tt_common.cuh"
 #include "flat_internal.cuh"
 
@@ -197,10 +195,8 @@ extern "C" __attribute__((visibility("default"))) int tt_attention_logits(const 
   cudaStream_t st = (cudaStream_t)stream;
   const bool fast = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0) &&
                     ((reinterpret_cast<uintptr_t>(W1) & 15) == 0);
-  // Tensor-core path (3xTF32, fp32-accurate) for aligned shapes with H <= 256; TT_B200_ATTN_LOGITS=fma keeps the
-  // CUDA-core FFMA2 kernel.
-  static const bool want_tc = [] { const char* e = getenv("TT_B200_ATTN_LOGITS"); return !(e && strcmp(e, "fma") == 0); }();
-  if (fast && want_tc && R >= 64 && R < (1LL << 31)) {
+  // Tensor-core paths (fp32-accurate) for aligned shapes; the rest runs on the CUDA cores (FFMA2 tiled, else generic).
+  if (fast && R >= 64 && R < (1LL << 31)) {
     // D % 64 == 0, D <= 384, H <= 128: the fp16 two-piece kernel of the fused pooling in its logits-only mode
     int e = launch_attn_logits_fused(x, R, D, W1, b1, W2, b2, H, logits, st);
     if (e != TT_ERR_UNSUPPORTED) return e;

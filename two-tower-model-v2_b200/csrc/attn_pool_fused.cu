@@ -24,7 +24,8 @@
 // (64 B/cycle while the tensor pipe is busy).  L2->SM traffic is x twice (TMA + pooling re-read), nothing else.
 //
 // Persistent CTAs (one per SM, 20 warps); CTA c owns a contiguous range of buyers and walks its rows in 64-row tiles:
-//   warp 0 lane 0   : TMA producer  - raw fp32 [64 rows x 64 cols] (two 128B-swizzled boxes) per K-block, 6-stage ring
+//   warp 0 lane 0   : TMA producer  - raw fp32 [64 rows x 64 cols] (two 128B-swizzled boxes) per K-block, 6-stage ring;
+//                                     with the L2 evict_last hint when pooling (the pooling warps re-read the rows)
 //   warps 8-11      : splitters     - raw fp32 -> scaled fp16 hi/lo tiles in the UMMA K-major 128B-swizzle layout
 //                                     (3-stage ring), fence.proxy.async, arrive
 //   warp 1 lane 0   : MMA issuer    - per K-block 4 K-steps x 3 MMAs (M = 128 hidden, N = 64 rows, K = 16) into the main
@@ -78,9 +79,6 @@ struct AttnFusedParams {
   int* flag;               // raised when a value leaves the fp16 range
   long long R;
   int B, S, D, H, nkb;
-  int mode;                // bit 0: TMA loads with the L2 evict_last hint; bit 1: bulk L2 prefetch of whole tiles ahead;
-                           // bits 2-4 (TT_B200_ATTN_MODE, timing experiments only, wrong results): 4 no cross MMAs,
-                           // 8 no MMAs at all, 16 no fp16 split arithmetic
 };
 
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
@@ -164,34 +162,16 @@ attn_pool_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const AttnFus
   if (warp == 0) {
     // =========================== TMA producer =====================================================
     if (lane == 0) {
-      // The boxes below are 128-byte segments at a 1536-byte stride and every row comes back nkb times: fetched from
-      // DRAM that way the stream ran at ~2.6 TB/s (r01 tf32 kernel and the first version of this one alike).  Rows of
-      // a tile are contiguous in memory, so the producer first asks L2 for whole tiles (plain contiguous bulk
-      // prefetches, a few tiles ahead): DRAM sees sequential 96 KB bursts, the boxes and the pooling re-read hit L2.
-      const bool l2_keep = (p.mode & 1) != 0, l2_prefetch = (p.mode & 2) != 0;
-      constexpr int PF_AHEAD = 3;
-      auto prefetch_tile = [&](int t) {
-        if (!l2_prefetch) return;
-        const long long rr = r0 + (long long)t * AF_TILE;
-        long long nbytes = ((rr + AF_TILE <= p.R) ? (long long)AF_TILE : (p.R - rr)) * p.D * 4;
-        const char* src = reinterpret_cast<const char*>(p.x + rr * p.D);
-        for (long long off = 0; off < nbytes; off += 16384) {
-          const unsigned int sz = (unsigned int)((nbytes - off < 16384) ? (nbytes - off) : 16384);
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src + off), "r"(sz) : "memory");
-        }
-      };
-      for (int t = 0; t < PF_AHEAD && t < ntiles; ++t) prefetch_tile(t);
       int stage = 0;
       uint32_t phase = 0;
       for (int t = 0; t < ntiles; ++t) {
-        if (t + PF_AHEAD < ntiles) prefetch_tile(t + PF_AHEAD);
         const int row = (int)(r0 + (long long)t * AF_TILE);
         for (int kb = 0; kb < nkb; ++kb) {
           mbar_wait(smem_u32(empty_raw + stage), phase ^ 1, 500 + stage);
           const uint32_t fb = smem_u32(full_raw + stage);
           const uint32_t dst = smem_u32(raw_ring + (size_t)stage * AF_RAW_STAGE);
           mbar_arrive_expect_tx(fb, (uint32_t)AF_RAW_STAGE);
-          if (l2_keep) {      // the rows are read again by the pooling warps: ask L2 to keep them (evict_last)
+          if (POOL) {         // the rows are read again by the pooling warps: ask L2 to keep them (evict_last)
             tma_load_2d_hint(dst, &tmap_x, fb, kb * 64, row, kEvictLast);
             tma_load_2d_hint(dst + AF_RAW_STAGE / 2, &tmap_x, fb, kb * 64 + 32, row, kEvictLast);
           } else {
@@ -226,9 +206,9 @@ attn_pool_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const AttnFus
             const uint32_t a_hi = tmem_base + w_hi_col + (uint32_t)((kb * 4 + k) * 8);
             const uint32_t a_lo = tmem_base + w_lo_col + (uint32_t)((kb * 4 + k) * 8);
             const uint32_t first = (uint32_t)((kb | k) != 0);
-            if (!(p.mode & 8)) mma_f16_ts(d_main, a_hi, xh + koff, idesc, first);                 // hi.hi   -> main accumulator
-            if (!(p.mode & 12)) mma_f16_ts(d_cross, a_lo, xh + koff, idesc, first);                // lo_w.hi_x
-            if (!(p.mode & 12)) mma_f16_ts(d_cross, a_hi, xl + koff, idesc, 1u);                   // hi_w.lo_x -> cross accumulator
+            mma_f16_ts(d_main, a_hi, xh + koff, idesc, first);                 // hi.hi   -> main accumulator
+            mma_f16_ts(d_cross, a_lo, xh + koff, idesc, first);                // lo_w.hi_x
+            mma_f16_ts(d_cross, a_hi, xl + koff, idesc, 1u);                   // hi_w.lo_x -> cross accumulator
           }
           mma_commit(smem_u32(empty_b + stage));
           if (kb == nkb - 1) mma_commit(smem_u32(tmem_full));
@@ -350,8 +330,8 @@ attn_pool_fused_kernel(const __grid_constant__ CUtensorMap tmap_x, const AttnFus
       uint8_t* lo_tile = hi_tile + AF_B_STAGE / 2;
 #pragma unroll
       for (int i = 0; i < UPT; ++i) {
-        uint4 hi = make_uint4(0, 0, 0, 0), lo = hi;
-        if (!(p.mode & 16)) split8(fa[i], fb[i], hi, lo, mabs);
+        uint4 hi, lo;
+        split8(fa[i], fb[i], hi, lo, mabs);
         *reinterpret_cast<uint4*>(hi_tile + row[i] * 128 + cpos[i]) = hi;
         *reinterpret_cast<uint4*>(lo_tile + row[i] * 128 + cpos[i]) = lo;
       }
@@ -572,11 +552,6 @@ attn_pool_fallback_kernel(const float* __restrict__ x, const float* __restrict__
   }
 }
 
-static int fused_mode() {
-  static const int m = [] { const char* e = getenv("TT_B200_ATTN_MODE"); return e ? atoi(e) : 1; }();
-  return m;
-}
-
 struct FusedWs { size_t wp, meta, total; };
 static FusedWs fused_ws_layout(int nkb) {
   FusedWs w{};
@@ -592,7 +567,8 @@ static bool fused_shape_ok(const float* x, const float* out, long long B, long l
 }
 
 // Logits-only mode (tt_attention_logits; e.g. once over the whole catalog for the gather path): the same kernel without
-// the pooling warps, logits written to global memory; the weight pieces live in a stream-ordered scratch block.
+// the pooling warps, logits written to global memory; the weight pieces live in a stream-ordered scratch block.  Nothing
+// re-reads the rows, so the TMA loads carry no L2 evict_last hint.
 int launch_attn_logits_fused(const float* x, long long R, int D, const float* W1, const float* b1, const float* W2,
                              const float* b2, int H, float* logits, cudaStream_t st) {
   if (!(D % 64 == 0 && D <= 64 * AF_MAX_KB && H >= 1 && H <= AF_M && R >= 64 && R < (1LL << 31) &&
@@ -617,7 +593,6 @@ int launch_attn_logits_fused(const float* x, long long R, int D, const float* W1
     AttnFusedParams p{};
     p.x = x; p.logits_out = logits; p.Wp = Wp; p.b1 = b1; p.W2 = W2; p.b2 = b2; p.inv_scale = inv_scale; p.flag = flag;
     p.R = R; p.B = (int)R; p.S = 1; p.D = D; p.H = H; p.nkb = nkb;
-    p.mode = fused_mode() & ~3;      // (diagnostic bits only)
     const size_t smem = (size_t)AF_RAW_STAGES * AF_RAW_STAGE + (size_t)AF_B_STAGES * AF_B_STAGE + AF_RMAX * sizeof(float) +
                         2 * 4 * AF_TILE * sizeof(float) + 512 + 1024;
     const long long tiles = (R + AF_TILE - 1) / AF_TILE;
@@ -683,7 +658,6 @@ extern "C" __attribute__((visibility("default"))) int tt_pool_attention_fused(co
     p.x = x + bdone * S * D; p.w = w + bdone * S; p.out = out + bdone * D; p.Wp = Wp;
     p.b1 = b1; p.W2 = W2; p.b2 = b2; p.inv_scale = inv_scale; p.flag = flag;
     p.R = nb * S; p.B = (int)nb; p.S = S; p.D = D; p.H = H; p.nkb = nkb;
-    p.mode = fused_mode();
     const int grid = (int)(nb < sms ? nb : sms);
     // programmatic dependent launch: the x stream (TMA, splitters) starts under the weight-preparation kernel's tail;
     // only the epilogue warps (W1 pieces, scale) and the flag wait for it.  The preparation kernel itself is a plain

@@ -447,21 +447,14 @@ __device__ __forceinline__ float warp_select_rounds(float* v, int n, int r, floa
 constexpr int SEL_WQ = 8;   // queries (warps) per CTA
 __global__ void __launch_bounds__(SEL_WQ * 32)
 select_threshold_tile_kernel(const float* __restrict__ sample, int slots, int ld, int nq, int r, float* __restrict__ thr,
-                             float* __restrict__ topr, int topr_ld, int query_major) {
+                             float* __restrict__ topr, int topr_ld) {
   pdl_trigger();
   pdl_wait();
   extern __shared__ float sv[];   // [SEL_WQ][slots]
   const int q0 = blockIdx.x * SEL_WQ;
-  if (query_major) {              // chunk maxima: sample[q][slots] (value index fastest)
-    for (int e = threadIdx.x; e < slots * SEL_WQ; e += blockDim.x) {
-      const int qq = e / slots, i = e % slots;
-      sv[e] = (q0 + qq < nq) ? sample[(size_t)(q0 + qq) * slots + i] : -INFINITY;
-    }
-  } else {                        // tile maxima: sample[slot][ld] (query fastest)
-    for (int e = threadIdx.x; e < slots * SEL_WQ; e += blockDim.x) {
-      const int i = e / SEL_WQ, qq = e % SEL_WQ;
-      sv[qq * slots + i] = (q0 + qq < ld) ? sample[(size_t)i * ld + q0 + qq] : -INFINITY;
-    }
+  for (int e = threadIdx.x; e < slots * SEL_WQ; e += blockDim.x) {      // tile maxima: sample[slot][ld] (query fastest)
+    const int i = e / SEL_WQ, qq = e % SEL_WQ;
+    sv[qq * slots + i] = (q0 + qq < ld) ? sample[(size_t)i * ld + q0 + qq] : -INFINITY;
   }
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -821,7 +814,7 @@ static int launch_scan_t(const CUtensorMap& tq, const CUtensorMap& tx, const Sca
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 2;
   count_launch();
   TT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, tq, tx, sp));
   return TT_OK;
@@ -856,9 +849,8 @@ static int make_scan_params(const ScanPlan& pl, const void* qh, const void* Xh, 
 // 1M x 384: 150.4 vs 155.2 us per step at nq = 1; at nq = 4 the four selections in a row delay the first epilogue
 // enough to stall the MMAs (174.9 vs 158.3 us), so larger batches keep the separate kernel.
 static bool fold_select(const ScanPlan& pl, int nq) {
-  static const bool on = [] { const char* e = getenv("TT_B200_FOLD_SELECT"); return !(e && e[0] == '0'); }();
   const int nvals = pl.sample_tile_max ? pl.sample_slots : pl.sample_slots * CHUNKS;
-  return on && nq == 1 && !pl.pair && pl.nqu == 1 && nvals <= 4096;
+  return nq == 1 && !pl.pair && pl.nqu == 1 && nvals <= 4096;
 }
 
 int launch_sample(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr, float* topr,
@@ -885,20 +877,11 @@ int launch_sample(const ScanPlan& pl, const void* qh, const void* Xh, long long 
     TT_CHECK_CUDA(cudaFuncSetAttribute(select_threshold_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
     TT_CHECK_CUDA(launch_pdl(select_threshold_tile_kernel, dim3((nq + SEL_WQ - 1) / SEL_WQ), dim3(SEL_WQ * 32), sm, st,
                              (const float*)sample_buf, pl.sample_slots, pl.nq_pad, nq,
-                             topr ? min(pl.sample_rank, SHARD_TOPR) : pl.sample_rank, thr, topr, (int)SHARD_TOPR, 0));
+                             topr ? min(pl.sample_rank, SHARD_TOPR) : pl.sample_rank, thr, topr, (int)SHARD_TOPR));
   } else {
+    // chunk maxima: more than 4096 values per query (up to 4096 took the radix select above)
     TT_CHECK_ARG(topr == nullptr, "top-r lists need the tile sampling mode");
     const int nvals = pl.sample_slots * CHUNKS;
-    if (nvals <= 4096 && pl.sample_rank <= 64) {
-      // few values, small rank: one warp per query (r rounds of warp arg-max over register-cached values) instead of a
-      // CTA per query with two block barriers per round (9.7 us at nq = 1, 1M x 384)
-      const size_t smw = (size_t)nvals * SEL_WQ * sizeof(float);
-      TT_CHECK_CUDA(cudaFuncSetAttribute(select_threshold_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smw));
-      TT_CHECK_CUDA(launch_pdl(select_threshold_tile_kernel, dim3((nq + SEL_WQ - 1) / SEL_WQ), dim3(SEL_WQ * 32), smw, st,
-                               (const float*)sample_buf, nvals, pl.nq_pad, nq, pl.sample_rank, thr, (float*)nullptr, 0, 1));
-      TT_CHECK_LAUNCH();
-      return TT_OK;
-    }
     int npad = 1;
     while (npad < nvals) npad <<= 1;
     const size_t sm = (size_t)npad * sizeof(float);

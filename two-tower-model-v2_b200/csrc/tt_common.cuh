@@ -57,12 +57,8 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 // serialization attribute, calls pdl_trigger() first thing (its successor may be scheduled as soon as every CTA of
 // this grid has started) and pdl_wait() before it touches global memory (returns once the predecessor grid has
 // completed and its writes are visible).  The successor's launch latency and prologue (barrier init, TMEM
-// allocation, descriptor prefetch) then hide under the predecessor's tail.  TT_B200_PDL=0 disables the attribute
-// (the device-side instructions are no-ops without it).
-inline bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("TT_B200_PDL"); return !(e && e[0] == '0'); }();
-  return on;
-}
+// allocation, descriptor prefetch) then hide under the predecessor's tail.  The device-side instructions are no-ops
+// in a kernel launched without the attribute.
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
   cudaLaunchConfig_t cfg{};
@@ -74,7 +70,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 

@@ -258,7 +258,6 @@ class ShardedFlatIPIndex:
         # "auto" tries p2p on CUDA and falls back to nccl if the IPC set-up fails.
         self.exchange = os.environ.get("TT_B200_EXCHANGE", exchange)
         self.exchange_used = None
-        self.pipelined = os.environ.get("TT_B200_SHARD_PIPELINE", "1") != "0"
         self._inflight = []
 
     @property
@@ -414,7 +413,7 @@ class ShardedFlatIPIndex:
         k_local = min(k, self.local.ntotal)
         p2p = self._p2p_for(nq, k, q.device, world, lay)
         global_thr = self._global_threshold(world, nq, k, exclude)
-        if p2p is not None and global_thr and self.pipelined:
+        if p2p is not None and global_thr:
             return self._search_pipelined(q, k, nq, world, lay, rec, p2p, exclude)
         self.flush()          # never interleave the two schedules
         views = record_views(rec, lay, nq, k)
