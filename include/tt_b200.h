@@ -229,6 +229,34 @@ int tt_flat_search_exact_excl(const float* q, int nq, const int32_t* qsel, int n
                               float* scores, int64_t* ids, const int64_t* excl, int E,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* Label filters: the exact top-K over the rows whose label word satisfies the query's masks (e.g. "in stock", "in
+ * category X or Y").
+ *   labels  u32 [N]       one word per row, 16-byte aligned; the bits mean whatever the caller assigns
+ *   require u32 [nq, 2]   {all, any} per query, 8-byte aligned.  Row r is ALLOWED for query q iff
+ *                             (labels[r] & all) == all  and  (any == 0 or (labels[r] & any) != 0)
+ *                         so {0, 0} allows every row.
+ * Both must be non-NULL (the unfiltered calls are tt_flat_search / tt_flat_search_excl).  Filters compose with the
+ * exclusion lists above: the result is the exact fp32 top-K over rows that are allowed and not listed, ordered as
+ * above, with a (-inf, -1) tail when fewer than K such rows exist.  A disallowed row never appears in an output.
+ * Disallowed rows never reach the scan's sample or threshold test, so the sampled threshold is a lower bound of the
+ * allowed rows' scores and the certificate reads over allowed rows: "every allowed row not rescored scores below the
+ * bound".  The plan does not depend on the filter: the workspace is tt_flat_search_excl_workspace_bytes(N, D, nq, K,
+ * E) (E = 0 without a list).  tt_flat_search_exact_filtered reads the masks (and the list) of the QUERY row qsel[i];
+ * an uncertified query is re-run there with the same masks.  Single-device calls only: the shard entry points take
+ * no filter. */
+int tt_flat_search_filtered(const float* q, int nq,
+                            const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
+                            int K, int64_t id_offset,
+                            float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified,
+                            const uint32_t* labels, const uint32_t* require,
+                            const int64_t* excl, int E,
+                            void* workspace, size_t workspace_bytes, void* stream);
+int tt_flat_search_exact_filtered(const float* q, int nq, const int32_t* qsel, int nsel,
+                                  const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                                  float* scores, int64_t* ids, const uint32_t* labels, const uint32_t* require,
+                                  const int64_t* excl, int E,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+
 /* Merge G per-shard sorted top-K lists into one: scores_g f32 [G, nq, K], ids_g i64 [G, nq, K]
  * (the layout an all-gather of per-rank [nq,K] results produces) -> [nq, K], same ordering
  * (score descending, id ascending). */

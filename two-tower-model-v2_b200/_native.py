@@ -63,6 +63,12 @@ SIGNATURES = {
                                           c_void_p, c_size_t, c_void_p]),
     "tt_flat_search_exact_excl": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int64,
                                           c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_search_filtered": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64,
+                                        c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                        c_void_p, c_size_t, c_void_p]),
+    "tt_flat_search_exact_filtered": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int64,
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
+                                              c_void_p]),
     "tt_flat_shard_plan_ok":(c_int, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_sample": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p,

@@ -97,7 +97,7 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_excl_wor
 static int flat_search_impl(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
                             int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
                             int32_t* flags, int32_t* n_uncertified, float* bound, const int64_t* excl, int E,
-                            void* workspace, size_t workspace_bytes, void* stream) {
+                            void* workspace, size_t workspace_bytes, void* stream, const LabelArgs& lab = LabelArgs{}) {
   TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
   TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   TT_CHECK_ARG(q && Xn && Xh && stats && scores && ids && flags && n_uncertified, "null pointer");
@@ -122,6 +122,9 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
       fill_int_kernel<<<(nq + 255) / 256, 256, 0, st>>>(reinterpret_cast<int*>(bound), nq, (int)0xff800000);
       TT_CHECK_LAUNCH();
     }
+    if (lab.labels)
+      return tt_flat_search_exact_filtered(q, nq, nullptr, nq, Xn, N, D, K, id_offset, scores, ids, lab.labels, lab.require,
+                                           excl, E, workspace, workspace_bytes, stream);
     return tt_flat_search_exact_excl(q, nq, nullptr, nq, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
                                      workspace_bytes, stream);
   }
@@ -138,7 +141,7 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
   float* sample = reinterpret_cast<float*>(ws + w.sample);
 
   if (int e = launch_prep_queries(q, nq, pl.nq_pad, D, pl.Dp, stats, qn, qh, eps, n_uncertified, st)) return e;
-  if (int e = launch_scan(pl, qh, Xh, N, nq, thr, cnt, cand, sample, st)) return e;
+  if (int e = launch_scan(pl, qh, Xh, N, nq, thr, cnt, cand, sample, st, lab)) return e;
   return launch_finalize(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, cnt, cand, scores,
                          reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st,
                          reinterpret_cast<const long long*>(excl), E);
@@ -158,6 +161,21 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_excl(const 
                                    void* workspace, size_t workspace_bytes, void* stream) {
   return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
                           excl, E, workspace, workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_filtered(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
+                                       int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
+                                       int32_t* flags, int32_t* n_uncertified, const uint32_t* labels,
+                                       const uint32_t* require, const int64_t* excl, int E, void* workspace,
+                                       size_t workspace_bytes, void* stream) {
+  TT_CHECK_ARG(labels != nullptr && require != nullptr, "null labels or require (the unfiltered call is tt_flat_search_excl)");
+  TT_CHECK_ARG((reinterpret_cast<uintptr_t>(labels) & 15) == 0, "labels must be 16-byte aligned");
+  TT_CHECK_ARG((reinterpret_cast<uintptr_t>(require) & 7) == 0, "require must be 8-byte aligned");
+  LabelArgs lab;
+  lab.labels = labels;
+  lab.require = require;
+  return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
+                          excl, E, workspace, workspace_bytes, stream, lab);
 }
 
 extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,

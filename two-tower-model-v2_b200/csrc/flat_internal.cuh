@@ -32,21 +32,30 @@ struct ScanPlan {
 
 ScanPlan make_scan_plan(long long N, int D, int nq, int K);
 
+// Label filter of a search (tt_flat_search_filtered): labels u32 [N] (16-byte aligned), require u32 [nq, 2] = {all,
+// any}.  Both NULL = the unfiltered scan.
+struct LabelArgs {
+  const uint32_t* labels = nullptr;
+  const uint32_t* require = nullptr;
+};
+
 // zero_me (may be NULL): an int the kernel sets to 0 (the call's n_uncertified counter)
 int launch_prep_queries(const float* q, int nq, int nq_pad, int D, int Dp, const float* stats,
                         float* qn, void* qh, float* eps, int* zero_me, cudaStream_t st);
 
 // sample pass (if plan.use_threshold) + threshold selection + main scan
 int launch_scan(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq,
-                float* thr, unsigned int* seg_cnt, void* cand, float* sample_buf, cudaStream_t st);
+                float* thr, unsigned int* seg_cnt, void* cand, float* sample_buf, cudaStream_t st,
+                const LabelArgs& lab = LabelArgs{});
 
 // the pieces launch_scan is made of (the sharded path runs them with an exchange in between)
 ScanPlan make_shard_plan(long long N_local, long long N_total, int D, int nq, int K, bool* global_ok);
 int launch_sample(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr, float* topr,
-                  float* sample_buf, cudaStream_t st, bool skip_select = false);
+                  float* sample_buf, cudaStream_t st, bool skip_select = false, const LabelArgs& lab = LabelArgs{});
 int launch_select_gathered(const float* topr_g, int G, int nq, int r, float* thr, int* zero_me, cudaStream_t st);
 int launch_main_scan(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr,
-                     unsigned int* seg_cnt, void* cand, cudaStream_t st, const float* sel_sample = nullptr);
+                     unsigned int* seg_cnt, void* cand, cudaStream_t st, const float* sel_sample = nullptr,
+                     const LabelArgs& lab = LabelArgs{});
 
 // fp32 rescoring of every candidate, exact sort, certificate; excl i64 [nq, E] (E > 0) drops the listed rows
 int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,

@@ -37,7 +37,15 @@
 //            scores of distinct rows, so the threshold is a guaranteed lower bound of the r-th best
 //            bf16 score of the whole catalog.
 //   MAIN   : scan every tile, append scores >= threshold.
+//
+// FILTER instances (per-row label words, per-query masks; tt_flat_search_filtered) turn every accumulator column whose
+// row the query does not allow into -inf before the maximum and the threshold test, in both passes.  The sampled
+// maxima are then maxima of allowed rows, so the threshold is a lower bound of the r-th best ALLOWED score and the
+// certificate of the finalize kernel holds over allowed rows unchanged.  The threshold these instances compare against
+// is max(thr, -FLT_MAX): it is -inf on the every-row-a-candidate route and for a query whose sample holds fewer allowed
+// maxima than the rank, and -inf >= -inf would append masked columns.
 #include <cuda.h>
+#include <float.h>
 #include <math.h>
 #include "tt_common.cuh"
 #include "sm100_ptx.cuh"
@@ -48,10 +56,10 @@ namespace tt {
 
 using namespace ptx;
 
-template <int BLOCK_M, bool SAMPLE, bool PAIR>
+template <int BLOCK_M, bool SAMPLE, bool PAIR, bool FILTER>
 __global__ void __launch_bounds__(SCAN_THREADS, 1)
 flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
-                 const ScanParams p) {
+                 const std::conditional_t<FILTER, FilterScanParams, ScanParams> p) {
   constexpr int A_KB_BYTES = BLOCK_M * BLOCK_K * 2;
   constexpr int B_ROWS = PAIR ? BLOCK_N / 2 : BLOCK_N;            // rows of a tile this CTA loads
   constexpr int B_STAGE_BYTES = B_ROWS * BLOCK_K * 2;
@@ -198,13 +206,15 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
     const bool valid = (q_local >= 0) && (q < p.nq);
 
     float thr = INFINITY;
+    LabelFilter flt{0u, 0u, 1u};                       // FILTER: this query's masks (padding lanes allow every row)
+    if constexpr (FILTER) { if (valid) flt = make_label_filter(__ldg(p.require + q)); }
     if (!SAMPLE) {
       if (p.sel_n > 0) {
         // batch of one: no separate selection kernel - the 128 epilogue threads pick the threshold from the sampled
         // maxima while the producer and the MMA warp already stream the first tile
         uint32_t* sel_tmp = reinterpret_cast<uint32_t*>(bars) + 48;      // two free words of the barrier block
         for (int qq = 0; qq < p.nq; ++qq) {
-          const float t = epilogue_select(p.sel_sample, p.sel_n, p.sel_ld, qq, p.sel_query_major, p.sel_rank, scratch_base,
+          const float t = epilogue_select<FILTER>(p.sel_sample, p.sel_n, p.sel_ld, qq, p.sel_query_major, p.sel_rank, scratch_base,
                                           sel_tmp, (int)threadIdx.x - 128);
           if (q == qq) thr = t;
         }
@@ -213,6 +223,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
       } else if (valid) {
         thr = __ldg(p.thr + q);
       }
+      if (FILTER) thr = fmaxf(thr, -FLT_MAX);
     }
     uint2* my_cand = SAMPLE ? nullptr : (p.cand + ((size_t)(valid ? q : 0) * p.nslices + slice) * p.seg_cap);
     unsigned int my_cnt = 0;
@@ -224,6 +235,9 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
       const int slot = slice + t * p.nslices;
       const long long row0 = (long long)slot * p.tile_stride * BLOCK_N;
       const int ncols = (int)min((long long)BLOCK_N, p.N - row0);   // last tile may be partial
+      if constexpr (FILTER) {   // the tile's label words into L1 while the MMAs run
+        if (lane < CHUNKS && lane * 32 < ncols) asm volatile("prefetch.global.L1 [%0];" :: "l"(p.labels + row0 + lane * 32));
+      }
       mbar_wait(smem_u32(tmem_full_bar + buf), use_phase, 300 + buf);
       tc_fence_after();
       const uint32_t taddr0 = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(buf * BLOCK_N);
@@ -294,6 +308,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
           __syncwarp();
           tmem_ld_32x32(taddr0 + (uint32_t)(c * 32 + 64), b0);
           tmem_ld_32x32(taddr0 + (uint32_t)(c * 32 + 96), b1);
+          if constexpr (FILTER) { mask_columns32(a0, p.labels + row0 + c * 32, flt); mask_columns32(a1, p.labels + row0 + c * 32 + 32, flt); }
           consume(a0, a1, c);
           tmem_ld_wait();
           if (c + 4 < CHUNKS) {
@@ -301,6 +316,7 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
             tmem_ld_32x32(taddr0 + (uint32_t)(c * 32 + 128), a0);
             tmem_ld_32x32(taddr0 + (uint32_t)(c * 32 + 160), a1);
           }
+          if constexpr (FILTER) { mask_columns32(b0, p.labels + row0 + c * 32 + 64, flt); mask_columns32(b1, p.labels + row0 + c * 32 + 96, flt); }
           consume(b0, b1, c + 2);
         }
         if (SAMPLE && p.sample_tile_max && q_local >= 0)
@@ -311,14 +327,20 @@ flat_scan_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_consta
           float tile_max = -INFINITY;
           for (int c = 0; c < CHUNKS; ++c) {
             const int limit = min(32, ncols - c * 32);
-            const float m = (limit > 0) ? max_columns(taddr0 + (uint32_t)(c * 32), limit) : -INFINITY;
+            float m;
+            if constexpr (FILTER)
+              m = (limit > 0) ? max_columns_filtered(taddr0 + (uint32_t)(c * 32), limit, (uint32_t)row0 + (uint32_t)(c * 32), p.labels, flt)
+                              : -INFINITY;
+            else
+              m = (limit > 0) ? max_columns(taddr0 + (uint32_t)(c * 32), limit) : -INFINITY;
             if (p.sample_tile_max) tile_max = fmaxf(tile_max, m);
             else if (valid) sample_row[c] = m;
           }
           if (p.sample_tile_max && q_local >= 0)
             p.sample_out[(size_t)slot * p.sample_ld + (size_t)(qb * BLOCK_M + q_local)] = tile_max;
         } else {
-          append_columns(taddr0, ncols, thr, (uint32_t)row0, my_cand, my_cnt, (unsigned int)p.seg_cap);
+          if constexpr (FILTER) append_columns_filtered(taddr0, ncols, thr, (uint32_t)row0, my_cand, my_cnt, (unsigned int)p.seg_cap, p.labels, flt);
+          else append_columns(taddr0, ncols, thr, (uint32_t)row0, my_cand, my_cnt, (unsigned int)p.seg_cap);
         }
       }
       // release this accumulator buffer to the MMA issuer (on the leader CTA)
@@ -796,10 +818,11 @@ ScanPlan make_scan_plan(long long N, int D, int nq, int K) {
   return pl;
 }
 
-template <int BLOCK_M, bool SAMPLE, bool PAIR>
-static int launch_scan_t(const CUtensorMap& tq, const CUtensorMap& tx, const ScanParams& sp, int units, size_t smem,
+template <int BLOCK_M, bool SAMPLE, bool PAIR, bool FILTER>
+static int launch_scan_t(const CUtensorMap& tq, const CUtensorMap& tx, const FilterScanParams& fsp, int units, size_t smem,
                          cudaStream_t st) {
-  auto kern = flat_scan_kernel<BLOCK_M, SAMPLE, PAIR>;
+  const std::conditional_t<FILTER, FilterScanParams, ScanParams>& sp = fsp;
+  auto kern = flat_scan_kernel<BLOCK_M, SAMPLE, PAIR, FILTER>;
   TT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)(PAIR ? 2 * units : units));
@@ -820,26 +843,36 @@ static int launch_scan_t(const CUtensorMap& tq, const CUtensorMap& tx, const Sca
   return TT_OK;
 }
 
+template <bool SAMPLE, bool FILTER>
+static int launch_scan_tiling(const ScanPlan& pl, const CUtensorMap& tq, const CUtensorMap& tx, const FilterScanParams& sp,
+                              int units, cudaStream_t st) {
+  if (pl.pair) return launch_scan_t<128, SAMPLE, true, FILTER>(tq, tx, sp, units, pl.smem_bytes, st);
+  if (pl.block_m == 128) return launch_scan_t<128, SAMPLE, false, FILTER>(tq, tx, sp, units, pl.smem_bytes, st);
+  return launch_scan_t<64, SAMPLE, false, FILTER>(tq, tx, sp, units, pl.smem_bytes, st);
+}
+
+// the FILTER instances run when the call has label words
 template <bool SAMPLE>
-static int launch_scan_mode(const ScanPlan& pl, const CUtensorMap& tq, const CUtensorMap& tx, const ScanParams& sp,
+static int launch_scan_mode(const ScanPlan& pl, const CUtensorMap& tq, const CUtensorMap& tx, const FilterScanParams& sp,
                             int units, cudaStream_t st) {
-  if (pl.pair) return launch_scan_t<128, SAMPLE, true>(tq, tx, sp, units, pl.smem_bytes, st);
-  if (pl.block_m == 128) return launch_scan_t<128, SAMPLE, false>(tq, tx, sp, units, pl.smem_bytes, st);
-  return launch_scan_t<64, SAMPLE, false>(tq, tx, sp, units, pl.smem_bytes, st);
+  return sp.labels ? launch_scan_tiling<SAMPLE, true>(pl, tq, tx, sp, units, st)
+                   : launch_scan_tiling<SAMPLE, false>(pl, tq, tx, sp, units, st);
 }
 
 static int make_scan_params(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr,
-                            unsigned int* seg_cnt, void* cand, float* sample_buf, CUtensorMap* tq, CUtensorMap* tx,
-                            ScanParams* sp) {
+                            unsigned int* seg_cnt, void* cand, float* sample_buf, const LabelArgs& lab, CUtensorMap* tq,
+                            CUtensorMap* tx, FilterScanParams* sp) {
   if (int e = make_tmap_bf16(tq, qh, pl.nq_pad, pl.Dp, pl.block_m)) return e;
   if (int e = make_tmap_bf16(tx, Xh, N, pl.Dp, pl.pair ? BLOCK_N / 2 : BLOCK_N)) return e;
-  *sp = ScanParams{};
+  *sp = FilterScanParams{};
   sp->N = N; sp->nq = nq; sp->num_kb = pl.num_kb; sp->num_stages = pl.num_stages; sp->nqu = pl.nqu;
   sp->num_kb_res = pl.num_kb_res; sp->stage_bytes = pl.stage_bytes;
   sp->thr = thr; sp->seg_cnt = seg_cnt; sp->cand = reinterpret_cast<uint2*>(cand); sp->seg_cap = pl.seg_cap;
   sp->sample_out = sample_buf;
   sp->sample_tile_max = pl.sample_tile_max ? 1 : 0;
   sp->sample_ld = pl.nq_pad;
+  sp->labels = lab.labels;
+  sp->require = reinterpret_cast<const uint2*>(lab.require);
   return TT_OK;
 }
 
@@ -854,10 +887,10 @@ static bool fold_select(const ScanPlan& pl, int nq) {
 }
 
 int launch_sample(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr, float* topr,
-                  float* sample_buf, cudaStream_t st, bool skip_select) {
+                  float* sample_buf, cudaStream_t st, bool skip_select, const LabelArgs& lab) {
   CUtensorMap tq, tx;
-  ScanParams sp;
-  if (int e = make_scan_params(pl, qh, Xh, N, nq, thr, nullptr, nullptr, sample_buf, &tq, &tx, &sp)) return e;
+  FilterScanParams sp;
+  if (int e = make_scan_params(pl, qh, Xh, N, nq, thr, nullptr, nullptr, sample_buf, lab, &tq, &tx, &sp)) return e;
   sp.num_slots = pl.sample_slots; sp.tile_stride = pl.sample_stride; sp.nslices = pl.sample_slices;
   if (int e = launch_scan_mode<true>(pl, tq, tx, sp, pl.sample_slices * pl.nqu, st)) return e;
   if (skip_select) return TT_OK;
@@ -902,10 +935,10 @@ int launch_select_gathered(const float* topr_g, int G, int nq, int r, float* thr
 }
 
 int launch_main_scan(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq, float* thr,
-                     unsigned int* seg_cnt, void* cand, cudaStream_t st, const float* sel_sample) {
+                     unsigned int* seg_cnt, void* cand, cudaStream_t st, const float* sel_sample, const LabelArgs& lab) {
   CUtensorMap tq, tx;
-  ScanParams sp;
-  if (int e = make_scan_params(pl, qh, Xh, N, nq, thr, seg_cnt, cand, nullptr, &tq, &tx, &sp)) return e;
+  FilterScanParams sp;
+  if (int e = make_scan_params(pl, qh, Xh, N, nq, thr, seg_cnt, cand, nullptr, lab, &tq, &tx, &sp)) return e;
   sp.num_slots = pl.num_tiles; sp.tile_stride = 1; sp.nslices = pl.main_slices;
   if (sel_sample) {       // thresholds selected in the kernel's prologue from the sample pass's maxima
     sp.sel_sample = sel_sample; sp.thr_out = thr;
@@ -919,16 +952,16 @@ int launch_main_scan(const ScanPlan& pl, const void* qh, const void* Xh, long lo
 }
 
 int launch_scan(const ScanPlan& pl, const void* qh, const void* Xh, long long N, int nq,
-                float* thr, unsigned int* seg_cnt, void* cand, float* sample_buf, cudaStream_t st) {
+                float* thr, unsigned int* seg_cnt, void* cand, float* sample_buf, cudaStream_t st, const LabelArgs& lab) {
   bool fold = false;
   if (pl.use_threshold) {
     fold = fold_select(pl, nq);
-    if (int e = launch_sample(pl, qh, Xh, N, nq, thr, nullptr, sample_buf, st, fold)) return e;
+    if (int e = launch_sample(pl, qh, Xh, N, nq, thr, nullptr, sample_buf, st, fold, lab)) return e;
   } else {
     count_launch();
     TT_CHECK_CUDA(launch_pdl(fill_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, thr, nq, -INFINITY));
   }
-  return launch_main_scan(pl, qh, Xh, N, nq, thr, seg_cnt, cand, st, fold ? sample_buf : nullptr);
+  return launch_main_scan(pl, qh, Xh, N, nq, thr, seg_cnt, cand, st, fold ? sample_buf : nullptr, lab);
 }
 
 // Plan of one shard of a catalog of N_total rows: tiling and slicing follow the shard, the sampling

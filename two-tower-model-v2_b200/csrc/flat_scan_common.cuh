@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda.h>
 #include <math.h>
+#include <type_traits>
 #include "tt_common.cuh"
 #include "sm100_ptx.cuh"
 #include "flat_internal.cuh"
@@ -50,6 +51,39 @@ struct ScanParams {
   int sample_ld;          // tile mode: leading dimension (nq_pad)
 };
 
+// Parameters of the FILTER instances (both passes): row r is allowed for query q iff
+// make_label_filter(require[q]).allows(labels[r]).  A separate type, so that the unfiltered instances keep theirs.
+struct FilterScanParams : ScanParams {
+  const uint32_t* labels;   // [N], 16-byte aligned
+  const uint2* require;     // [nq] {all, any}
+};
+
+// The label filter of one query: (label & all) == all, and (label & any) != 0 unless any == 0.  any_free = 1 when
+// any == 0, so that the second test passes for every label, 0 included.
+struct LabelFilter {
+  uint32_t all, any, any_free;
+  __device__ __forceinline__ bool allows(uint32_t label) const {
+    return ((label & all) == all) && (((label & any) | any_free) != 0u);
+  }
+};
+__device__ __forceinline__ LabelFilter make_label_filter(uint2 req) {
+  return LabelFilter{req.x, req.y, req.y == 0u ? 1u : 0u};
+}
+constexpr uint32_t NEG_INF_BITS = 0xff800000u;
+
+// 32 accumulator columns of rows lab[0..31] (16-byte aligned): every disallowed column becomes -inf.  All lanes of a
+// warp read the same words (broadcast loads).
+__device__ __forceinline__ void mask_columns32(uint32_t (&v)[32], const uint32_t* __restrict__ lab, const LabelFilter& f) {
+#pragma unroll
+  for (int j = 0; j < 32; j += 4) {
+    const uint4 l = __ldg(reinterpret_cast<const uint4*>(lab + j));
+    if (!f.allows(l.x)) v[j] = NEG_INF_BITS;
+    if (!f.allows(l.y)) v[j + 1] = NEG_INF_BITS;
+    if (!f.allows(l.z)) v[j + 2] = NEG_INF_BITS;
+    if (!f.allows(l.w)) v[j + 3] = NEG_INF_BITS;
+  }
+}
+
 __device__ __forceinline__ float max3(float a, float b, float c) {
   float r;
   asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c));   // FMNMX3 (sm_100)
@@ -90,6 +124,9 @@ static __device__ __noinline__ void append_columns(uint32_t taddr, int ncols, fl
 // r-th largest of the n <= 4096 sampled maxima of query q, by the 128 epilogue threads of a CTA (et = 0..127): the
 // values sit in registers as order-preserving keys, four 8-bit radix passes over a 256-bin shared-memory histogram
 // (`hist`, 1 KB) fix the key byte by byte; `tmp` = two words of shared memory.  Named barrier 1 (128 threads).
+// One copy per FILTER value: ptxas fits a callee's registers to all its callers, and the unfiltered scan kernels keep
+// the code they had without the FILTER instances.
+template <bool FILTER>
 static __device__ __noinline__ float epilogue_select(const float* __restrict__ sample, int n, int ld, int q, int query_major,
                                                      int r, uint32_t* hist, uint32_t* tmp, int et) {
   constexpr int VPT = 32;
@@ -150,6 +187,41 @@ static __device__ __noinline__ float max_columns(uint32_t taddr, int ncols) {
     tmem_ld_wait();
 #pragma unroll
     for (int j = 0; j < 8; ++j) if (c + j < ncols) m = fmaxf(m, __uint_as_float(v[j]));
+  }
+  return m;
+}
+// The same two slow paths over allowed rows only (FILTER instances); column c is row row_base + c.  thr must not be
+// -inf here (the caller clamps it to -FLT_MAX), so a masked column can never qualify.
+static __device__ __noinline__ void append_columns_filtered(uint32_t taddr, int ncols, float thr, uint32_t row_base,
+                                                            uint2* seg, unsigned int& cnt, unsigned int seg_cap,
+                                                            const uint32_t* __restrict__ labels, LabelFilter f) {
+#pragma unroll 1
+  for (int c = 0; c < ncols; c += 8) {
+    uint32_t v[8];
+    __syncwarp();
+    tmem_ld_32x8(taddr + (uint32_t)c, v);
+    tmem_ld_wait();
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      if (c + j < ncols && __uint_as_float(v[j]) >= thr && f.allows(__ldg(labels + row_base + (uint32_t)(c + j)))) {
+        if (cnt < seg_cap) seg[cnt] = make_uint2(v[j], row_base + (uint32_t)(c + j));
+        ++cnt;
+      }
+    }
+  }
+}
+static __device__ __noinline__ float max_columns_filtered(uint32_t taddr, int ncols, uint32_t row_base,
+                                                          const uint32_t* __restrict__ labels, LabelFilter f) {
+  float m = -INFINITY;
+#pragma unroll 1
+  for (int c = 0; c < ncols; c += 8) {
+    uint32_t v[8];
+    __syncwarp();
+    tmem_ld_32x8(taddr + (uint32_t)c, v);
+    tmem_ld_wait();
+#pragma unroll
+    for (int j = 0; j < 8; ++j)
+      if (c + j < ncols && f.allows(__ldg(labels + row_base + (uint32_t)(c + j)))) m = fmaxf(m, __uint_as_float(v[j]));
   }
   return m;
 }

@@ -623,6 +623,20 @@ exact_exclude_kernel(const long long* __restrict__ excl, int E, const int* __res
   }
 }
 
+// Label filters on the exact path: every row query qsel[s] does not allow gets the same sentinel, so select, collect
+// and sort treat it like an excluded row.  O(N) per query slot; require u32 [nq, 2] = {all, any} of the QUERY row.
+__global__ void __launch_bounds__(256)
+exact_filter_kernel(const uint32_t* __restrict__ labels, const uint32_t* __restrict__ require, const int* __restrict__ qsel,
+                    int slot0, long long N, float* __restrict__ scores_ws) {
+  const int s = blockIdx.y;
+  const int qi = qsel ? qsel[slot0 + s] : (slot0 + s);
+  const uint32_t all = require[2 * (long long)qi], any = require[2 * (long long)qi + 1];
+  for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < N; r += (long long)gridDim.x * blockDim.x) {
+    const uint32_t l = labels[r];
+    if ((l & all) != all || (any != 0u && (l & any) == 0u)) scores_ws[(long long)s * N + r] = __uint_as_float(EXCL_SCORE_BITS);
+  }
+}
+
 __global__ void exact_init_kernel(SelState* st, unsigned int* hist, int nslot, int K) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < nslot) { st[i].prefix = 0ull; st[i].kremain = K; st[i].count = 0u; }
@@ -760,7 +774,8 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_exact_wo
 
 static int flat_search_exact_impl(const float* q, int nq, const int32_t* qsel, int nsel, const float* Xn, int64_t N,
                                   int D, int K, int64_t id_offset, float* scores, int64_t* ids, const int64_t* excl,
-                                  int E, void* workspace, size_t workspace_bytes, void* stream) {
+                                  int E, void* workspace, size_t workspace_bytes, void* stream,
+                                  const uint32_t* labels = nullptr, const uint32_t* require = nullptr) {
   TT_CHECK_ARG(q && Xn && scores && ids && workspace, "null pointer");
   TT_CHECK_ARG(N >= 1 && N < (1LL << 32) && D >= 1, "need 1 <= N < 2^32, D >= 1");
   TT_CHECK_ARG(K >= 1 && K <= N && K <= TT_FLAT_MAX_K, "need 1 <= K <= min(N, TT_FLAT_MAX_K)");
@@ -795,6 +810,10 @@ static int flat_search_exact_impl(const float* q, int nq, const int32_t* qsel, i
                                                   scores_ws);
       TT_CHECK_LAUNCH();
     }
+    if (labels) {
+      exact_filter_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(labels, require, qsel, slot0, N, scores_ws);
+      TT_CHECK_LAUNCH();
+    }
     exact_init_kernel<<<(nslot * 256 + 255) / 256, 256, 0, st>>>(state, hist, nslot, K);
     TT_CHECK_LAUNCH();
     for (int shift = 56; shift >= 0; shift -= 8) {
@@ -806,7 +825,7 @@ static int flat_search_exact_impl(const float* q, int nq, const int32_t* qsel, i
     exact_collect_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(scores_ws, N, state, keys, K);
     TT_CHECK_LAUNCH();
     exact_sort_kernel<<<nslot, 256, (size_t)P * 8, st>>>(keys, qsel, slot0, K, id_offset, scores,
-                                                         reinterpret_cast<long long*>(ids), E > 0);
+                                                         reinterpret_cast<long long*>(ids), E > 0 || labels != nullptr);
     TT_CHECK_LAUNCH();
   }
   return TT_OK;
@@ -828,4 +847,16 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact_excl(
   TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   return flat_search_exact_impl(q, nq, qsel, nsel, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
                                 workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact_filtered(const float* q, int nq, const int32_t* qsel, int nsel,
+                                             const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                                             float* scores, int64_t* ids, const uint32_t* labels, const uint32_t* require,
+                                             const int64_t* excl, int E, void* workspace, size_t workspace_bytes,
+                                             void* stream) {
+  TT_CHECK_ARG(labels != nullptr && require != nullptr, "null labels or require (the unfiltered call is tt_flat_search_exact_excl)");
+  TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
+  TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
+  return flat_search_exact_impl(q, nq, qsel, nsel, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
+                                workspace_bytes, stream, labels, require);
 }

@@ -22,7 +22,7 @@ import torch
 
 from .buyer_tower import BuyerTower
 from .config import DEFAULT_EVENT_WEIGHTS, get_event_weight
-from .vector_db import PendingSearch, VectorDatabase
+from .vector_db import PendingSearch, VectorDatabase, require_masks
 
 
 class RetrievalPipeline:
@@ -65,21 +65,26 @@ class RetrievalPipeline:
         return self.tower.forward_gather(self.table, indices, weights, self.item_logits)
 
     def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int, *,
-                              exclude_history: bool = False) -> PendingSearch:
+                              exclude_history: bool = False, require_all=0, require_any=0) -> PendingSearch:
         """exclude_history: the pooled history rows `indices` (-1 padded; the last `max_interaction_history`
         interactions when they come from encode_histories) are also the exclusion list of the search, so no buyer
-        is shown the items they have just viewed, carted or bought.  No extra host-to-device copy."""
+        is shown the items they have just viewed, carted or bought.  No extra host-to-device copy.
+        require_all / require_any: label masks (scalars or one per buyer, host values): only items whose label word
+        (VectorDatabase.set_labels) has every bit of require_all and, unless require_any is 0, one bit of require_any."""
         k = min(k, self.index.ntotal)                                                  # vector_db.py:159
+        req = require_masks(require_all, require_any, int(indices.shape[0]))
         emb = self.encode_device(indices, weights)
-        if not exclude_history:
-            return self.index.search_async(emb, k)
-        excl = indices.to(device=self.index.device, dtype=torch.int64).contiguous()
-        return self.index.search_async(emb, k, exclude=excl)
+        kw = {} if req is None else {"require": req}
+        if exclude_history:
+            kw["exclude"] = indices.to(device=self.index.device, dtype=torch.int64).contiguous()
+        return self.index.search_async(emb, k, **kw)
 
-    def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *, exclude_history: bool = False):
+    def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *, exclude_history: bool = False,
+                        require_all=0, require_any=0):
         """-> (scores f32 [B,k'], row indices i64 [B,k']) numpy; one H2D of the padded history, one D2H.
-        exclude_history: leave out the buyer's last `max_interaction_history` interacted items (see
-        retrieve_device_async); a buyer with fewer than k' other items gets (-inf, -1) at the tail."""
+        exclude_history: leave out the buyer's last `max_interaction_history` interacted items; require_all /
+        require_any: label masks (see retrieve_device_async); a buyer with fewer than k' allowed items gets (-inf, -1)
+        at the tail."""
         idx, w, _ = self.encode_histories(batch)
         key = idx.shape
         pins = self._pins.get(key)
@@ -92,25 +97,26 @@ class RetrievalPipeline:
         pins[1].copy_(torch.from_numpy(w))
         dev = self.index.device
         idx_dev, w_dev = pins[0].to(dev, non_blocking=True), pins[1].to(dev, non_blocking=True)
-        if exclude_history:
-            pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=True)
-        else:
-            pending = self.retrieve_device_async(idx_dev, w_dev, k)
+        pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=exclude_history,
+                                             require_all=require_all, require_any=require_any)
         scores, ids, _ = pending.result()
         return scores.cpu().numpy(), ids.cpu().numpy()
 
     def retrieve(self, interactions: Sequence[Dict[str, Any]], k: int = 10, *,
-                 exclude_history: bool = False) -> List[Tuple[str, float]]:
+                 exclude_history: bool = False, require_all=0, require_any=0) -> List[Tuple[str, float]]:
         """One request, the shape of server.py:241-244 -> [(product_id, score)] in descending score.
-        exclude_history: never return the items of the buyer's last `max_interaction_history` interactions."""
-        scores, ids = self.retrieve_arrays([interactions], k, exclude_history=exclude_history)
+        exclude_history: never return the items of the buyer's last `max_interaction_history` interactions.
+        require_all / require_any: label masks (see retrieve_device_async)."""
+        scores, ids = self.retrieve_arrays([interactions], k, exclude_history=exclude_history, require_all=require_all,
+                                           require_any=require_any)
         pids = self.db.product_ids
         return [(pids[i], float(s)) for i, s in zip(ids[0].tolist(), scores[0].tolist()) if 0 <= i < len(pids)]
 
     def retrieve_batch(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *,
-                       exclude_history: bool = False) -> List[List[Tuple[str, float]]]:
-        """exclude_history: as in retrieve, per buyer."""
-        scores, ids = self.retrieve_arrays(batch, k, exclude_history=exclude_history)
+                       exclude_history: bool = False, require_all=0, require_any=0) -> List[List[Tuple[str, float]]]:
+        """exclude_history: as in retrieve, per buyer; require_all / require_any: scalars or one value per buyer."""
+        scores, ids = self.retrieve_arrays(batch, k, exclude_history=exclude_history, require_all=require_all,
+                                           require_any=require_any)
         pids = self.db.product_ids
         n = len(pids)
         return [[(pids[i], s) for i, s in zip(ri, rs) if 0 <= i < n] for rs, ri in zip(scores.tolist(), ids.tolist())]

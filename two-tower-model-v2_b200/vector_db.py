@@ -123,6 +123,51 @@ def read_native_shard(path: str):
 
 
 # ---------------------------------------------------------------------------------------------
+# Label filters (tt_flat_search_filtered): one u32 label word per row, masks {all, any} per query.  Both travel as int32
+# tensors holding the u32 bit patterns.
+_U32_LIMIT = 1 << 32
+
+
+def u32_words(values, what: str):
+    """Integer values in [0, 2^32) -> int32 words with the same bits: a numpy array for host input, a tensor on the same
+    device for a CUDA tensor.  int32 / uint32 tensors are taken as raw words; any other integer input is range-checked
+    (an int64 CUDA tensor with one device-to-host read)."""
+    if isinstance(values, torch.Tensor) and values.is_cuda:
+        if values.dtype == torch.int32:
+            return values
+        if values.dtype == torch.uint32:
+            return values.view(torch.int32)
+        if values.dtype != torch.int64:
+            raise ValueError(f"{what} must be an integer tensor (int64, int32 or uint32), got {values.dtype}")
+        if bool(((values < 0) | (values >= _U32_LIMIT)).any()):
+            raise ValueError(f"{what} must be in [0, 2^32)")
+        return torch.where(values >= (1 << 31), values - _U32_LIMIT, values).to(torch.int32)
+    if isinstance(values, torch.Tensor):
+        values = values.numpy()
+    arr = np.asarray(values)
+    if arr.size == 0:
+        arr = arr.astype(np.int64)
+    if arr.dtype == np.bool_ or not np.issubdtype(arr.dtype, np.integer):
+        raise ValueError(f"{what} must hold integers in [0, 2^32), got dtype {arr.dtype}")
+    if arr.size and (int(arr.min()) < 0 or int(arr.max()) >= _U32_LIMIT):
+        raise ValueError(f"{what} must be in [0, 2^32), got values in [{int(arr.min())}, {int(arr.max())}]")
+    return arr.astype(np.uint32).view(np.int32)          # a fresh contiguous copy (0-d input stays 0-d)
+
+
+def require_masks(require_all, require_any, nq: int) -> Optional[np.ndarray]:
+    """(all, any) masks, each a scalar or one value per query -> int32 words [nq, 2], or None when every query's masks
+    are (0, 0) (no filter)."""
+    cols = []
+    for name, v in (("require_all", require_all), ("require_any", require_any)):
+        w = u32_words(v, name)
+        if w.ndim > 1 or (w.ndim == 1 and w.shape[0] != nq):
+            raise ValueError(f"{name} must be a scalar or one value per query ({nq}), got shape {w.shape}")
+        cols.append(np.broadcast_to(w, (nq,)))
+    req = np.ascontiguousarray(np.stack(cols, 1))
+    return req if req.any() else None
+
+
+# ---------------------------------------------------------------------------------------------
 class _FlagRing:
     """A few pinned int32 slots: the status words of a search (uncertified count[, exchange time-out]) are
     copied into one of them asynchronously, so the host can look at them later without draining the stream.
@@ -191,6 +236,8 @@ class FlatIPIndex:
         self._xh_store: Optional[torch.Tensor] = None
         self.stats = torch.zeros(4, device=self.device, dtype=torch.float32)
         self.id_offset = 0
+        self.labels: Optional[torch.Tensor] = None        # int32 [N] (u32 label words) once set_labels was called
+        self._labels_store: Optional[torch.Tensor] = None
         self._ws: Dict[Tuple[int, int], torch.Tensor] = {}
         self._exact_ws: Optional[torch.Tensor] = None
         self._ring: Optional[_FlagRing] = None
@@ -216,6 +263,13 @@ class FlatIPIndex:
                 xh[:old].copy_(self.xh)
             self._xn_store, self._xh_store = xn, xh
         self.xn, self.xh = self._xn_store[:n], self._xh_store[:n]
+        if self._labels_store is not None:             # labels stay aligned with the rows; new rows get 0
+            if self._labels_store.shape[0] < self._xn_store.shape[0]:
+                lab = torch.zeros(self._xn_store.shape[0], device=self.device, dtype=torch.int32)
+                lab[:old].copy_(self._labels_store[:old])
+                self._labels_store = lab
+            self._labels_store[old:n].zero_()
+            self.labels = self._labels_store[:n]
         self._ws.clear()
         self._exact_ws = None
 
@@ -228,8 +282,18 @@ class FlatIPIndex:
                                             self.xn.data_ptr(), self.xh.data_ptr(), row0, self.stats.data_ptr(),
                                             ops._stream()), "tt_flat_build")
 
-    def add(self, x, normalize: bool = True, chunk_rows: int = 1 << 17) -> None:
-        """Appends rows (numpy [n,d] or a torch tensor on any device)."""
+    def add(self, x, normalize: bool = True, chunk_rows: int = 1 << 17, labels=None) -> None:
+        """Appends rows (numpy [n,d] or a torch tensor on any device).  `labels` (n values in [0, 2^32), see
+        set_labels) are the new rows' label words; without them the new rows of a labelled index get 0."""
+        if labels is not None:
+            n_new = x.shape[0]
+            words = u32_words(labels, "labels")
+            if tuple(words.shape) != (n_new,):
+                raise ValueError(f"expected {n_new} label words, got shape {tuple(words.shape)}")
+            row0 = self.ntotal
+            self.add(x, normalize, chunk_rows)
+            self._store_labels(words, torch.arange(row0, row0 + n_new))
+            return
         if isinstance(x, np.ndarray):
             if x.ndim != 2 or x.shape[1] != self.d:
                 raise ValueError(f"expected [n, {self.d}] rows, got {x.shape}")
@@ -283,6 +347,55 @@ class FlatIPIndex:
         self.id_offset = id_offset
         return self
 
+    # -- label words -----------------------------------------------------------------------
+    def set_labels(self, labels, rows=None) -> None:
+        """Sets the u32 label word of every row (`labels` [ntotal]), or of the listed `rows` only (in-place update;
+        `labels` then has one value per listed row).  numpy or CUDA input, values in [0, 2^32); int32 / uint32 tensors
+        are taken as raw words.  Stream-ordered: a search enqueued after this call sees the new words.  Rows that never
+        got a label have the word 0.  Labels are serving state: save / load do not store them."""
+        if self.ntotal == 0:
+            raise ValueError("empty index")
+        words = u32_words(labels, "labels")
+        if rows is None:
+            if tuple(words.shape) != (self.ntotal,):
+                raise ValueError(f"expected one label word per row ({self.ntotal}), got shape {tuple(words.shape)}")
+        else:
+            r = rows if isinstance(rows, torch.Tensor) else torch.from_numpy(np.asarray(rows))
+            if r.dim() != 1 or r.dtype not in (torch.int64, torch.int32) or tuple(words.shape) != (r.shape[0],):
+                raise ValueError(f"rows must be a 1-D integer array with one entry per label word, got rows "
+                                 f"{r.dtype} {tuple(r.shape)} and labels {tuple(words.shape)}")
+            if r.numel() and (int(r.min()) < 0 or int(r.max()) >= self.ntotal):
+                raise ValueError(f"rows must be in [0, {self.ntotal})")
+        self._store_labels(words, None if rows is None else r)
+
+    def _store_labels(self, words, rows: Optional[torch.Tensor]) -> None:
+        """Writes validated int32 words (numpy or CUDA) to all rows, or to the given rows."""
+        w = torch.from_numpy(words) if isinstance(words, np.ndarray) else words
+        with torch.cuda.device(self.device):
+            if self._labels_store is None:
+                self._labels_store = torch.zeros(self._xn_store.shape[0], device=self.device, dtype=torch.int32)
+                self.labels = self._labels_store[:self.ntotal]
+            if rows is None:
+                self.labels.copy_(w.to(self.device))
+            else:
+                self.labels.index_copy_(0, rows.to(self.device, torch.int64), w.to(self.device))
+
+    def _requires(self, require, nq: int) -> Optional[torch.Tensor]:
+        """Validates per-query label masks (CUDA or numpy [nq, 2] = {all, any}, or [2] for every query) -> int32 [nq, 2]
+        on this device, or None when every query's masks are (0, 0): the unfiltered search runs."""
+        if require is None:
+            return None
+        w = u32_words(require, "require")
+        if tuple(w.shape) not in ((2,), (nq, 2)):
+            raise ValueError(f"require must be [nq={nq}, 2] or [2] ({{all, any}} masks), got shape {tuple(w.shape)}")
+        if not bool(w.any()):
+            return None
+        if self.labels is None:
+            raise ValueError("a label filter needs label words: call set_labels() first")
+        if isinstance(w, np.ndarray):
+            w = torch.from_numpy(w)
+        return w.to(self.device).expand(nq, 2).contiguous()
+
     def rows_host(self) -> np.ndarray:
         """The stored fp32 rows (what faiss.write_index would serialise)."""
         return self.xn.cpu().numpy()
@@ -316,7 +429,7 @@ class FlatIPIndex:
             self._ws[key] = ws
         return ws
 
-    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
+    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
         """Asynchronous search of CUDA f32 queries [nq,D] on the current stream.
 
         Returns (scores [nq,k] f32, ids [nq,k] i64, flags [nq] i32, n_uncertified [1] i32) device
@@ -324,6 +437,8 @@ class FlatIPIndex:
         passed to `search_exact_device` (`search_checked_device` / `search_async` do both).
         `exclude` (CUDA i64 [nq, E], E <= 1024, ids as returned, -1 = padding): the top-k over the rows query i does
         not list in exclude[i]; with fewer than k allowed rows the tail is (-inf, -1).
+        `require` (CUDA or numpy [nq, 2] = {all, any} u32 masks, or [2] for every query): only rows whose label word
+        has every bit of `all` and, unless any == 0, one bit of `any` (see set_labels); composes with `exclude`.
         """
         if self.ntotal == 0:
             raise ValueError("empty index")
@@ -331,6 +446,7 @@ class FlatIPIndex:
             raise ValueError(f"expected queries [nq, {self.d}], got {tuple(q.shape)}")
         if not 1 <= k <= min(self.ntotal, _native.TT_FLAT_MAX_K):
             raise ValueError(f"k must be in [1, min(ntotal, {_native.TT_FLAT_MAX_K})], got {k}")
+        req = self._requires(require, q.shape[0])
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
         excl = self._exclusions(exclude, nq)
@@ -340,7 +456,15 @@ class FlatIPIndex:
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
         lib = _native.load()
         with torch.cuda.device(self.device):
-            if excl is None:
+            if req is not None:
+                E = 0 if excl is None else excl.shape[1]
+                ws = self._workspace(max(nq, 1), k, E)
+                _native.check(lib.tt_flat_search_filtered(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, scores.data_ptr(), ids.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    self.labels.data_ptr(), req.data_ptr(), 0 if excl is None else excl.data_ptr(), E, ws.data_ptr(),
+                    ws.numel(), ops._stream()), "tt_flat_search_filtered")
+            elif excl is None:
                 ws = self._workspace(max(nq, 1), k)
                 _native.check(lib.tt_flat_search(
                     q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
@@ -357,9 +481,10 @@ class FlatIPIndex:
 
     def search_exact_device(self, q: torch.Tensor, k: int, scores: Optional[torch.Tensor] = None,
                             ids: Optional[torch.Tensor] = None, qsel: Optional[torch.Tensor] = None, *,
-                            exclude: Optional[torch.Tensor] = None):
+                            exclude: Optional[torch.Tensor] = None, require=None):
         """Always-exact fp32 path; with `qsel` (i32 query rows) only those rows of scores/ids are rewritten.
-        `exclude` [nq, E] is indexed by query row (qsel[i]), as in search_device."""
+        `exclude` [nq, E] and `require` [nq, 2] are indexed by query row (qsel[i]), as in search_device."""
+        req = self._requires(require, q.shape[0])
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
         excl = self._exclusions(exclude, nq)
@@ -372,7 +497,13 @@ class FlatIPIndex:
         if self._exact_ws is None or self._exact_ws.numel() < need:
             self._exact_ws = torch.empty(need, device=self.device, dtype=torch.uint8)
         with torch.cuda.device(self.device):
-            if excl is None:
+            if req is not None:
+                _native.check(lib.tt_flat_search_exact_filtered(
+                    q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
+                    self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(), self.labels.data_ptr(), req.data_ptr(),
+                    0 if excl is None else excl.data_ptr(), 0 if excl is None else excl.shape[1],
+                    self._exact_ws.data_ptr(), self._exact_ws.numel(), ops._stream()), "tt_flat_search_exact_filtered")
+            elif excl is None:
                 _native.check(lib.tt_flat_search_exact(
                     q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
                     self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(), self._exact_ws.data_ptr(),
@@ -442,11 +573,15 @@ class FlatIPIndex:
                                                   ops._stream()), "tt_flat_scan_scores")
         return out
 
-    def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None) -> PendingSearch:
+    def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None,
+                     require=None) -> PendingSearch:
         """Enqueues a search and returns at once; `.result()` checks the certificate later, so a caller can
-        keep the next batch's kernels queued behind this one (no idle GPU between batches).  `exclude`: see
-        search_device; uncertified queries are re-run exactly with the same lists."""
+        keep the next batch's kernels queued behind this one (no idle GPU between batches).  `exclude`, `require`:
+        see search_device; uncertified queries are re-run exactly with the same lists and masks.  (Masks in a CUDA
+        tensor cost one device-to-host read to tell a filter from (0, 0); numpy masks cost none.)"""
         kw = {} if exclude is None else {"exclude": exclude}
+        if require is not None:
+            kw["require"] = require
         scores, ids, flags, nunc = self.search_device(q, k, **kw)
         if self._ring is None:
             self._ring = _FlagRing()
@@ -460,9 +595,9 @@ class FlatIPIndex:
             return scores, ids, n_bad
         return PendingSearch(finish)
 
-    def search_checked_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
+    def search_checked_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
         """search_device + re-run of uncertified queries through the exact path (one host sync)."""
-        return self.search_async(q, k, **({} if exclude is None else {"exclude": exclude})).result()
+        return self.search_async(q, k, exclude=exclude, require=require).result()
 
     def post_flag(self, nunc_dev: torch.Tensor):
         if self._ring is None:
@@ -525,25 +660,29 @@ class FlatIPIndex:
                     nunc.data_ptr(), bound.data_ptr(), excl.data_ptr(), excl.shape[1], ws.data_ptr(), ws.numel(),
                     ops._stream()), "tt_flat_shard_search_excl")
 
-    def search_host_async(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None) -> PendingSearch:
+    def search_host_async(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None,
+                          require=None) -> PendingSearch:
         """Host-to-host search, asynchronous: stages q through pinned memory, enqueues H2D + search + D2H and
         returns; `.result()` -> (scores, ids, n_rerun) numpy arrays.  Up to 3 calls may be in flight.
-        `exclude`: numpy int64 [nq, E] (see search_device)."""
-        return host_search_async(self, self.search_async, self.device, self.d, q, k, exclude=exclude)
+        `exclude`: numpy int64 [nq, E]; `require`: numpy [nq, 2] or [2] label masks (see search_device)."""
+        return host_search_async(self, self.search_async, self.device, self.d, q, k, exclude=exclude, require=require)
 
-    def search(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+    def search(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None,
+               require=None) -> Tuple[np.ndarray, np.ndarray]:
         """Host-to-host search, the shape of faiss `index.search(q, k)`: q f32 [nq,d] (un-normalised:
         the device op applies q/(||q||+1e-8)) -> (scores f32 [nq,k], ids i64 [nq,k]).  `exclude`: numpy int64
-        [nq, E] ids to leave out per query (-1 = padding); short results end in (-inf, -1)."""
-        scores, ids, _ = self.search_host_async(q, k, exclude=exclude).result()
+        [nq, E] ids to leave out per query (-1 = padding); `require`: label masks {all, any} per query ([nq, 2] or
+        [2]); short results end in (-inf, -1)."""
+        scores, ids, _ = self.search_host_async(q, k, exclude=exclude, require=require).result()
         return scores, ids
 
 
 def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int, depth: int = 3, *,
-                      exclude: Optional[np.ndarray] = None) -> PendingSearch:
+                      exclude: Optional[np.ndarray] = None, require=None) -> PendingSearch:
     """Shared host round trip of FlatIPIndex / ShardedFlatIPIndex: pinned staging buffers in a ring of `depth`
     sets per (nq, k) so that consecutive batches overlap their copies with the previous batch's kernels.
-    `exclude` (numpy int64 [nq, E]) is copied to the device with the queries and passed on as `exclude=`."""
+    `exclude` (numpy int64 [nq, E]) is copied to the device with the queries and passed on as `exclude=`; `require`
+    (label masks, FlatIPIndex only) is passed on as `require=`."""
     q = np.ascontiguousarray(q, dtype=np.float32)
     if q.ndim != 2 or q.shape[1] != d:
         raise ValueError(f"expected queries [nq, {d}], got {q.shape}")
@@ -576,10 +715,10 @@ def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int
         dq = hq.to(device, non_blocking=True)
         evs[slot] = torch.cuda.Event()
         evs[slot].record(stream)
-        if exclude is None:
-            pending = search_async(dq, k)
-        else:
-            pending = search_async(dq, k, exclude=torch.from_numpy(exclude).to(device))
+        kw = {} if exclude is None else {"exclude": torch.from_numpy(exclude).to(device)}
+        if require is not None:
+            kw["require"] = require
+        pending = search_async(dq, k, **kw)
 
     def finish():
         scores, ids, n_bad = pending.result()        # exact re-run (if any) is enqueued before the copies below
@@ -661,18 +800,34 @@ class VectorDatabase:
                 json.dump(self.id_to_index, f, ensure_ascii=False, indent=2)
         print(f"Saved FAISS index to {index_path}")
 
+    # -- label words ---------------------------------------------------------------------------
+    def set_labels(self, labels, product_ids: Optional[List[str]] = None) -> None:
+        """Sets the u32 label words the `require` filters test (e.g. bit 0 = in stock, bits 1-31 = category groups):
+        one per index row in index order, or one per listed product id.  An unknown product id raises ValueError and
+        changes nothing.  Labels are serving state: save_index / load_index do not store them."""
+        if self.index is None:
+            raise ValueError("Index not built. Call build_index() or load_index() first.")
+        if product_ids is None:
+            self.index.set_labels(labels)
+            return
+        unknown = [p for p in product_ids if p not in self.id_to_index]
+        if unknown:
+            raise ValueError(f"{len(unknown)} unknown product ids, e.g. {unknown[:3]}")
+        self.index.set_labels(labels, rows=np.array([self.id_to_index[p] for p in product_ids], np.int64))
+
     # -- search --------------------------------------------------------------------------------
     def search_batch(self, query_embeddings: np.ndarray, k: int = 10, *,
-                     exclude_rows: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+                     exclude_rows: Optional[np.ndarray] = None, require=None) -> Tuple[np.ndarray, np.ndarray]:
         """Array-returning retrieval: (scores f32 [nq,k'], row indices i64 [nq,k']) with k' = min(k, ntotal).
-        `exclude_rows` int64 [nq, E] (-1 = padding): row indices query i must not return; with fewer than k' allowed
-        rows the tail is (-inf, -1)."""
+        `exclude_rows` int64 [nq, E] (-1 = padding): row indices query i must not return; `require` [nq, 2] or [2]:
+        {all, any} label masks (see FlatIPIndex.search_device); with fewer than k' allowed rows the tail is (-inf, -1)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         k = min(k, self.index.ntotal)   # vector_db.py:159
-        if exclude_rows is None:
-            return self.index.search(np.asarray(query_embeddings), k)
-        return self.index.search(np.asarray(query_embeddings), k, exclude=exclude_rows)
+        kw = {} if exclude_rows is None else {"exclude": exclude_rows}
+        if require is not None:
+            kw["require"] = require
+        return self.index.search(np.asarray(query_embeddings), k, **kw)
 
     def _exclude_rows(self, lists, nq: int) -> Optional[np.ndarray]:
         """Product-id lists (one per query) -> row indices int64 [nq, E], -1 padded; unknown ids are dropped.
@@ -687,19 +842,24 @@ class VectorDatabase:
         return out
 
     def retrieve(self, query_embedding: np.ndarray, k: int = 10, *,
-                 exclude: Optional[List[str]] = None) -> List[Tuple[str, float]]:
+                 exclude: Optional[List[str]] = None, require_all=0, require_any=0) -> List[Tuple[str, float]]:
         """vector_db.py:130-169 — descending score; only query row 0 is returned, as in the reference.
-        `exclude`: product ids that must not be returned (e.g. the buyer's own history); unknown ids are ignored."""
+        `exclude`: product ids that must not be returned (e.g. the buyer's own history); unknown ids are ignored.
+        `require_all` / `require_any`: label masks (scalars, or one per query row): only products whose label word has
+        every bit of require_all and, unless require_any is 0, one bit of require_any (see set_labels)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         query_embedding = np.asarray(query_embedding)
         if query_embedding.ndim == 1:
             query_embedding = query_embedding.reshape(1, -1)
+        nq = query_embedding.shape[0]
+        kw = {}
+        req = require_masks(require_all, require_any, nq)
+        if req is not None:
+            kw["require"] = req
         if exclude is not None:
-            rows = self._exclude_rows([exclude] * query_embedding.shape[0], query_embedding.shape[0])
-            scores, indices = self.search_batch(query_embedding, k, exclude_rows=rows)
-        else:
-            scores, indices = self.search_batch(query_embedding, k)
+            kw["exclude_rows"] = self._exclude_rows([exclude] * nq, nq)
+        scores, indices = self.search_batch(query_embedding, k, **kw)
         results = []
         for idx, score in zip(indices[0], scores[0]):
             if 0 <= idx < len(self.product_ids):
@@ -707,17 +867,22 @@ class VectorDatabase:
         return results
 
     def retrieve_batch(self, query_embeddings: np.ndarray, k: int = 10, *,
-                       exclude: Optional[List[List[str]]] = None) -> List[List[Tuple[str, float]]]:
-        """vector_db.py:171-209.  `exclude`: one list of product ids per query that it must not return."""
+                       exclude: Optional[List[List[str]]] = None, require_all=0,
+                       require_any=0) -> List[List[Tuple[str, float]]]:
+        """vector_db.py:171-209.  `exclude`: one list of product ids per query that it must not return.
+        `require_all` / `require_any`: label masks, scalars or one per query (see retrieve)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
+        nq = np.asarray(query_embeddings).shape[0]
+        kw = {}
+        req = require_masks(require_all, require_any, nq)
+        if req is not None:
+            kw["require"] = req
         if exclude is not None:
-            nq = np.asarray(query_embeddings).shape[0]
             if len(exclude) != nq:
                 raise ValueError(f"exclude needs one list per query ({nq}), got {len(exclude)}")
-            scores, indices = self.search_batch(query_embeddings, k, exclude_rows=self._exclude_rows(exclude, nq))
-        else:
-            scores, indices = self.search_batch(query_embeddings, k)
+            kw["exclude_rows"] = self._exclude_rows(exclude, nq)
+        scores, indices = self.search_batch(query_embeddings, k, **kw)
         pids = self.product_ids
         n = len(pids)
         all_results = []
