@@ -242,8 +242,8 @@ int tt_flat_search_exact_excl(const float* q, int nq, const int32_t* qsel, int n
  * allowed rows' scores and the certificate reads over allowed rows: "every allowed row not rescored scores below the
  * bound".  The plan does not depend on the filter: the workspace is tt_flat_search_excl_workspace_bytes(N, D, nq, K,
  * E) (E = 0 without a list).  tt_flat_search_exact_filtered reads the masks (and the list) of the QUERY row qsel[i];
- * an uncertified query is re-run there with the same masks.  Single-device calls only: the shard entry points take
- * no filter. */
+ * an uncertified query is re-run there with the same masks.  The shard entry points have _filtered forms too (below,
+ * after the _excl shard calls). */
 int tt_flat_search_filtered(const float* q, int nq,
                             const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
                             int K, int64_t id_offset,
@@ -317,6 +317,34 @@ int tt_flat_shard_search_excl(int nq, const float* Xn, const void* Xh, int64_t N
                               float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
                               const int64_t* excl, int E,
                               void* workspace, size_t workspace_bytes, void* stream);
+/* The shard searches with label filters (see tt_flat_search_filtered).  labels u32 [N_local] is THIS shard's words in
+ * local row order (16-byte aligned); require u32 [nq, 2] is the same on every rank (8-byte aligned).  Both must be
+ * non-NULL; excl / E compose as in the _excl calls (global ids, E = 0 without a list).  Disallowed rows never reach the
+ * sample, so each shard's top-r list holds maxima over its allowed rows (all -inf when no sampled row is allowed), the
+ * gathered threshold is a lower bound over allowed rows and every shard's bound keeps its meaning over them:
+ * tt_shard_merge and its certificate apply unchanged.  The plan and the workspace do not depend on the filter: call
+ * tt_flat_shard_plan_ok / tt_flat_shard_workspace_bytes / tt_flat_shard_sample_filtered with K_plan as above (K
+ * without a list) and tt_flat_shard_search_filtered with K.  tt_flat_search_shard_filtered serves a route_exact or
+ * unsupported plan through tt_flat_search_exact_filtered with bound = -inf.  A shard whose allowed rows are fewer than
+ * K pads its record with -inf / -1.  An uncertified query is re-run on every shard through
+ * tt_flat_search_exact_filtered (id_offset = the shard's first global row) with the same masks. */
+int tt_flat_search_shard_filtered(const float* q, int nq,
+                                  const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
+                                  int K, int64_t id_offset,
+                                  float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
+                                  const uint32_t* labels, const uint32_t* require,
+                                  const int64_t* excl, int E,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+int tt_flat_shard_sample_filtered(const float* q, int nq, const void* Xh, const float* stats,
+                                  int64_t N_local, int64_t N_total, int D, int K,
+                                  const uint32_t* labels, const uint32_t* require, float* topr,
+                                  void* workspace, size_t workspace_bytes, void* stream);
+int tt_flat_shard_search_filtered(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total, int D,
+                                  int K, int64_t id_offset, const float* topr_g, int G,
+                                  float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, float* bound,
+                                  const uint32_t* labels, const uint32_t* require,
+                                  const int64_t* excl, int E,
+                                  void* workspace, size_t workspace_bytes, void* stream);
 int tt_shard_merge(const void* gathered, size_t rank_stride, size_t off_scores, size_t off_ids,
                    size_t off_bound, size_t off_flags, int G, int nq, int K,
                    float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, void* stream);

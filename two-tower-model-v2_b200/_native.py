@@ -69,6 +69,14 @@ SIGNATURES = {
     "tt_flat_search_exact_filtered": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int64,
                                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
                                               c_void_p]),
+    "tt_flat_search_shard_filtered": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int,
+                                              c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_shard_sample_filtered": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int,
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_shard_search_filtered": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64,
+                                              c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
     "tt_flat_shard_plan_ok":(c_int, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_sample": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p,

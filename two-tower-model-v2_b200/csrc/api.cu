@@ -163,17 +163,25 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_excl(const 
                           excl, E, workspace, workspace_bytes, stream);
 }
 
+// The filter arguments of the *_filtered calls -> lab; nullptr when they are valid, else the error message.
+static const char* label_args(const uint32_t* labels, const uint32_t* require, LabelArgs* lab) {
+  if (labels == nullptr || require == nullptr)
+    return "null labels or require (the unfiltered calls are the ones without _filtered)";
+  if ((reinterpret_cast<uintptr_t>(labels) & 15) != 0) return "labels must be 16-byte aligned";
+  if ((reinterpret_cast<uintptr_t>(require) & 7) != 0) return "require must be 8-byte aligned";
+  lab->labels = labels;
+  lab->require = require;
+  return nullptr;
+}
+
 extern "C" __attribute__((visibility("default"))) int tt_flat_search_filtered(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
                                        int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
                                        int32_t* flags, int32_t* n_uncertified, const uint32_t* labels,
                                        const uint32_t* require, const int64_t* excl, int E, void* workspace,
                                        size_t workspace_bytes, void* stream) {
-  TT_CHECK_ARG(labels != nullptr && require != nullptr, "null labels or require (the unfiltered call is tt_flat_search_excl)");
-  TT_CHECK_ARG((reinterpret_cast<uintptr_t>(labels) & 15) == 0, "labels must be 16-byte aligned");
-  TT_CHECK_ARG((reinterpret_cast<uintptr_t>(require) & 7) == 0, "require must be 8-byte aligned");
   LabelArgs lab;
-  lab.labels = labels;
-  lab.require = require;
+  const char* bad = label_args(labels, require, &lab);
+  TT_CHECK_ARG(bad == nullptr, bad);
   return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
                           excl, E, workspace, workspace_bytes, stream, lab);
 }
@@ -196,6 +204,20 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard_excl(
                           excl, E, workspace, workspace_bytes, stream);
 }
 
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard_filtered(const float* q, int nq, const float* Xn, const void* Xh,
+                                             const float* stats, int64_t N, int D, int K, int64_t id_offset,
+                                             float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified,
+                                             float* bound, const uint32_t* labels, const uint32_t* require,
+                                             const int64_t* excl, int E, void* workspace, size_t workspace_bytes,
+                                             void* stream) {
+  TT_CHECK_ARG(bound != nullptr, "null bound");
+  LabelArgs lab;
+  const char* bad = label_args(labels, require, &lab);
+  TT_CHECK_ARG(bad == nullptr, bad);
+  return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, bound,
+                          excl, E, workspace, workspace_bytes, stream, lab);
+}
+
 // ------------------------------------------------------------------------------------------
 // Sharded catalogs with ONE threshold for the whole catalog (include/tt_b200.h).
 extern "C" __attribute__((visibility("default"))) int tt_flat_shard_plan_ok(int64_t N_local, int64_t N_total, int D, int nq, int K) {
@@ -212,9 +234,9 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_shard_workspace
   return ok ? search_ws_layout(pl, D, nq).total : 0;
 }
 
-extern "C" __attribute__((visibility("default"))) int tt_flat_shard_sample(const float* q, int nq, const void* Xh, const float* stats, int64_t N_local,
-                                    int64_t N_total, int D, int K, float* topr, void* workspace,
-                                    size_t workspace_bytes, void* stream) {
+static int flat_shard_sample_impl(const float* q, int nq, const void* Xh, const float* stats, int64_t N_local,
+                                  int64_t N_total, int D, int K, float* topr, void* workspace, size_t workspace_bytes,
+                                  void* stream, const LabelArgs& lab) {
   TT_CHECK_ARG(q && Xh && stats && topr && workspace, "null pointer");
   TT_CHECK_ARG(nq >= 1 && N_local >= 1 && N_local < (1LL << 31) && N_total >= N_local && D >= 1 && K >= 1, "bad sizes");
   TT_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "workspace must be 256-byte aligned");
@@ -227,13 +249,32 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_shard_sample(const
   unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
   if (int e = launch_prep_queries(q, nq, pl.nq_pad, D, pl.Dp, stats, reinterpret_cast<float*>(ws + w.qn), ws + w.qh,
                                   reinterpret_cast<float*>(ws + w.eps), nullptr, st)) return e;
-  return launch_sample(pl, ws + w.qh, Xh, N_local, nq, nullptr, topr, reinterpret_cast<float*>(ws + w.sample), st);
+  return launch_sample(pl, ws + w.qh, Xh, N_local, nq, nullptr, topr, reinterpret_cast<float*>(ws + w.sample), st,
+                       false, lab);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_shard_sample(const float* q, int nq, const void* Xh, const float* stats, int64_t N_local,
+                                    int64_t N_total, int D, int K, float* topr, void* workspace,
+                                    size_t workspace_bytes, void* stream) {
+  return flat_shard_sample_impl(q, nq, Xh, stats, N_local, N_total, D, K, topr, workspace, workspace_bytes, stream,
+                                LabelArgs{});
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_shard_sample_filtered(const float* q, int nq, const void* Xh, const float* stats,
+                                             int64_t N_local, int64_t N_total, int D, int K, const uint32_t* labels,
+                                             const uint32_t* require, float* topr, void* workspace,
+                                             size_t workspace_bytes, void* stream) {
+  LabelArgs lab;
+  const char* bad = label_args(labels, require, &lab);
+  TT_CHECK_ARG(bad == nullptr, bad);
+  return flat_shard_sample_impl(q, nq, Xh, stats, N_local, N_total, D, K, topr, workspace, workspace_bytes, stream, lab);
 }
 
 static int flat_shard_search_impl(int nq, const float* Xn, const void* Xh, int64_t N_local, int64_t N_total, int D,
                                   int K, int64_t id_offset, const float* topr_g, int G, float* scores, int64_t* ids,
                                   int32_t* flags, int32_t* n_uncertified, float* bound, const int64_t* excl, int E,
-                                  void* workspace, size_t workspace_bytes, void* stream) {
+                                  void* workspace, size_t workspace_bytes, void* stream,
+                                  const LabelArgs& lab = LabelArgs{}) {
   TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
   TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   TT_CHECK_ARG(Xn && Xh && topr_g && scores && ids && flags && n_uncertified && bound && workspace, "null pointer");
@@ -252,7 +293,7 @@ static int flat_shard_search_impl(int nq, const float* Xn, const void* Xh, int64
   float* thr = reinterpret_cast<float*>(ws + w.thr);
   unsigned int* cnt = reinterpret_cast<unsigned int*>(ws + w.cnt);
   if (int e = launch_select_gathered(topr_g, G, nq, pl.sample_rank, thr, n_uncertified, st)) return e;
-  if (int e = launch_main_scan(pl, ws + w.qh, Xh, N_local, nq, thr, cnt, ws + w.cand, st)) return e;
+  if (int e = launch_main_scan(pl, ws + w.qh, Xh, N_local, nq, thr, cnt, ws + w.cand, st, nullptr, lab)) return e;
   return launch_finalize(pl, qn, Xn, N_local, D, nq, K, id_offset, thr, eps, cnt, ws + w.cand, scores,
                          reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st,
                          reinterpret_cast<const long long*>(excl), E);
@@ -273,6 +314,19 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_shard_search_excl(
                                          void* stream) {
   return flat_shard_search_impl(nq, Xn, Xh, N_local, N_total, D, K, id_offset, topr_g, G, scores, ids, flags,
                                 n_uncertified, bound, excl, E, workspace, workspace_bytes, stream);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_shard_search_filtered(int nq, const float* Xn, const void* Xh, int64_t N_local,
+                                             int64_t N_total, int D, int K, int64_t id_offset, const float* topr_g,
+                                             int G, float* scores, int64_t* ids, int32_t* flags,
+                                             int32_t* n_uncertified, float* bound, const uint32_t* labels,
+                                             const uint32_t* require, const int64_t* excl, int E, void* workspace,
+                                             size_t workspace_bytes, void* stream) {
+  LabelArgs lab;
+  const char* bad = label_args(labels, require, &lab);
+  TT_CHECK_ARG(bad == nullptr, bad);
+  return flat_shard_search_impl(nq, Xn, Xh, N_local, N_total, D, K, id_offset, topr_g, G, scores, ids, flags,
+                                n_uncertified, bound, excl, E, workspace, workspace_bytes, stream, lab);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -187,26 +187,28 @@ class ShardedRetrievalPipeline:
         return ops.pool_partial_merge(gathered, self.attention)
 
     def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int, *,
-                              exclude_history: bool = False) -> PendingSearch:
+                              exclude_history: bool = False, require_all=0, require_any=0) -> PendingSearch:
         """exclude_history: the pooled history rows (global ids, -1 padded; the last `max_interaction_history`
-        interactions when built by RetrievalPipeline.encode_histories) are the exclusion list of the search."""
+        interactions when built by RetrievalPipeline.encode_histories) are the exclusion list of the search.
+        require_all / require_any: label masks, scalars or one per buyer, as in RetrievalPipeline (the words come from
+        ShardedFlatIPIndex.set_labels)."""
         k = min(k, self.n_total)                                                       # vector_db.py:159
+        req = require_masks(require_all, require_any, int(indices.shape[0]))
         emb = self.encode_device(indices, weights, k)
-        if not exclude_history:
-            return self.sharded.search_async(emb, k)
-        excl = indices.to(device=self.table.device, dtype=torch.int64).contiguous()
-        return self.sharded.search_async(emb, k, exclude=excl)
+        kw = {} if req is None else {"require": req}
+        if exclude_history:
+            kw["exclude"] = indices.to(device=self.table.device, dtype=torch.int64).contiguous()
+        return self.sharded.search_async(emb, k, **kw)
 
     def retrieve_host_async(self, idx_host: torch.Tensor, w_host: torch.Tensor, k: int, *,
-                            exclude_history: bool = False) -> PendingSearch:
+                            exclude_history: bool = False, require_all=0, require_any=0) -> PendingSearch:
         """Pinned host tensors in (history rows / weights of the WHOLE batch, the same on every rank), numpy out.
-        exclude_history: as in retrieve_device_async (the copied history rows are the list)."""
+        exclude_history: as in retrieve_device_async (the copied history rows are the list); require_all /
+        require_any: label masks as in retrieve_device_async."""
         dev = self.table.device
         idx_dev, w_dev = idx_host.to(dev, non_blocking=True), w_host.to(dev, non_blocking=True)
-        if exclude_history:
-            pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=True)
-        else:
-            pending = self.retrieve_device_async(idx_dev, w_dev, k)
+        pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=exclude_history,
+                                             require_all=require_all, require_any=require_any)
 
         def finish():
             s, i, n_bad = pending.result()

@@ -238,7 +238,8 @@ class ShardedFlatIPIndex:
 
     `local_index` provides `ntotal`, `search_shard_into(q, k_local, scores, ids, bound, flags)` and
     `search_exact_into(q, k_local, scores, ids, qsel)`, both writing the first k_local columns of the
-    [nq,k] record views (see FlatIPIndex).
+    [nq,k] record views (see FlatIPIndex).  Label filters also need `id_offset` (its first global row), `labels` and
+    `set_labels(words, rows=None)`; the local calls then get `require=` (a LabelMasks) next to `exclude=`.
     `merge(gathered[G,nbytes] uint8, layout, nq, k) -> (scores, ids, flags, n_uncertified)`.
     """
 
@@ -358,19 +359,70 @@ class ShardedFlatIPIndex:
         return world > 1 and n_local_min >= k and plan_ok is not None and plan_ok(self.n_total, nq, k, max(n_local_min, 0))
 
     @staticmethod
-    def _kw(exclude):
-        """Keyword arguments of the local calls: none without a list, so stand-ins that predate it keep working."""
-        return {} if exclude is None else {"exclude": exclude}
+    def _kw(exclude, require=None):
+        """Keyword arguments of the local calls: none without a list or a filter, so stand-ins that predate them keep
+        working."""
+        kw = {} if exclude is None else {"exclude": exclude}
+        if require is not None:
+            kw["require"] = require
+        return kw
+
+    # -- label filters ----------------------------------------------------------------------------------------
+    def set_labels(self, labels, rows=None) -> None:
+        """Sets label words in GLOBAL row order: `labels` [n_total] (each rank keeps the words of its rows), or one
+        word per listed global row id in `rows` (each rank applies the entries that fall in its shard).  Every rank calls
+        it with the same arguments; there is no communication.  Every rank ends up with a label array, zero-filled where
+        no word was given, so that a filtered search finds labels on every rank.  Values as in FlatIPIndex.set_labels."""
+        import numpy as np
+        from .vector_db import u32_words
+        words = u32_words(labels, "labels")
+        if isinstance(words, np.ndarray):
+            # as uint32, so that the local set_labels range check accepts words with bit 31 set (int32 reads them < 0)
+            words = words.view(np.uint32)
+        lo = int(self.local.id_offset)
+        hi = lo + int(self.local.ntotal)
+        if rows is None:
+            if tuple(words.shape) != (self.n_total,):
+                raise ValueError(f"expected one label word per catalog row ({self.n_total}), got shape {tuple(words.shape)}")
+            self.local.set_labels(words[lo:hi])
+            return
+        r = rows if isinstance(rows, torch.Tensor) else torch.from_numpy(np.asarray(rows))
+        if r.dim() != 1 or r.dtype not in (torch.int64, torch.int32) or tuple(words.shape) != (r.shape[0],):
+            raise ValueError(f"rows must be a 1-D integer array with one entry per label word, got rows "
+                             f"{r.dtype} {tuple(r.shape)} and labels {tuple(words.shape)}")
+        if r.numel() and (int(r.min()) < 0 or int(r.max()) >= self.n_total):
+            raise ValueError(f"rows must be in [0, {self.n_total})")
+        mine = (r >= lo) & (r < hi)
+        local_words = words[mine.cpu().numpy()] if isinstance(words, np.ndarray) else words[mine.to(words.device)]
+        self.local.set_labels(local_words, rows=(r[mine] - lo).to(torch.int64))
+
+    def _requires(self, require, nq: int, device):
+        """Per-query label masks ([nq, 2] or [2], numpy or CUDA, replicated on every rank) -> LabelMasks on `device`, or
+        None when every mask is (0, 0).  Decided on replicated values, so every rank takes the same branch; CUDA masks
+        cost one device-to-host read here, host masks none."""
+        from .vector_db import LabelMasks, u32_words
+        if require is None:
+            return None
+        w = u32_words(require, "require")
+        if tuple(w.shape) not in ((2,), (nq, 2)):
+            raise ValueError(f"require must be [nq={nq}, 2] or [2] ({{all, any}} masks), got shape {tuple(w.shape)}")
+        if not bool(w.any()):
+            return None
+        if getattr(self.local, "labels", None) is None:
+            raise ValueError("a label filter needs label words: call set_labels() first")
+        if not isinstance(w, torch.Tensor):
+            w = torch.from_numpy(w)
+        return LabelMasks(w.to(device, non_blocking=True).expand(nq, 2).contiguous())
 
     def _local_search(self, q: torch.Tensor, k: int, k_local: int, world: int, views, p2p=None, status=None,
-                      exclude=None) -> None:
+                      exclude=None, require=None) -> None:
         """Fills this rank's record.  With every shard holding >= k rows and a plan for it, all ranks use ONE
         threshold estimated from a sample of the whole catalog (a small all-gather of per-rank top-r sampled
         scores): candidates per rank drop to ~1/G of the single-device count.  Otherwise each shard picks its
         own threshold."""
         scores, ids, bound, flags = views
         nq = q.shape[0]
-        kw = self._kw(exclude)
+        kw = self._kw(exclude, require)
         if self._global_threshold(world, nq, k, exclude):
             from ._native import TT_SHARD_TOPR
             key = ("topr", nq, world)
@@ -388,7 +440,7 @@ class ShardedFlatIPIndex:
         else:
             self.local.search_shard_into(q, k_local, scores, ids, bound, flags, **kw)
 
-    def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
+    def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
         """Enqueues the sharded search of one batch and returns a PendingSearch; `.result()` looks at the global
         certificate later (no host sync between consecutive batches).
 
@@ -402,10 +454,13 @@ class ShardedFlatIPIndex:
         flight gets the full overlap; with fewer the stages simply run back to back.
 
         `exclude` (i64 [nq, E], GLOBAL ids, -1 = padding, replicated on every rank like q): the exact top-k over the
-        rows query i does not list; with fewer than k allowed rows the tail is (-inf, -1)."""
+        rows query i does not list; with fewer than k allowed rows the tail is (-inf, -1).
+        `require` ([nq, 2] or [2] {all, any} label masks, numpy or CUDA, replicated like q; see set_labels and
+        FlatIPIndex.search_device): only rows whose label word the query's masks allow; composes with `exclude`."""
         from .vector_db import PendingSearch
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         nq = q.shape[0]
+        require = self._requires(require, nq, q.device)
         if exclude is not None and exclude.shape[1] == 0:
             exclude = None
         self._validate(world, q.device)
@@ -414,7 +469,7 @@ class ShardedFlatIPIndex:
         p2p = self._p2p_for(nq, k, q.device, world, lay)
         global_thr = self._global_threshold(world, nq, k, exclude)
         if p2p is not None and global_thr:
-            return self._search_pipelined(q, k, nq, world, lay, rec, p2p, exclude)
+            return self._search_pipelined(q, k, nq, world, lay, rec, p2p, exclude, require)
         self.flush()          # never interleave the two schedules
         views = record_views(rec, lay, nq, k)
         scores, ids, bound, flags = views
@@ -423,19 +478,19 @@ class ShardedFlatIPIndex:
             ids.fill_(-1)
         if p2p is not None:
             status = self._bufs.setdefault(("status", nq, k, world), torch.zeros(2, dtype=torch.int32, device=q.device))
-            self._local_search(q, k, k_local, world, views, p2p, status, exclude)
+            self._local_search(q, k, k_local, world, views, p2p, status, exclude, require)
             gathered = p2p.all_gather(1, rec, status)
             s, i, fl, n_unc = self._merge(gathered, lay, nq, k, status[0:1])
             n_unc = status
         else:
-            self._local_search(q, k, k_local, world, views, exclude=exclude)
+            self._local_search(q, k, k_local, world, views, exclude=exclude, require=require)
             self._exchange(rec, gathered, world)
             s, i, fl, n_unc = self._merge(gathered, lay, nq, k)
         post = getattr(self.local, "post_flag", None)
         token = post(n_unc) if post is not None else None
-        return PendingSearch(lambda: self._finish(q, k, s, i, fl, n_unc, token, exclude))
+        return PendingSearch(lambda: self._finish(q, k, s, i, fl, n_unc, token, exclude, require))
 
-    def _finish(self, q, k, s, i, fl, n_unc, token, exclude=None):
+    def _finish(self, q, k, s, i, fl, n_unc, token, exclude=None, require=None):
         # identical on every rank: all ranks merged the same records
         st = self.local.read_flag(token) if token is not None else int(n_unc)
         if isinstance(st, list):
@@ -447,8 +502,11 @@ class ShardedFlatIPIndex:
             return s, i, 0
         # Re-run the flagged queries alone (this rank's record buffer may already hold a later batch):
         # exact fp32 search of every shard, a small exchange, merge, scatter into the result.
+        from .vector_db import LabelMasks
         rows = torch.nonzero(fl != 1).flatten()
         kw = {} if exclude is None else {"exclude": exclude[rows].contiguous()}
+        if require is not None:
+            kw["require"] = LabelMasks(require.words[rows].contiguous())
         s2, i2 = self.search_exact_device(q[rows].contiguous(), k, **kw)
         s[rows] = s2
         i[rows] = i2
@@ -457,7 +515,7 @@ class ShardedFlatIPIndex:
     # -- 3-stage pipeline -----------------------------------------------------------------------------------------
     NSLOT = 3      # batches in flight: workspaces / status words are per slot
 
-    def _search_pipelined(self, q, k, nq, world, lay, rec, p2p, exclude=None):
+    def _search_pipelined(self, q, k, nq, world, lay, rec, p2p, exclude=None, require=None):
         from ._native import TT_SHARD_TOPR
         from .vector_db import PendingSearch
         self._pipe_seq = getattr(self, "_pipe_seq", 0) + 1
@@ -466,9 +524,9 @@ class ShardedFlatIPIndex:
         topr = self._bufs.setdefault(("topr1", nq, world), torch.empty((nq, TT_SHARD_TOPR), device=dev, dtype=torch.float32))
         status = self._bufs.setdefault(("status", nq, k, world, slot), torch.zeros(2, dtype=torch.int32, device=dev))
         b = {"q": q, "k": k, "nq": nq, "world": world, "lay": lay, "rec": rec, "p2p": p2p, "slot": slot, "status": status,
-             "stage": 0, "out": None, "exclude": exclude}
+             "stage": 0, "out": None, "exclude": exclude, "require": require}
         # stage A: sample pass + push of the top-r lists (no wait)
-        self.local.shard_sample(q, k, self.n_total, topr, slot, **self._kw(exclude))
+        self.local.shard_sample(q, k, self.n_total, topr, slot, **self._kw(exclude, require))
         b["seq0"] = p2p.push(0, topr.view(torch.uint8).view(-1))
         b["stage"] = 1
         self._inflight.append(b)
@@ -486,7 +544,7 @@ class ShardedFlatIPIndex:
             topr_g = p2p.wait(0, b["seq0"], b["status"]).view(torch.float32).view(world, nq, TT_SHARD_TOPR)
             scores, ids, bound, flags = record_views(b["rec"], lay, nq, k)
             self.local.shard_search_into(nq, k, self.n_total, topr_g, scores, ids, bound, flags, b["slot"],
-                                         **self._kw(b["exclude"]))
+                                         **self._kw(b["exclude"], b["require"]))
             b["seq1"] = p2p.push(1, b["rec"])
             b["stage"] = 2
         if b["stage"] < 3 <= to_stage:          # stage C
@@ -510,17 +568,20 @@ class ShardedFlatIPIndex:
                     break
         self._inflight = [x for x in self._inflight if x["stage"] < 3]
         s, i, fl, token = b["out"]
-        return self._finish(b["q"], b["k"], s, i, fl, b["status"], token, b["exclude"])
+        return self._finish(b["q"], b["k"], s, i, fl, b["status"], token, b["exclude"], b["require"])
 
-    def search_exact_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
+    def search_exact_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
         """Always-exact fp32 path over the sharded catalog (collective: every rank calls it with the same q):
         fp32 exact search of every shard, one exchange of the records (NCCL / plain copy), merge.  Serves the
-        queries the global certificate rejects and the parity checks of bench.py / tests.  With `exclude` a query
-        may have fewer than k allowed rows: its merged list then ends in (-inf, -1), which is exact here."""
+        queries the global certificate rejects and the parity checks of bench.py / tests.  With `exclude` or `require`
+        a query may have fewer than k allowed rows: its merged list then ends in (-inf, -1), which is exact here."""
+        from .vector_db import LabelMasks
         if exclude is not None and exclude.shape[1] == 0:
             exclude = None
-        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         nsel = q.shape[0]
+        if not isinstance(require, LabelMasks):
+            require = self._requires(require, nsel, q.device)
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         k_local = min(k, self.local.ntotal)
         lay2 = record_layout(nsel, k)
         rec2 = torch.zeros(lay2.nbytes, dtype=torch.uint8, device=q.device)
@@ -532,33 +593,37 @@ class ShardedFlatIPIndex:
         f_l.fill_(1)
         if k_local > 0:
             self.local.search_exact_into(q, k_local, s_l, i_l, torch.arange(nsel, device=q.device, dtype=torch.int32),
-                                         **self._kw(exclude))
+                                         **self._kw(exclude, require))
         self._exchange(rec2, gathered2, world)
         s2, i2, fl2, n_unc2 = self._merge(gathered2, lay2, nsel, k)
-        if exclude is None:
+        if exclude is None and require is None:
             if int(n_unc2):
                 raise RuntimeError("sharded search: queries still uncertified after the exact re-run")
         elif bool(((fl2 != 1) & (fl2 != -2)).any()):     # -2 alone: fewer than k allowed rows, exact as padded
             raise RuntimeError("sharded search: queries still uncertified after the exact re-run")
         return s2, i2
 
-    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None):
+    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
         """q replicated on every rank -> global (scores, ids) [nq,k] on every rank, and the number of
         queries that failed the global certificate and were re-run through the exact path."""
-        return self.search_async(q, k, **self._kw(exclude)).result()
+        return self.search_async(q, k, **self._kw(exclude, require)).result()
 
-    def search_host_async(self, q, k: int, *, exclude=None):
+    def search_host_async(self, q, k: int, *, exclude=None, require=None):
         """numpy in / numpy out round trip (pinned staging), asynchronous; `.result()` -> (scores, ids, n_rerun).
-        `exclude`: numpy int64 [nq, E] global ids (see search_async)."""
+        `exclude`: numpy int64 [nq, E] global ids; `require`: label masks [nq, 2] or [2] (see search_async)."""
         from .vector_db import host_search_async
-        return host_search_async(self, self.search_async, self.local.device, self.local.d, q, k, exclude=exclude)
+        return host_search_async(self, self.search_async, self.local.device, self.local.d, q, k, exclude=exclude,
+                                 require=require)
 
-    def search_host_sliced_async(self, q_local, k: int):
+    def search_host_sliced_async(self, q_local, k: int, *, require=None):
         """Serving layout for G ranks fronting one sharded catalog: every rank submits ITS share of the batch
         (numpy [nq_local, D], the same row count on every rank).  The shares are all-gathered on the device (rank
         order = batch order), the whole batch is searched as usual, and each rank gets back the results of its own
         rows: host copies are nq_local*D*4 bytes in and nq_local*k*12 bytes out per rank instead of the whole batch
-        on every rank.  `.result()` -> (scores [nq_local,k], ids [nq_local,k], n_rerun) numpy."""
+        on every rank.  `.result()` -> (scores [nq_local,k], ids [nq_local,k], n_rerun) numpy.
+        `require`: the label masks of THIS rank's share, [nq_local, 2] or [2] (see search_async).  They are
+        all-gathered with the shares, so either every rank passes masks or none does.  Deciding whether the gathered
+        masks filter at all costs one device-to-host read."""
         import numpy as np
         from .vector_db import PendingSearch
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
@@ -568,6 +633,11 @@ class ShardedFlatIPIndex:
         if q_local.ndim != 2 or q_local.shape[1] != d:
             raise ValueError(f"expected queries [nq_local, {d}], got {q_local.shape}")
         nl = q_local.shape[0]
+        if require is not None:          # validated before the first collective: a bad mask raises, not hangs
+            from .vector_db import u32_words
+            w = u32_words(require, "require")
+            if tuple(w.shape) not in ((2,), (nl, 2)):
+                raise ValueError(f"require must be [nq_local={nl}, 2] or [2], got shape {tuple(w.shape)}")
         rings = self.__dict__.setdefault("_sliced_rings", {})
         ring = rings.get((nl, k))
         if ring is None:
@@ -594,7 +664,18 @@ class ShardedFlatIPIndex:
                 dist.all_gather_into_tensor(dq_all.view(-1), dq_local.view(-1), group=self.group)
             else:
                 dq_all[0].copy_(dq_local)
-            pending = self.search_async(dq_all.view(world * nl, d), k)
+            kw = {}
+            if require is not None:
+                if not isinstance(w, torch.Tensor):
+                    w = torch.from_numpy(w)
+                req_local = w.to(dev).expand(nl, 2).contiguous()
+                req_all = torch.empty((world, nl, 2), device=dev, dtype=torch.int32)
+                if world > 1:
+                    dist.all_gather_into_tensor(req_all.view(-1), req_local.view(-1), group=self.group)
+                else:
+                    req_all[0].copy_(req_local)
+                kw["require"] = req_all.view(world * nl, 2)
+            pending = self.search_async(dq_all.view(world * nl, d), k, **kw)
 
         def finish():
             scores, ids, n_bad = pending.result()

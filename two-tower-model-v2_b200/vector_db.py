@@ -15,7 +15,7 @@ from __future__ import annotations
 import json
 import struct
 from pathlib import Path
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import numpy as np
 import torch
@@ -165,6 +165,13 @@ def require_masks(require_all, require_any, nq: int) -> Optional[np.ndarray]:
         cols.append(np.broadcast_to(w, (nq,)))
     req = np.ascontiguousarray(np.stack(cols, 1))
     return req if req.any() else None
+
+
+class LabelMasks(NamedTuple):
+    """Label masks already validated: int32 [nq, 2] on the index's device, at least one of them not (0, 0).
+    ShardedFlatIPIndex normalises `require` into this once per batch, so that the per-shard calls of that batch neither
+    validate the masks again nor read them back to the host (which would stall the pipelined schedule)."""
+    words: torch.Tensor
 
 
 # ---------------------------------------------------------------------------------------------
@@ -385,6 +392,14 @@ class FlatIPIndex:
         on this device, or None when every query's masks are (0, 0): the unfiltered search runs."""
         if require is None:
             return None
+        if isinstance(require, LabelMasks):
+            w = require.words
+            if tuple(w.shape) != (nq, 2) or w.dtype != torch.int32 or w.device != self.device or not w.is_contiguous():
+                raise ValueError(f"LabelMasks must hold contiguous int32 [nq={nq}, 2] words on {self.device}, got "
+                                 f"{w.dtype} {tuple(w.shape)} on {w.device}")
+            if self.labels is None:
+                raise ValueError("a label filter needs label words: call set_labels() first")
+            return w
         w = u32_words(require, "require")
         if tuple(w.shape) not in ((2,), (nq, 2)):
             raise ValueError(f"require must be [nq={nq}, 2] or [2] ({{all, any}} masks), got shape {tuple(w.shape)}")
@@ -516,10 +531,13 @@ class FlatIPIndex:
         return scores, ids
 
     def search_shard_into(self, q: torch.Tensor, k: int, scores: torch.Tensor, ids: torch.Tensor,
-                          bound: torch.Tensor, flags: torch.Tensor, *, exclude: Optional[torch.Tensor] = None) -> None:
+                          bound: torch.Tensor, flags: torch.Tensor, *, exclude: Optional[torch.Tensor] = None,
+                          require=None) -> None:
         """Shard-local search for ShardedFlatIPIndex (tt_flat_search_shard): fills the caller's record views.
         scores/ids are [nq, k_record] with k_record >= k; only the first k columns of each row are written.
-        `exclude` holds GLOBAL ids (ids of other shards are ignored here)."""
+        `exclude` holds GLOBAL ids (ids of other shards are ignored here); `require`: label masks as in search_device,
+        tested against this shard's label words."""
+        req = self._requires(require, q.shape[0])
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
         excl = self._exclusions(exclude, nq)
@@ -529,7 +547,15 @@ class FlatIPIndex:
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
         lib = _native.load()
         with torch.cuda.device(self.device):
-            if excl is None:
+            if req is not None:
+                E = 0 if excl is None else excl.shape[1]
+                ws = self._workspace(max(nq, 1), k, E)
+                _native.check(lib.tt_flat_search_shard_filtered(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, s_out.data_ptr(), i_out.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    bound.data_ptr(), self.labels.data_ptr(), req.data_ptr(), 0 if excl is None else excl.data_ptr(), E,
+                    ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_search_shard_filtered")
+            elif excl is None:
                 ws = self._workspace(max(nq, 1), k)
                 _native.check(lib.tt_flat_search_shard(
                     q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
@@ -547,9 +573,11 @@ class FlatIPIndex:
             ids[:, :k].copy_(i_out)
 
     def search_exact_into(self, q: torch.Tensor, k: int, scores: torch.Tensor, ids: torch.Tensor,
-                          qsel: torch.Tensor, *, exclude: Optional[torch.Tensor] = None) -> None:
+                          qsel: torch.Tensor, *, exclude: Optional[torch.Tensor] = None, require=None) -> None:
         """Exact fp32 re-run of the query rows `qsel`, written into [nq, k_record] record views."""
         kw = {} if exclude is None else {"exclude": exclude}
+        if require is not None:
+            kw["require"] = require
         if scores.shape[1] == k and scores.is_contiguous() and ids.is_contiguous():
             self.search_exact_device(q, k, scores, ids, qsel, **kw)
             return
@@ -623,30 +651,50 @@ class FlatIPIndex:
         return ws
 
     def shard_sample(self, q: torch.Tensor, k: int, n_total: int, topr: torch.Tensor, slot: int = 0, *,
-                     exclude: Optional[torch.Tensor] = None) -> None:
+                     exclude: Optional[torch.Tensor] = None, require=None) -> None:
         """Phase 1 of the sharded search: fills topr f32 [nq, TT_SHARD_TOPR] (this shard's largest sampled scores).
         `slot` selects the workspace (phase 2 of the same batch must use the same slot; batches in flight at the same
         time need different slots).  With `exclude` [nq, E] the sample is planned for K_plan = min(k + E, n_total,
-        TT_FLAT_MAX_K); phase 2 must get the same list."""
+        TT_FLAT_MAX_K); phase 2 must get the same list.  With `require` (label masks, see search_device) only the
+        allowed rows are sampled; phase 2 must get the same masks."""
+        req = self._requires(require, q.shape[0])
         if exclude is not None and exclude.shape[1] > 0:
             k = _native.plan_k(k, exclude.shape[1], n_total)
         q = ops._f32c(q, "queries")
         ws = self._shard_workspace(n_total, q.shape[0], k, slot)
+        lib = _native.load()
         with torch.cuda.device(self.device):
-            _native.check(_native.load().tt_flat_shard_sample(
-                q.data_ptr(), q.shape[0], self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, n_total, self.d, k,
-                topr.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_shard_sample")
+            if req is not None:
+                _native.check(lib.tt_flat_shard_sample_filtered(
+                    q.data_ptr(), q.shape[0], self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, n_total, self.d, k,
+                    self.labels.data_ptr(), req.data_ptr(), topr.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()),
+                    "tt_flat_shard_sample_filtered")
+            else:
+                _native.check(lib.tt_flat_shard_sample(
+                    q.data_ptr(), q.shape[0], self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, n_total, self.d, k,
+                    topr.data_ptr(), ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_shard_sample")
 
     def shard_search_into(self, nq: int, k: int, n_total: int, topr_g: torch.Tensor, scores: torch.Tensor,
                           ids: torch.Tensor, bound: torch.Tensor, flags: torch.Tensor, slot: int = 0, *,
-                          exclude: Optional[torch.Tensor] = None) -> None:
+                          exclude: Optional[torch.Tensor] = None, require=None) -> None:
         """Phase 2: global threshold from the gathered lists [G, nq, TT_SHARD_TOPR], main scan, finalize into
-        the record views (scores/ids must be contiguous [nq,k]).  `exclude`: the list phase 1 was given."""
+        the record views (scores/ids must be contiguous [nq,k]).  `exclude`, `require`: the list and the masks phase 1
+        was given."""
+        req = self._requires(require, nq)
         excl = self._exclusions(exclude, nq)
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
         lib = _native.load()
         with torch.cuda.device(self.device):
-            if excl is None:
+            if req is not None:
+                E = 0 if excl is None else excl.shape[1]
+                ws = self._shard_workspace(n_total, nq, _native.plan_k(k, E, n_total), slot)
+                _native.check(lib.tt_flat_shard_search_filtered(
+                    nq, self.xn.data_ptr(), self.xh.data_ptr(), self.ntotal, n_total, self.d, k, self.id_offset,
+                    topr_g.data_ptr(), topr_g.shape[0], scores.data_ptr(), ids.data_ptr(), flags.data_ptr(),
+                    nunc.data_ptr(), bound.data_ptr(), self.labels.data_ptr(), req.data_ptr(),
+                    0 if excl is None else excl.data_ptr(), E, ws.data_ptr(), ws.numel(), ops._stream()),
+                    "tt_flat_shard_search_filtered")
+            elif excl is None:
                 ws = self._shard_workspace(n_total, nq, k, slot)
                 _native.check(lib.tt_flat_shard_search(
                     nq, self.xn.data_ptr(), self.xh.data_ptr(), self.ntotal, n_total, self.d, k, self.id_offset,
