@@ -257,6 +257,59 @@ int tt_flat_search_exact_filtered(const float* q, int nq, const int32_t* qsel, i
                                   const int64_t* excl, int E,
                                   void* workspace, size_t workspace_bytes, void* stream);
 
+/* Range search: every row whose fp32 score is STRICTLY greater than a per-query radius (faiss's inner-product
+ * range_search), how many there are, and the best L of them.
+ *   radius  f32 [nq]      finite; queries are renormalised as in tt_flat_search
+ *   L       1 <= L <= TT_FLAT_RANGE_MAX_RESULTS (L may exceed N)
+ *   counts  i64 [nq]      exact number of rows above the radius that are allowed (labels / require) and not excluded
+ *                         (excl), whether or not the list below was truncated
+ *   scores  f32 [nq, L], ids i64 [nq, L]   the best min(counts[q], L) of them (row + id_offset), ordered by (score
+ *                         desc, id asc); the tail is score -inf / id -1
+ *   flags   i32 [nq]      1 = certified exact; <= 0 = -(reason bits): 1 a candidate segment overflowed (need[q] holds
+ *                         the query's largest segment count: a re-run with the same nq, whose segments hold need[q]
+ *                         candidates, fits it; a re-run with fewer queries may slice the catalog differently),
+ *                         2 more candidates within reach of the L-th result than one CTA ranks, 4 score self-check
+ *                         failed, 8 the L-th result does not clear the bound of the rows that were not rescored.  Re-run
+ *                         a query with bit 1 through tt_flat_range_search with a larger workspace, any other through
+ *                         tt_flat_range_search_exact.
+ *   need    i32 [nq]      largest number of candidates one (query, catalog slice) segment received
+ *   n_uncertified i32 [1] number of flags != 1
+ *   labels, require       label filter as in tt_flat_search_filtered: both NULL (no filter) or both non-NULL
+ *   excl, E               exclusion lists as in tt_flat_search_excl (E = 0 without a list)
+ * The scan keeps every row whose bf16 score is >= thr = radius - eps (rounded toward -inf), eps the per-query bound
+ * on |bf16 score - fp32 score|: no sample pass and no threshold selection.  A candidate with a bf16 score above
+ * radius + eps is counted without rescoring; the band in between is rescored in fp32.  The best L are chosen like the
+ * top-K finalize does (L-th largest bf16 score, rescoring within PRUNE_MARGIN * eps of it) and certified the same way.
+ * Candidate room: tt_flat_range_workspace_bytes(N, D, nq, cand_budget) sizes the workspace for about cand_budget
+ * candidates per query (each of the plan's catalog slices holds twice an even share); tt_flat_range_search sizes its
+ * segments from the workspace_bytes it is given, so a larger workspace gives more room.  Widths the scan does not take
+ * (D > 1024) run the exact path inside tt_flat_range_search (flags 1, need 0).  Ids are row + id_offset, so a shard can
+ * call the same entry point.
+ * tt_flat_range_search_exact: CUDA-core fp32 over every row (the exact path of tt_flat_search_exact), same outputs for
+ * the query rows qsel[i] (NULL = all nq, nsel = nq); labels / require / excl of the QUERY row.  Its workspace is
+ * tt_flat_range_exact_workspace_bytes(N, D, nsel, L). */
+#define TT_FLAT_RANGE_MAX_RESULTS 16384
+size_t tt_flat_range_workspace_bytes(int64_t N, int D, int nq, int64_t cand_budget);
+int tt_flat_range_search(const float* q, int nq,
+                         const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
+                         const float* radius, int L, int64_t id_offset,
+                         int64_t* counts, float* scores, int64_t* ids, int32_t* flags, int32_t* need,
+                         int32_t* n_uncertified,
+                         const uint32_t* labels, const uint32_t* require,
+                         const int64_t* excl, int E,
+                         void* workspace, size_t workspace_bytes, void* stream);
+size_t tt_flat_range_exact_workspace_bytes(int64_t N, int D, int nsel, int L);
+/* Diagnostic: after a tt_flat_range_search call on the tensor-core path that used `workspace`, copy out every query's
+ * candidate count, summed over its segments before the capacity clamp (device pointer cnt_out i32 [nq]). */
+int tt_flat_range_debug_read(const void* workspace, int64_t N, int D, int nq, int32_t* cnt_out, void* stream);
+int tt_flat_range_search_exact(const float* q, int nq, const int32_t* qsel, int nsel,
+                               const float* Xn, int64_t N, int D,
+                               const float* radius, int L, int64_t id_offset,
+                               int64_t* counts, float* scores, int64_t* ids,
+                               const uint32_t* labels, const uint32_t* require,
+                               const int64_t* excl, int E,
+                               void* workspace, size_t workspace_bytes, void* stream);
+
 /* Merge G per-shard sorted top-K lists into one: scores_g f32 [G, nq, K], ids_g i64 [G, nq, K]
  * (the layout an all-gather of per-rank [nq,K] results produces) -> [nq, K], same ordering
  * (score descending, id ascending). */
@@ -372,7 +425,8 @@ int tt_p2p_wait(const int32_t* flags, int G, int32_t seq, double timeout_seconds
                 void* stream);
 
 /* Measurement hooks (bench.py).  tt_kernel_launch_count: kernels this library has launched in this
- * process.  tt_profile_scan_arm(n): the next n main-scan launches of tt_flat_search are bracketed by
+ * process.  tt_profile_scan_arm(n): the next n main-scan launches of tt_flat_search (and of the other searches,
+ * tt_flat_range_search included) are bracketed by
  * CUDA events on their stream; tt_profile_scan_read: waits for them, writes their durations in ms,
  * returns how many were recorded (-1 on a CUDA error) and disarms. */
 int64_t tt_kernel_launch_count(void);

@@ -17,6 +17,7 @@ LIB_PATH = _HERE / "lib" / "libtt_b200.so"
 TT_FLAT_MAX_K = 2048
 TT_SHARD_TOPR = 32
 TT_FLAT_MAX_EXCLUDE = 1024
+TT_FLAT_RANGE_MAX_RESULTS = 16384
 ABI_VERSION = 1
 
 
@@ -77,6 +78,15 @@ SIGNATURES = {
     "tt_flat_shard_search_filtered": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64,
                                               c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                               c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_range_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int64]),
+    "tt_flat_range_search": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_int, c_int64,
+                                     c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_range_exact_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int]),
+    "tt_flat_range_debug_read": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p]),
+    "tt_flat_range_search_exact": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_void_p, c_int,
+                                           c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                           c_void_p, c_size_t, c_void_p]),
     "tt_flat_shard_plan_ok":(c_int, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int, c_int, c_int]),
     "tt_flat_shard_sample": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_void_p,

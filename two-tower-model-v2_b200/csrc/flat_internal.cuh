@@ -63,6 +63,16 @@ int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long l
                     const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
                     float* bound_out, cudaStream_t st, const long long* excl = nullptr, int E = 0);
 
+// Range search (flat_range.cu): the scan plan of make_scan_plan's tiling and slices, with candidate segments sized for
+// about cand_budget candidates per query (twice an even share per slice).  No sample pass.
+ScanPlan make_range_plan(long long N, int D, int nq, long long cand_budget);
+
+// One group of nslot <= EX_QB query slots of the exact path (flat_select.cu; see its definition)
+constexpr int EX_QB = 8;   // queries scored per pass over the fp32 table
+int launch_exact_group(const float* q, const int32_t* qsel, int slot0, int nslot, const float* Xn, long long N, int D, int K,
+                       long long id_offset, float* scores, int64_t* ids, bool out_by_query, const int64_t* excl, int E,
+                       const uint32_t* labels, const uint32_t* require, void* workspace, cudaStream_t st);
+
 // shared TMA descriptor helper (flat_scan.cu) and the tensor-core attention-logits launcher (attn_logits_tc.cu)
 int make_tmap_f32(void* tensor_map /* CUtensorMap* */, const void* base, long long rows, int cols, int box_rows, int box_cols);
 int launch_attn_logits_tc(const float* x, long long R, int D, const float* W1, const float* b1, const float* W2,

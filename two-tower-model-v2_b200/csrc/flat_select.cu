@@ -8,102 +8,9 @@
 // fp32 inner products, k largest, sorted descending, int64 labels.
 #include "tt_common.cuh"
 #include "flat_internal.cuh"
+#include "flat_select_common.cuh"
 
 namespace tt {
-
-// In-place bitonic sort of P (power of two) keys in shared memory, descending.
-template <typename T>
-__device__ __forceinline__ void bitonic_sort_desc(T* key, int P) {
-  for (int k = 2; k <= P; k <<= 1) {
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      for (int i = threadIdx.x; i < P; i += blockDim.x) {
-        const int ixj = i ^ j;
-        if (ixj > i) {
-          const T a = key[i], b = key[ixj];
-          const bool up = (i & k) == 0;          // "up" blocks are sorted descending
-          if (up ? (a < b) : (a > b)) { key[i] = b; key[ixj] = a; }
-        }
-      }
-      __syncthreads();
-    }
-  }
-}
-
-__device__ __forceinline__ int next_pow2(int n) {
-  int p = 1;
-  while (p < n) p <<= 1;
-  return p;
-}
-
-// fp32 dot of a shared-memory query with a global row, warp-cooperative.
-__device__ __forceinline__ float warp_dot(const float* __restrict__ qs, const float* __restrict__ row, int D,
-                                          int lane, bool vec) {
-  float a = 0.f;
-  if (vec) {
-    const float4* r4 = reinterpret_cast<const float4*>(row);
-    const float4* q4 = reinterpret_cast<const float4*>(qs);
-    for (int c = lane; c < (D >> 2); c += 32) {
-      const float4 x = __ldg(r4 + c);
-      const float4 y = q4[c];
-      a = fmaf(x.x, y.x, a); a = fmaf(x.y, y.y, a); a = fmaf(x.z, y.z, a); a = fmaf(x.w, y.w, a);
-    }
-  } else {
-    for (int d = lane; d < D; d += 32) a = fmaf(__ldg(row + d), qs[d], a);
-  }
-  return warp_sum(a);
-}
-
-// ------------------------------------------------------------------------------------------
-// Per-query exclusion lists (tt_flat_search_excl & co.): excl i64 [nq, E], entry = local row + id_offset; entries
-// below 0 are padding, ids outside [id_offset, id_offset + N) are ignored, duplicates are harmless.  A CTA stages
-// its query's list in shared memory as local rows sorted descending; EXCL_NONE fills the unused slots (rows are
-// < 2^31, so it never matches one).  Membership is then a binary search.
-constexpr unsigned int EXCL_NONE = 0xffffffffu;
-
-// ex[j] for j < P (P = next_pow2(E)); returns true if the query excludes a row of this shard.  No barrier.
-__device__ __forceinline__ bool stage_exclusions(const long long* __restrict__ excl, int E, int q, long long id_offset,
-                                                 long long N, unsigned int* ex, int P) {
-  bool any = false;
-  for (int j = threadIdx.x; j < P; j += blockDim.x) {
-    unsigned int v = EXCL_NONE;
-    if (j < E) {
-      const long long id = excl[(long long)q * E + j];
-      const long long r = id - id_offset;
-      if (id >= 0 && r >= 0 && r < N) { v = (unsigned int)r; any = true; }
-    }
-    ex[j] = v;
-  }
-  return any;
-}
-
-__device__ __forceinline__ bool is_excluded(const unsigned int* ex, int P, unsigned int row) {
-  int lo = 0, hi = P;   // first position whose entry is <= row (the list is descending)
-  while (lo < hi) { const int mid = (lo + hi) >> 1; if (ex[mid] > row) lo = mid + 1; else hi = mid; }
-  return lo < P && ex[lo] == row;
-}
-
-// In-place, order-keeping compaction of key[0, n) to the keys `keep(key)` accepts; returns the new count.  Chunks of
-// NT keys move left only, so a chunk never overwrites keys not yet read.  n must be the same in every thread.
-template <int NT, typename Keep>
-__device__ __forceinline__ int compact_keys(unsigned long long* key, int n, int* s_wsum, Keep keep_fn) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int out = 0;
-  for (int base = 0; base < n; base += NT) {
-    const int i = base + (int)threadIdx.x;
-    const unsigned long long kk64 = (i < n) ? key[i] : 0ull;
-    const bool keep = (i < n) && keep_fn(kk64);
-    const unsigned int bal = __ballot_sync(0xffffffffu, keep);
-    if (lane == 0) s_wsum[warp] = __popc(bal);
-    __syncthreads();                       // also orders every read of this chunk before the writes below
-    int wbase = 0, tot = 0;
-#pragma unroll
-    for (int w = 0; w < NT / 32; ++w) { const int c = s_wsum[w]; if (w < warp) wbase += c; tot += c; }
-    if (keep) key[out + wbase + __popc(bal & ((1u << lane) - 1u))] = kk64;
-    out += tot;
-    __syncthreads();
-  }
-  return out;
-}
 
 // ------------------------------------------------------------------------------------------
 // finalize: one CTA per query.
@@ -116,6 +23,8 @@ __device__ __forceinline__ int compact_keys(unsigned long long* key, int n, int*
 //      c = max(scan threshold, cutoff), hence an fp32 score below c + eps.  If the K-th best rescored
 //      fp32 score f_K >= c + eps, no such row can enter the top-K: the result is exact.  Otherwise the
 //      query is flagged and the host re-runs it through the exact path.
+// Twins in flat_select_common.cuh: radix_select_desc and rescore_rows restate steps 2 and 4 for the range finalize
+// (flat_range.cu), which must give a row the same fp32 score as this kernel; change them together.
 // EXCL (exclusion lists): right after the gather, candidates whose row the query excludes are dropped, so n, b_K,
 // the cutoff and m all count allowed rows only, and the certificate reads "every ALLOWED row not rescored has a
 // bf16 score < c".  Excluded rows are typically a query's best ones: the caller plans the scan for
@@ -123,7 +32,6 @@ __device__ __forceinline__ int compact_keys(unsigned long long* key, int n, int*
 constexpr int FIN_THREADS = 256;          // large batches: one 256-thread CTA per query, several CTAs per SM
 constexpr int FIN_THREADS_WIDE = 1024;    // small batches (fewer queries than SMs): the latency-bound phases of the
                                           // single query (gather, fp32 rescoring of ~200 scattered rows) get 4x the warps
-constexpr float PRUNE_MARGIN = 1.5f;       // in units of eps; typical |bf16 - fp32| is ~eps/25
 constexpr int RANK_BY_COUNT_MAX = 1024;    // survivors up to this many are ranked by counting, else bitonic sort
 
 template <int FIN_THREADS, bool EXCL>
@@ -539,8 +447,6 @@ shard_merge_kernel(const unsigned char* __restrict__ gathered, size_t rank_strid
 
 // ------------------------------------------------------------------------------------------
 // exact path
-constexpr int EX_QB = 8;   // queries scored per pass over the fp32 table
-
 struct SelState {
   unsigned long long prefix;   // bits of the K-th key decided so far
   int kremain;                 // rank still to resolve inside the current prefix bucket
@@ -766,6 +672,61 @@ static size_t exact_ws_layout(int64_t N, int K, size_t* off_state, size_t* off_h
   return o;
 }
 
+namespace tt {
+// One group of nslot <= EX_QB query slots of the exact path; slot s serves query row qi = qsel[slot0 + s] (slot0 + s
+// without qsel).  fp32 scores of every row go to the first EX_QB * N floats of `workspace` (rows the query excludes or
+// does not allow hold EXCL_SCORE_BITS), then the exact top-K of each slot is written to row qi of scores / ids [*, K]
+// (out_by_query), or to row s.  workspace: exact_ws_layout(N, K) bytes.
+int launch_exact_group(const float* q, const int32_t* qsel, int slot0, int nslot, const float* Xn, long long N, int D, int K,
+                       long long id_offset, float* scores, int64_t* ids, bool out_by_query, const int64_t* excl, int E,
+                       const uint32_t* labels, const uint32_t* require, void* workspace, cudaStream_t st) {
+  size_t o_state, o_hist, o_keys;
+  (void)exact_ws_layout(N, K, &o_state, &o_hist, &o_keys);
+  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
+  float* scores_ws = reinterpret_cast<float*>(ws);
+  SelState* state = reinterpret_cast<SelState*>(ws + o_state);
+  unsigned int* hist = reinterpret_cast<unsigned int*>(ws + o_hist);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + o_keys);
+  const int sms = num_sms();
+  const size_t smem_q = (size_t)EX_QB * D * sizeof(float);
+  TT_CHECK_CUDA(cudaFuncSetAttribute(exact_scores_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q));
+  int P = 1;
+  while (P < K) P <<= 1;
+  if ((size_t)P * 8 > 48 * 1024)   // K > 4096: only the range search's exact path selects that many
+    TT_CHECK_CUDA(cudaFuncSetAttribute(exact_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, P * 8));
+  long long gs = (N + 255) / 256;
+  if (gs > (long long)sms * 8) gs = (long long)sms * 8;
+  long long gw = (N + 7) / 8;
+  if (gw > (long long)sms * 4) gw = (long long)sms * 4;
+  exact_scores_kernel<<<(unsigned)gw, 256, smem_q, st>>>(q, qsel, slot0, nslot, Xn, N, D, scores_ws);
+  TT_CHECK_LAUNCH();
+  if (E > 0) {
+    exact_exclude_kernel<<<nslot, 256, 0, st>>>(reinterpret_cast<const long long*>(excl), E, qsel, slot0, id_offset, N,
+                                                scores_ws);
+    TT_CHECK_LAUNCH();
+  }
+  if (labels) {
+    exact_filter_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(labels, require, qsel, slot0, N, scores_ws);
+    TT_CHECK_LAUNCH();
+  }
+  exact_init_kernel<<<(nslot * 256 + 255) / 256, 256, 0, st>>>(state, hist, nslot, K);
+  TT_CHECK_LAUNCH();
+  for (int shift = 56; shift >= 0; shift -= 8) {
+    exact_hist_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(scores_ws, N, state, hist, shift);
+    TT_CHECK_LAUNCH();
+    exact_pick_kernel<<<nslot, 256, 0, st>>>(state, hist, shift);
+    TT_CHECK_LAUNCH();
+  }
+  exact_collect_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(scores_ws, N, state, keys, K);
+  TT_CHECK_LAUNCH();
+  exact_sort_kernel<<<nslot, 256, (size_t)P * 8, st>>>(keys, out_by_query ? qsel : nullptr, out_by_query ? slot0 : 0, K,
+                                                       id_offset, scores, reinterpret_cast<long long*>(ids),
+                                                       E > 0 || labels != nullptr);
+  TT_CHECK_LAUNCH();
+  return TT_OK;
+}
+}  // namespace tt
+
 extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_exact_workspace_bytes(int64_t N, int D, int nsel, int K) {
   (void)D; (void)nsel;
   size_t a, b, c;
@@ -786,47 +747,10 @@ static int flat_search_exact_impl(const float* q, int nq, const int32_t* qsel, i
   const size_t need = exact_ws_layout(N, K, &o_state, &o_hist, &o_keys);
   if (workspace_bytes < need) { set_error("tt_flat_search_exact: workspace too small"); return TT_ERR_WORKSPACE; }
   cudaStream_t st = (cudaStream_t)stream;
-  unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
-  float* scores_ws = reinterpret_cast<float*>(ws);
-  SelState* state = reinterpret_cast<SelState*>(ws + o_state);
-  unsigned int* hist = reinterpret_cast<unsigned int*>(ws + o_hist);
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + o_keys);
-
-  const int sms = num_sms();
-  const size_t smem_q = (size_t)EX_QB * D * sizeof(float);
-  TT_CHECK_CUDA(cudaFuncSetAttribute(exact_scores_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_q));
-  int P = 1;
-  while (P < K) P <<= 1;
-  long long gs = (N + 255) / 256;
-  if (gs > (long long)sms * 8) gs = (long long)sms * 8;
   for (int slot0 = 0; slot0 < nsel; slot0 += EX_QB) {
     const int nslot = (nsel - slot0 < EX_QB) ? (nsel - slot0) : EX_QB;
-    long long gw = (N + 7) / 8;
-    if (gw > (long long)sms * 4) gw = (long long)sms * 4;
-    exact_scores_kernel<<<(unsigned)gw, 256, smem_q, st>>>(q, qsel, slot0, nslot, Xn, N, D, scores_ws);
-    TT_CHECK_LAUNCH();
-    if (E > 0) {
-      exact_exclude_kernel<<<nslot, 256, 0, st>>>(reinterpret_cast<const long long*>(excl), E, qsel, slot0, id_offset, N,
-                                                  scores_ws);
-      TT_CHECK_LAUNCH();
-    }
-    if (labels) {
-      exact_filter_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(labels, require, qsel, slot0, N, scores_ws);
-      TT_CHECK_LAUNCH();
-    }
-    exact_init_kernel<<<(nslot * 256 + 255) / 256, 256, 0, st>>>(state, hist, nslot, K);
-    TT_CHECK_LAUNCH();
-    for (int shift = 56; shift >= 0; shift -= 8) {
-      exact_hist_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(scores_ws, N, state, hist, shift);
-      TT_CHECK_LAUNCH();
-      exact_pick_kernel<<<nslot, 256, 0, st>>>(state, hist, shift);
-      TT_CHECK_LAUNCH();
-    }
-    exact_collect_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(scores_ws, N, state, keys, K);
-    TT_CHECK_LAUNCH();
-    exact_sort_kernel<<<nslot, 256, (size_t)P * 8, st>>>(keys, qsel, slot0, K, id_offset, scores,
-                                                         reinterpret_cast<long long*>(ids), E > 0 || labels != nullptr);
-    TT_CHECK_LAUNCH();
+    if (int e = launch_exact_group(q, qsel, slot0, nslot, Xn, N, D, K, id_offset, scores, ids, true, excl, E, labels, require,
+                                   workspace, st)) return e;
   }
   return TT_OK;
 }

@@ -175,6 +175,53 @@ class LabelMasks(NamedTuple):
 
 
 # ---------------------------------------------------------------------------------------------
+# Range search helpers (host side)
+def range_max_results(max_results) -> int:
+    """max_results -> int in [1, TT_FLAT_RANGE_MAX_RESULTS]; anything else raises ValueError."""
+    if isinstance(max_results, (bool, np.bool_)) or not isinstance(max_results, (int, np.integer)):
+        raise ValueError(f"max_results must be an integer, got {type(max_results).__name__}")
+    if not 1 <= int(max_results) <= _native.TT_FLAT_RANGE_MAX_RESULTS:
+        raise ValueError(f"max_results must be in [1, {_native.TT_FLAT_RANGE_MAX_RESULTS}], got {max_results}")
+    return int(max_results)
+
+
+def range_csr(counts: np.ndarray, scores: np.ndarray, ids: np.ndarray):
+    """Padded per-query range results (counts [nq]; scores / ids [nq, L], best first, (-inf, -1) tail) -> faiss's
+    range_search layout (lims i64 [nq + 1], D f32 [total], I i64 [total]); query i keeps min(counts[i], L) entries."""
+    counts = np.asarray(counts, np.int64)
+    scores, ids = np.asarray(scores), np.asarray(ids)
+    n = np.minimum(counts, scores.shape[1])
+    lims = np.zeros(counts.shape[0] + 1, np.int64)
+    np.cumsum(n, out=lims[1:])
+    keep = np.arange(scores.shape[1])[None, :] < n[:, None]
+    return lims, scores[keep].astype(np.float32), ids[keep].astype(np.int64)
+
+
+def range_rerun_groups(rows: np.ndarray, need: np.ndarray, ws_bytes, budget_bytes: int):
+    """The overflowed query rows of a range search, in re-run groups: ascending need, each group as large as its
+    workspace ws_bytes(n_queries, largest_need) fits budget_bytes.  A row that does not fit alone forms a group of one."""
+    rows = np.asarray(rows, np.int64)
+    order = rows[np.argsort(np.asarray(need)[rows], kind="stable")]
+    groups, cur = [], []
+    for r in order.tolist():
+        if cur and ws_bytes(len(cur) + 1, int(need[r])) > budget_bytes:
+            groups.append(np.array(cur, np.int64))
+            cur = []
+        cur.append(r)
+    if cur:
+        groups.append(np.array(cur, np.int64))
+    return groups
+
+
+def _plan_slices(n: int, d: int, nq: int) -> int:
+    """Catalog slices of the scan plan for nq queries (the range search keeps the top-K planner's slices)."""
+    import ctypes
+    out = (ctypes.c_int32 * 16)()
+    _native.check(_native.load().tt_flat_plan_describe(n, d, nq, 1, out), "tt_flat_plan_describe")
+    return int(out[13])
+
+
+# ---------------------------------------------------------------------------------------------
 class _FlagRing:
     """A few pinned int32 slots: the status words of a search (uncertified count[, exchange time-out]) are
     copied into one of them asynchronously, so the host can look at them later without draining the stream.
@@ -627,6 +674,188 @@ class FlatIPIndex:
         """search_device + re-run of uncertified queries through the exact path (one host sync)."""
         return self.search_async(q, k, exclude=exclude, require=require).result()
 
+    # -- range search (tt_flat_range_search) -----------------------------------------------------
+    # Bytes of workspace one range call takes at most: the first pass sizes its candidate budget to fit, and the
+    # re-runs of overflowed queries run in groups that fit.
+    RANGE_WS_BUDGET = 2 << 30
+
+    def _radii(self, radius, nq: int) -> torch.Tensor:
+        """A Python float (every query), or a numpy / CUDA [nq] array -> contiguous f32 [nq] on this device.  A bad shape
+        or a non-finite radius (after the cast to f32) raises ValueError; a CUDA radius costs one device-to-host read."""
+        if isinstance(radius, torch.Tensor):
+            if radius.dim() != 1 or radius.shape[0] != nq or radius.dtype == torch.bool or radius.is_complex():
+                raise ValueError(f"radius must be a float or a real [nq={nq}] array, got {radius.dtype} {tuple(radius.shape)}")
+            r = radius.to(self.device, torch.float32).contiguous()
+            if not bool(torch.isfinite(r).all()):
+                raise ValueError("radius must be finite")
+            return r
+        a = np.asarray(radius) if not isinstance(radius, (float, int)) or isinstance(radius, bool) else np.float64(radius)
+        if a.shape not in ((), (nq,)) or a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.number) \
+                or np.issubdtype(a.dtype, np.complexfloating):
+            raise ValueError(f"radius must be a float or a real [nq={nq}] array, got {a.dtype} {a.shape}")
+        with np.errstate(over="ignore"):                   # beyond the f32 range: inf, rejected below
+            r = np.broadcast_to(a.astype(np.float32), (nq,)).copy()
+        if not np.isfinite(r).all():
+            raise ValueError("radius must be finite")
+        return torch.from_numpy(r).to(self.device)
+
+    def _range_args(self, q, radius, max_results, exclude, require):
+        """Validates a range search before anything is launched -> (q, radius f32 [nq], L, exclude, masks)."""
+        if self.ntotal == 0:
+            raise ValueError("empty index")
+        if q.dim() != 2 or q.shape[1] != self.d:
+            raise ValueError(f"expected queries [nq, {self.d}], got {tuple(q.shape)}")
+        L = range_max_results(max_results)
+        req = self._requires(require, q.shape[0])
+        rad = self._radii(radius, q.shape[0])
+        q = ops._f32c(q, "queries")
+        return q, rad, L, self._exclusions(exclude, q.shape[0]), req
+
+    def _range_workspace(self, nq: int, budget: int, cache: bool = True) -> torch.Tensor:
+        """The workspace of a range call; cache=False (the re-runs, whose budgets vary with each batch) allocates one that
+        is freed with the call instead of staying in the workspace cache."""
+        key = ("range", nq, budget)
+        ws = self._ws.get(key) if cache else None
+        if ws is None:
+            nbytes = int(_native.load().tt_flat_range_workspace_bytes(self.ntotal, self.d, nq, budget))
+            ws = torch.empty(max(nbytes, 256), device=self.device, dtype=torch.uint8)
+            if cache:
+                if len(self._ws) > 8:
+                    self._ws.clear()
+                self._ws[key] = ws
+        return ws
+
+    def _rerun_budget(self, n: int, need: int, first_slices: int) -> int:
+        """Candidate budget of a re-run of n overflowed queries whose fullest segment held `need` candidates in a first
+        pass over `first_slices` catalog slices.  The re-run's plan slices the catalog for n queries, often into more
+        slices; its segments (2 x budget / slices) must hold at least need candidates, and as many as the first pass's
+        total for that query (at most need x first_slices) spread over the re-run's slices."""
+        return need * max(first_slices, _plan_slices(self.ntotal, self.d, n))
+
+    def _range_budget(self, nq: int, L: int) -> int:
+        """Candidates per query the first pass makes room for: 2L, at least 16384, halved until the workspace fits."""
+        lib = _native.load()
+        b = max(2 * L, 16384)
+        while b > 64 and lib.tt_flat_range_workspace_bytes(self.ntotal, self.d, nq, b) > self.RANGE_WS_BUDGET:
+            b //= 2
+        return b
+
+    def _range_launch(self, q, rad, L: int, excl, req, budget: int, cache: bool = True):
+        nq = q.shape[0]
+        counts = torch.empty((nq,), device=self.device, dtype=torch.int64)
+        scores = torch.empty((nq, L), device=self.device, dtype=torch.float32)
+        ids = torch.empty((nq, L), device=self.device, dtype=torch.int64)
+        flags = torch.empty((max(nq, 1),), device=self.device, dtype=torch.int32)
+        need = torch.empty((max(nq, 1),), device=self.device, dtype=torch.int32)
+        nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
+        ws = self._range_workspace(max(nq, 1), budget, cache)
+        lib = _native.load()
+        with torch.cuda.device(self.device):
+            _native.check(lib.tt_flat_range_search(
+                q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                rad.data_ptr(), L, self.id_offset, counts.data_ptr(), scores.data_ptr(), ids.data_ptr(), flags.data_ptr(),
+                need.data_ptr(), nunc.data_ptr(), 0 if req is None else self.labels.data_ptr(),
+                0 if req is None else req.data_ptr(), 0 if excl is None else excl.data_ptr(),
+                0 if excl is None else excl.shape[1], ws.data_ptr(), ws.numel(), ops._stream()), "tt_flat_range_search")
+        return counts, scores, ids, flags[:nq], need[:nq], nunc
+
+    def _range_exact(self, q, rad, L: int, excl, req, counts, scores, ids, qsel: torch.Tensor) -> None:
+        """Exact fp32 re-run of the query rows qsel (i32, on this device) into counts / scores / ids."""
+        lib = _native.load()
+        nsel = int(qsel.numel())
+        need = int(lib.tt_flat_range_exact_workspace_bytes(self.ntotal, self.d, nsel, L))
+        if self._exact_ws is None or self._exact_ws.numel() < need:
+            self._exact_ws = torch.empty(need, device=self.device, dtype=torch.uint8)
+        with torch.cuda.device(self.device):
+            _native.check(lib.tt_flat_range_search_exact(
+                q.data_ptr(), q.shape[0], qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal, self.d, rad.data_ptr(), L,
+                self.id_offset, counts.data_ptr(), scores.data_ptr(), ids.data_ptr(),
+                0 if req is None else self.labels.data_ptr(), 0 if req is None else req.data_ptr(),
+                0 if excl is None else excl.data_ptr(), 0 if excl is None else excl.shape[1], self._exact_ws.data_ptr(),
+                self._exact_ws.numel(), ops._stream()), "tt_flat_range_search_exact")
+
+    def range_search_device(self, q: torch.Tensor, radius, max_results: int, *, exclude: Optional[torch.Tensor] = None,
+                            require=None):
+        """Asynchronous range search of CUDA f32 queries [nq, D] on the current stream: every row whose fp32 score is
+        strictly greater than `radius` (a float, or a numpy / CUDA [nq] array; finite).
+
+        Returns (counts [nq] i64, scores [nq, L] f32, ids [nq, L] i64, flags [nq] i32, need [nq] i32,
+        n_uncertified [1] i32) device tensors, L = max_results (1 <= L <= 16384): counts[i] rows qualify, the best
+        min(counts[i], L) of them come first (score desc, id asc), the tail is (-inf, -1).  Rows with flags != 1 are not
+        certified (see include/tt_b200.h); `range_search_async` re-runs them.  `exclude` and `require` as in
+        search_device: excluded and disallowed rows are never returned and never counted."""
+        q, rad, L, excl, req = self._range_args(q, radius, max_results, exclude, require)
+        return self._range_launch(q, rad, L, excl, req, self._range_budget(max(q.shape[0], 1), L))
+
+    def range_search_async(self, q: torch.Tensor, radius, max_results: int = _native.TT_FLAT_RANGE_MAX_RESULTS, *,
+                           exclude: Optional[torch.Tensor] = None, require=None) -> PendingSearch:
+        """range_search_device, then `.result()` -> (counts, scores, ids, n_rerun_tensor, n_rerun_exact) with every query
+        certified: queries whose candidates overflowed their segments are re-run through the tensor-core path with
+        segments sized from `need`, in groups whose workspace fits RANGE_WS_BUDGET; a query that alone does not fit, and
+        every other uncertified query, is re-run through the exact fp32 path with the same masks and list."""
+        q, rad, L, excl, req = self._range_args(q, radius, max_results, exclude, require)
+        nq = q.shape[0]
+        counts, scores, ids, flags, need, nunc = self._range_launch(q, rad, L, excl, req,
+                                                                    self._range_budget(max(nq, 1), L))
+        if self._ring is None:
+            self._ring = _FlagRing()
+        token = self._ring.post(nunc)
+
+        def finish():
+            if not self._ring.read(*token):
+                return counts, scores, ids, 0, 0
+            fl, nd = flags.cpu().numpy(), need.cpu().numpy()
+            over = np.flatnonzero((fl != 1) & ((-fl) & 1 == 1))
+            exact = [np.flatnonzero((fl != 1) & ((-fl) & 1 == 0))]
+            lib = _native.load()
+            first_slices = _plan_slices(self.ntotal, self.d, max(nq, 1))
+
+            def ws_bytes(n, need_max):
+                return int(lib.tt_flat_range_workspace_bytes(self.ntotal, self.d, n,
+                                                             self._rerun_budget(n, need_max, first_slices)))
+            n_tensor = 0
+            for g in range_rerun_groups(over, nd, ws_bytes, self.RANGE_WS_BUDGET):
+                need_max = int(nd[g].max())
+                if g.size == 1 and ws_bytes(1, need_max) > self.RANGE_WS_BUDGET:
+                    exact.append(g)
+                    continue
+                sel = torch.from_numpy(g).to(self.device)
+                c2, s2, i2, f2, _, _ = self._range_launch(
+                    q[sel].contiguous(), rad[sel].contiguous(), L, None if excl is None else excl[sel].contiguous(),
+                    None if req is None else req[sel].contiguous(), self._rerun_budget(g.size, need_max, first_slices),
+                    cache=False)
+                ok = f2 == 1
+                counts[sel[ok]], scores[sel[ok]], ids[sel[ok]] = c2[ok], s2[ok], i2[ok]
+                exact.append(g[~ok.cpu().numpy()])
+                n_tensor += g.size
+            rows = np.concatenate(exact)
+            if rows.size:
+                self._range_exact(q, rad, L, excl, req, counts, scores, ids,
+                                  torch.from_numpy(rows.astype(np.int32)).to(self.device))
+            return counts, scores, ids, n_tensor, int(rows.size)
+        return PendingSearch(finish)
+
+    def range_search(self, q: np.ndarray, radius, max_results: int = _native.TT_FLAT_RANGE_MAX_RESULTS, *,
+                     exclude: Optional[np.ndarray] = None, require=None):
+        """Host-to-host range search, the shape of faiss `index.range_search(q, radius)`: q f32 [nq, d] (un-normalised)
+        -> (lims i64 [nq + 1], D f32 [total], I i64 [total]); query i's rows are I[lims[i]:lims[i+1]], best first, at
+        most max_results of them (range_search_device's counts tell whether more qualified).  A row is returned iff its
+        fp32 score is strictly greater than the radius (a float or one per query).  `exclude`: numpy int64 [nq, E] ids
+        to leave out per query (-1 = padding); `require`: label masks as in search."""
+        q = np.ascontiguousarray(q, dtype=np.float32)
+        if q.ndim != 2 or q.shape[1] != self.d:
+            raise ValueError(f"expected queries [nq, {self.d}], got {q.shape}")
+        kw = {}
+        if exclude is not None:
+            exclude = np.ascontiguousarray(exclude, dtype=np.int64)
+            if exclude.ndim != 2 or exclude.shape[0] != q.shape[0]:
+                raise ValueError(f"expected exclusions [nq={q.shape[0]}, E], got {exclude.shape}")
+            kw["exclude"] = torch.from_numpy(exclude).to(self.device)
+        with torch.cuda.device(self.device):
+            dq = torch.from_numpy(q).to(self.device)
+            counts, scores, ids, _, _ = self.range_search_async(dq, radius, max_results, require=require, **kw).result()
+            return range_csr(counts.cpu().numpy(), scores.cpu().numpy(), ids.cpu().numpy())
+
     def post_flag(self, nunc_dev: torch.Tensor):
         if self._ring is None:
             self._ring = _FlagRing()
@@ -937,6 +1166,33 @@ class VectorDatabase:
         for query_scores, query_indices in zip(scores.tolist(), indices.tolist()):
             all_results.append([(pids[i], s) for i, s in zip(query_indices, query_scores) if 0 <= i < n])
         return all_results
+
+    def retrieve_above(self, query_embeddings: np.ndarray, min_score, max_results: int = _native.TT_FLAT_RANGE_MAX_RESULTS,
+                       *, exclude: Optional[List[List[str]]] = None, require_all=0,
+                       require_any=0) -> List[List[Tuple[str, float]]]:
+        """Every product whose score is strictly greater than `min_score` (a float, or one per query), best first, at
+        most `max_results` per query: a relevance floor whose result size changes from query to query.  `exclude` and
+        `require_all` / `require_any` as in retrieve_batch; excluded and disallowed products are never returned."""
+        if self.index is None:
+            raise ValueError("Index not built. Call build_index() or load_index() first.")
+        q = np.asarray(query_embeddings)
+        if q.ndim == 1:
+            q = q.reshape(1, -1)
+        nq = q.shape[0]
+        kw = {}
+        req = require_masks(require_all, require_any, nq)
+        if req is not None:
+            kw["require"] = req
+        if exclude is not None:
+            if len(exclude) != nq:
+                raise ValueError(f"exclude needs one list per query ({nq}), got {len(exclude)}")
+            kw["exclude"] = self._exclude_rows(exclude, nq)
+        lims, scores, rows = self.index.range_search(q, min_score, max_results, **kw)
+        pids = self.product_ids
+        n = len(pids)
+        s, r = scores.tolist(), rows.tolist()
+        return [[(pids[i], v) for i, v in zip(r[lims[j]:lims[j + 1]], s[lims[j]:lims[j + 1]]) if 0 <= i < n]
+                for j in range(nq)]
 
     def get_embedding(self, product_id: str) -> Optional[np.ndarray]:
         """vector_db.py:211-231 — the reference returns None in every branch; kept."""
