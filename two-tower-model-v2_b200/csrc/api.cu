@@ -70,10 +70,12 @@ extern "C" __attribute__((visibility("default"))) int tt_profile_scan_read(float
   return n;
 }
 
+namespace tt {
 __global__ void fill_int_kernel(int* p, int n, int v) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) p[i] = v;
 }
+}  // namespace tt
 
 extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_workspace_bytes(int64_t N, int D, int nq, int K) {
   if (N < 1 || D < 1 || nq < 1 || K < 1) return 0;

@@ -63,6 +63,9 @@ int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long l
                     const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
                     float* bound_out, cudaStream_t st, const long long* excl = nullptr, int E = 0);
 
+// p[0, n) = v (api.cu): the exact-path routes set every flag to 1 with it, and every shard bound to the bits of -inf
+__global__ void fill_int_kernel(int* p, int n, int v);
+
 // Range search (flat_range.cu): the scan plan of make_scan_plan's tiling and slices, with candidate segments sized for
 // about cand_budget candidates per query (twice an even share per slice).  No sample pass.
 ScanPlan make_range_plan(long long N, int D, int nq, long long cand_budget);

@@ -77,45 +77,14 @@ flat_range_finalize_kernel(const float* __restrict__ qn, const float* __restrict
   const int EP = EXCL ? next_pow2(E) : 0;
 
   // ---- 1. segment sizes -> offsets, the largest segment count, the query, the exclusion list ---------------
-  if (tid == 0) { s_off[0] = 0; s_any_ex = 0; s_bad = 0; s_m = 0; s_need = 0u; s_count = 0u; s_valid = 0u; s_fl = -INFINITY; }
-  __syncthreads();
-  for (int sl = tid; sl < nslices; sl += NT) {
-    const unsigned int c = seg_cnt[(size_t)q * nslices + sl];
-    if (c) atomicMax(&s_need, c);
-    s_off[sl + 1] = (int)min(c, (unsigned int)seg_cap);
-  }
-  for (int d = tid; d < D; d += NT) qs[d] = qn[(long long)q * D + d];
-  if constexpr (EXCL) {
-    if (stage_exclusions(excl, E, q, id_offset, N, ex, EP)) s_any_ex = 1;
-  }
-  __syncthreads();
-  if constexpr (EXCL) {
-    if (s_any_ex) bitonic_sort_desc(ex, EP);   // ends with a barrier
-  }
-  if (warp == 0) {
-    int carry = 0;
-    for (int base = 0; base < nslices; base += 32) {
-      const int sl = base + lane;
-      int v = (sl < nslices) ? s_off[sl + 1] : 0;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v += t; }
-      const int incl = carry + v;
-      if (sl < nslices) s_off[sl + 1] = incl;
-      carry = __shfl_sync(0xffffffffu, incl, 31);
-    }
-  }
-  __syncthreads();
+  if (tid == 0) { s_bad = 0; s_m = 0; s_count = 0u; s_valid = 0u; s_fl = -INFINITY; }
+  stage_query<NT, EXCL>(q, seg_cnt, nslices, seg_cap, qn, D, excl, E, id_offset, N, s_off, &s_need, qs, ex, EP, &s_any_ex);
   const bool overflow = s_need > (unsigned int)seg_cap;
   const int n = s_off[nslices];
   const float my_eps = eps[q], t = thr[q], h = hi[q], rad = radius[q];
   const bool any_ex = EXCL && s_any_ex;
   const bool vec = (D % 4 == 0) && ((reinterpret_cast<uintptr_t>(Xn) & 15) == 0);
-  // candidate i of the query (bf16 score bits, row): slice found by binary search over the offsets
-  auto cand_at = [&](int i) -> uint2 {
-    int lo = 0, hi_ = nslices;           // largest sl with s_off[sl] <= i
-    while (hi_ - lo > 1) { const int mid = (lo + hi_) >> 1; if (s_off[mid] <= i) lo = mid; else hi_ = mid; }
-    return cand[((size_t)q * nslices + lo) * seg_cap + (i - s_off[lo])];
-  };
+  auto cand_at = [&](int i) { return segment_entry(cand, s_off, nslices, seg_cap, q, i); };
   auto allowed = [&](uint32_t row) { return !(any_ex && is_excluded(ex, EP, row)); };
 
   // ---- 2. exact count: candidates above hi are certainly above the radius; the band [thr, hi] is rescored ------
@@ -259,21 +228,6 @@ flat_range_finalize_kernel(const float* __restrict__ qn, const float* __restrict
   }
 }
 
-template <int NT, bool EXCL>
-static int launch_range_finalize_t(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int L,
-                                   long long id_offset, const float* radius, const float* thr, const float* hi,
-                                   const float* eps, const unsigned int* seg_cnt, const void* cand, long long* counts,
-                                   float* scores, long long* ids, int* flags, int* need, int* n_uncertified,
-                                   const long long* excl, int E, int key_cap, size_t smem, cudaStream_t st) {
-  auto kern = flat_range_finalize_kernel<NT, EXCL>;
-  TT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  count_launch();
-  TT_CHECK_CUDA(launch_pdl(kern, dim3(nq), dim3(NT), smem, st, qn, Xn, N, D, L, id_offset, radius, thr, hi, eps, seg_cnt,
-                           reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap, key_cap, counts, scores, ids,
-                           flags, need, n_uncertified, excl, E));
-  return TT_OK;
-}
-
 static int launch_range_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int L,
                                  long long id_offset, const float* radius, const float* thr, const float* hi,
                                  const float* eps, const unsigned int* seg_cnt, const void* cand, long long* counts,
@@ -282,20 +236,16 @@ static int launch_range_finalize(const ScanPlan& pl, const float* qn, const floa
   TT_CHECK_ARG(pl.main_slices <= FINALIZE_MAX_SLICES, "too many catalog slices");
   const bool with_excl = excl != nullptr && E > 0;
   const int key_cap = range_key_cap(L);
-  size_t smem = (size_t)key_cap * 8 + (size_t)D * 4 + 16;
-  if (with_excl) {
-    int P = 1;
-    while (P < E) P <<= 1;
-    smem += (size_t)P * 4;
-  }
-#define TT_RANGE_FIN(NT_, EX_)                                                                                          \
-  launch_range_finalize_t<NT_, EX_>(pl, qn, Xn, N, D, nq, L, id_offset, radius, thr, hi, eps, seg_cnt, cand, counts,      \
-                                    scores, ids, flags, need, n_uncertified, EX_ ? excl : nullptr, EX_ ? E : 0, key_cap, \
-                                    smem, st)
-  // small batches get the wide CTA, as in the top-K finalize: the single query's streaming and rescoring are latency-bound
-  if (nq <= 16) return with_excl ? TT_RANGE_FIN(1024, true) : TT_RANGE_FIN(1024, false);
-  return with_excl ? TT_RANGE_FIN(256, true) : TT_RANGE_FIN(256, false);
-#undef TT_RANGE_FIN
+  const size_t smem = finalize_smem_bytes(key_cap, D, with_excl ? E : 0);
+  count_launch();
+  return launch_finalize_instance(nq, with_excl, [&](auto nt, auto ex) {
+    auto kern = flat_range_finalize_kernel<decltype(nt)::value, decltype(ex)::value>;
+    TT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    TT_CHECK_CUDA(launch_pdl(kern, dim3(nq), dim3(nt), smem, st, qn, Xn, N, D, L, id_offset, radius, thr, hi, eps, seg_cnt,
+                             reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap, key_cap, counts, scores, ids,
+                             flags, need, n_uncertified, ex ? excl : nullptr, ex ? E : 0));
+    return TT_OK;
+  });
 }
 
 ScanPlan make_range_plan(long long N, int D, int nq, long long cand_budget) {
@@ -473,11 +423,6 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_range_debug_read(c
   return TT_OK;
 }
 
-__global__ void range_fill_int_kernel(int* p, int n, int v) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) p[i] = v;
-}
-
 extern "C" __attribute__((visibility("default"))) int tt_flat_range_search(
     const float* q, int nq, const float* Xn, const void* Xh, const float* stats, int64_t N, int D, const float* radius,
     int L, int64_t id_offset, int64_t* counts, float* scores, int64_t* ids, int32_t* flags, int32_t* need,
@@ -503,7 +448,7 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_range_search(
     // rows too wide for the resident-query scan (D > 1024): the fp32 exact path serves the batch
     TT_CHECK_CUDA(cudaMemsetAsync(n_uncertified, 0, sizeof(int32_t), st));
     TT_CHECK_CUDA(cudaMemsetAsync(need, 0, (size_t)nq * sizeof(int32_t), st));
-    range_fill_int_kernel<<<(nq + 255) / 256, 256, 0, st>>>(flags, nq, 1);
+    fill_int_kernel<<<(nq + 255) / 256, 256, 0, st>>>(flags, nq, 1);
     TT_CHECK_LAUNCH();
     TT_CHECK_ARG((size_t)EX_QB * D * sizeof(float) <= 160 * 1024, "D too large");
     return flat_range_exact_impl(q, nq, nullptr, nq, Xn, N, D, radius, L, id_offset, counts, scores, ids, labels, require,

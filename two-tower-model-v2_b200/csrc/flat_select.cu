@@ -23,15 +23,10 @@ namespace tt {
 //      c = max(scan threshold, cutoff), hence an fp32 score below c + eps.  If the K-th best rescored
 //      fp32 score f_K >= c + eps, no such row can enter the top-K: the result is exact.  Otherwise the
 //      query is flagged and the host re-runs it through the exact path.
-// Twins in flat_select_common.cuh: radix_select_desc and rescore_rows restate steps 2 and 4 for the range finalize
-// (flat_range.cu), which must give a row the same fp32 score as this kernel; change them together.
 // EXCL (exclusion lists): right after the gather, candidates whose row the query excludes are dropped, so n, b_K,
 // the cutoff and m all count allowed rows only, and the certificate reads "every ALLOWED row not rescored has a
 // bf16 score < c".  Excluded rows are typically a query's best ones: the caller plans the scan for
 // K_plan = min(K + E, N, TT_FLAT_MAX_K) so that the candidate budget covers them.
-constexpr int FIN_THREADS = 256;          // large batches: one 256-thread CTA per query, several CTAs per SM
-constexpr int FIN_THREADS_WIDE = 1024;    // small batches (fewer queries than SMs): the latency-bound phases of the
-                                          // single query (gather, fp32 rescoring of ~200 scattered rows) get 4x the warps
 constexpr int RANK_BY_COUNT_MAX = 1024;    // survivors up to this many are ranked by counting, else bitonic sort
 
 template <int FIN_THREADS, bool EXCL>
@@ -52,53 +47,26 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
   __shared__ int s_off[FINALIZE_MAX_SLICES + 1];
   __shared__ unsigned int s_hist[256];
   __shared__ int s_wsum[FIN_THREADS / 32];
-  __shared__ int s_over, s_bad, s_digit, s_kk, s_any_ex;
+  __shared__ int s_bad, s_digit, s_kk, s_any_ex;
+  __shared__ unsigned int s_need;
   __shared__ float s_fk;
   const int q = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int NWARPS = FIN_THREADS / 32;
   const int EP = EXCL ? next_pow2(E) : 0;
 
-  // ---- 1. segment sizes -> offsets (parallel loads, warp-0 scan) --------------------------------
-  if (tid == 0) { s_over = 0; s_bad = 0; s_fk = -INFINITY; s_off[0] = 0; s_any_ex = 0; }
-  __syncthreads();
-  for (int sl = tid; sl < nslices; sl += FIN_THREADS) {
-    unsigned int c = seg_cnt[(size_t)q * nslices + sl];
-    if (c > (unsigned int)seg_cap) { c = (unsigned int)seg_cap; s_over = 1; }
-    s_off[sl + 1] = (int)c;
-  }
-  for (int d = tid; d < D; d += FIN_THREADS) qs[d] = qn[(long long)q * D + d];
-  if constexpr (EXCL) {
-    if (stage_exclusions(excl, E, q, id_offset, N, ex, EP)) s_any_ex = 1;
-  }
-  __syncthreads();
-  if constexpr (EXCL) {
-    if (s_any_ex) bitonic_sort_desc(ex, EP);   // ends with a barrier
-  }
-  if (warp == 0) {
-    int carry = 0;
-    for (int base = 0; base < nslices; base += 32) {
-      const int sl = base + lane;
-      int v = (sl < nslices) ? s_off[sl + 1] : 0;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v += t; }
-      int incl = carry + v;
-      if (incl > cand_cap) { incl = cand_cap; s_over = 1; }
-      if (sl < nslices) s_off[sl + 1] = incl;
-      carry = __shfl_sync(0xffffffffu, incl, 31);
-    }
-  }
-  __syncthreads();
-  const bool overflow = s_over != 0;
-  int n = s_off[nslices];
+  // ---- 1. segment sizes -> offsets, the query, the exclusion list; gather --------------------------
+  if (tid == 0) { s_bad = 0; s_fk = -INFINITY; }
+  stage_query<FIN_THREADS, EXCL>(q, seg_cnt, nslices, seg_cap, qn, D, excl, E, id_offset, N, s_off, &s_need, qs, ex, EP,
+                                 &s_any_ex);
+  const int total = s_off[nslices];
+  const bool overflow = s_need > (unsigned int)seg_cap || total > cand_cap;
+  int n = min(total, cand_cap);   // a longer list is cut to the cand_cap keys shared memory holds (overflow)
   const float my_eps = eps[q];
   const float t = thr[q];
 
-  // ---- gather: one candidate per thread step, slice found by binary search over the offsets ------
   for (int i = tid; i < n; i += FIN_THREADS) {
-    int lo = 0, hi = nslices;           // largest sl with s_off[sl] <= i
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (s_off[mid] <= i) lo = mid; else hi = mid; }
-    const uint2 e = cand[((size_t)q * nslices + lo) * seg_cap + (i - s_off[lo])];
+    const uint2 e = segment_entry(cand, s_off, nslices, seg_cap, q, i);
     key[i] = make_key(__uint_as_float(e.x), e.y);
   }
   __syncthreads();
@@ -108,47 +76,12 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
                                     [&](unsigned long long k) { return !is_excluded(ex, EP, key_row(k)); });
   }
 
-  // ---- 2. b_K by radix select on the ordered score bits (8 bits per pass, MSB first) --------------
+  // ---- 2. b_K by radix select on the ordered score bits ----------------------------------------------
   float cutoff = -INFINITY;
   if (n > K) {   // n == K: everything is rescored anyway
-    uint32_t prefix = 0u, mask = 0u;
-    int kk = K;
-    for (int shift = 24; shift >= 0; shift -= 8) {
-      if (tid < 256) s_hist[tid] = 0u;
-      __syncthreads();
-      for (int i = tid; i < n; i += FIN_THREADS) {
-        const uint32_t u = (uint32_t)(key[i] >> 32);
-        if ((u & mask) == prefix) atomicAdd(&s_hist[(u >> shift) & 255u], 1u);
-      }
-      __syncthreads();
-      if (warp == 0) {
-        // lane l owns bins 255-8l .. 248-8l (descending)
-        unsigned int loc[8];
-        unsigned int sum = 0;
-#pragma unroll
-        for (int j = 0; j < 8; ++j) { loc[j] = s_hist[255 - 8 * lane - j]; sum += loc[j]; }
-        unsigned int incl = sum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const unsigned int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-        const unsigned int excl = incl - sum;
-        if (excl < (unsigned int)kk && incl >= (unsigned int)kk) {   // exactly one lane
-          unsigned int above = excl;
-          int d = 255 - 8 * lane - 7;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            if (above + loc[j] >= (unsigned int)kk) { d = 255 - 8 * lane - j; break; }
-            above += loc[j];
-          }
-          s_digit = d;
-          s_kk = kk - (int)above;
-        }
-      }
-      __syncthreads();
-      prefix |= (uint32_t)s_digit << shift;
-      mask |= 255u << shift;
-      kk = s_kk;
-    }
-    cutoff = ordered_to_float(prefix) - PRUNE_MARGIN * my_eps;
+    const uint32_t b = radix_select_desc<FIN_THREADS>(n, K, s_hist, &s_digit, &s_kk,
+                                                      [&](int i) { return (uint32_t)(key[i] >> 32); });
+    cutoff = ordered_to_float(b) - PRUNE_MARGIN * my_eps;
   }
 
   // ---- 3. prune: in-place compaction of the survivors (chunks of FIN_THREADS, left-moving) ---------
@@ -166,9 +99,8 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
   constexpr int U = WIDE ? 2 : 4;
   for (int i0 = warp * U; i0 < m; i0 += NWARPS * U) {
     uint32_t row[U];
-    float bsc[U];
+    float bsc[U], sc[U];
     bool ok[U];
-    float a[U];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       const int i = i0 + u;
@@ -176,66 +108,17 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
       row[u] = key_row(kk64);
       bsc[u] = key_score(kk64);
       ok[u] = (i < m) && ((long long)row[u] < N);   // row >= N cannot happen unless the scan is broken
-      a[u] = 0.f;
     }
-    if (WIDE && vec && D <= 512) {
-      // every 16-byte piece of the U rows is requested before the first one is used: one memory latency per round
-      // instead of one per 128 columns (the rows are scattered over the table: DRAM or, after the prefetch, L2)
-      constexpr int NVX = 4;
-      const float4* q4 = reinterpret_cast<const float4*>(qs);
-      const int nvec = D >> 2;
-      float4 x[U][NVX];
+    rescore_rows<U, WIDE>(qs, Xn, D, vec, row, ok, sc, lane);
+    __syncwarp();
+    if (lane == 0) {
 #pragma unroll
       for (int u = 0; u < U; ++u) {
-        const float4* rp = reinterpret_cast<const float4*>(Xn + (long long)row[u] * D);
-#pragma unroll
-        for (int v = 0; v < NVX; ++v) {
-          const int cc = v * 32 + lane;
-          x[u][v] = (ok[u] && cc < nvec) ? __ldg(rp + cc) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      }
-#pragma unroll
-      for (int v = 0; v < NVX; ++v) {
-        const int cc = v * 32 + lane;
-        const float4 y = (cc < nvec) ? q4[cc] : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          a[u] = fmaf(x[u][v].x, y.x, a[u]); a[u] = fmaf(x[u][v].y, y.y, a[u]);
-          a[u] = fmaf(x[u][v].z, y.z, a[u]); a[u] = fmaf(x[u][v].w, y.w, a[u]);
-        }
-      }
-    } else if (vec) {
-      const float4* q4 = reinterpret_cast<const float4*>(qs);
-      for (int cc = lane; cc < (D >> 2); cc += 32) {
-        const float4 y = q4[cc];
-        float4 x[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u)
-          x[u] = ok[u] ? __ldg(reinterpret_cast<const float4*>(Xn + (long long)row[u] * D) + cc)
-                       : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-          a[u] = fmaf(x[u].x, y.x, a[u]); a[u] = fmaf(x[u].y, y.y, a[u]);
-          a[u] = fmaf(x[u].z, y.z, a[u]); a[u] = fmaf(x[u].w, y.w, a[u]);
-        }
-      }
-    } else {
-      for (int d = lane; d < D; d += 32) {
-        const float y = qs[d];
-#pragma unroll
-        for (int u = 0; u < U; ++u)
-          if (ok[u]) a[u] = fmaf(__ldg(Xn + (long long)row[u] * D + d), y, a[u]);
-      }
-    }
-    __syncwarp();
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const float sc = warp_sum(a[u]);
-      const int i = i0 + u;
-      if (lane == 0 && i < m) {
+        const int i = i0 + u;
+        if (i >= m) continue;
         if (ok[u]) {
-          key[i] = make_key(sc, row[u]);
-          if (!(fabsf(bsc[u] - sc) <= my_eps)) bad = 1;
+          key[i] = make_key(sc[u], row[u]);
+          if (!(fabsf(bsc[u] - sc[u]) <= my_eps)) bad = 1;
         } else {
           key[i] = 0ull;
           bad = 1;
@@ -298,41 +181,22 @@ flat_finalize_kernel(const float* __restrict__ qn, const float* __restrict__ Xn,
   }
 }
 
-template <int NT, bool EXCL>
-static int launch_finalize_t(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,
-                             long long id_offset, const float* thr, const float* eps, const unsigned int* seg_cnt,
-                             const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
-                             float* bound_out, const long long* excl, int E, size_t smem, cudaStream_t st) {
-  TT_CHECK_CUDA(cudaFuncSetAttribute(flat_finalize_kernel<NT, EXCL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  TT_CHECK_CUDA(launch_pdl(flat_finalize_kernel<NT, EXCL>, dim3(nq), dim3(NT), smem, st, qn, Xn, N, D, K, id_offset, thr, eps,
-                           seg_cnt, reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap, pl.cand_cap, scores,
-                           ids, flags, n_uncertified, bound_out, excl, E));
-  return TT_OK;
-}
-
 int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,
                     long long id_offset, const float* thr, const float* eps, const unsigned int* seg_cnt,
                     const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
                     float* bound_out, cudaStream_t st, const long long* excl, int E) {
   TT_CHECK_ARG(pl.main_slices <= FINALIZE_MAX_SLICES, "too many catalog slices");
   const bool with_excl = excl != nullptr && E > 0;
-  size_t smem = (size_t)pl.cand_cap * 8 + (size_t)D * 4 + 16;
-  if (with_excl) {
-    int P = 1;
-    while (P < E) P <<= 1;
-    smem += (size_t)P * 4;
-  }
+  const size_t smem = finalize_smem_bytes(pl.cand_cap, D, with_excl ? E : 0);
   count_launch();
-  // wide CTAs for small batches, measured (1M x 384): nq = 1 wide 20 us vs 31 us; nq = 128 wide 57 us vs 23 us
-  if (nq <= 16)
-    return with_excl ? launch_finalize_t<FIN_THREADS_WIDE, true>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand,
-                                                                scores, ids, flags, n_uncertified, bound_out, excl, E, smem, st)
-                     : launch_finalize_t<FIN_THREADS_WIDE, false>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand,
-                                                                 scores, ids, flags, n_uncertified, bound_out, nullptr, 0, smem, st);
-  return with_excl ? launch_finalize_t<FIN_THREADS, true>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand, scores,
-                                                         ids, flags, n_uncertified, bound_out, excl, E, smem, st)
-                   : launch_finalize_t<FIN_THREADS, false>(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, seg_cnt, cand, scores,
-                                                          ids, flags, n_uncertified, bound_out, nullptr, 0, smem, st);
+  return launch_finalize_instance(nq, with_excl, [&](auto nt, auto ex) {
+    auto kern = flat_finalize_kernel<decltype(nt)::value, decltype(ex)::value>;
+    TT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    TT_CHECK_CUDA(launch_pdl(kern, dim3(nq), dim3(nt), smem, st, qn, Xn, N, D, K, id_offset, thr, eps, seg_cnt,
+                             reinterpret_cast<const uint2*>(cand), pl.main_slices, pl.seg_cap, pl.cand_cap, scores, ids,
+                             flags, n_uncertified, bound_out, ex ? excl : nullptr, ex ? E : 0));
+    return TT_OK;
+  });
 }
 
 // ------------------------------------------------------------------------------------------

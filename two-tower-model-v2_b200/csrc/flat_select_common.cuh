@@ -1,6 +1,8 @@
-// Device helpers of the selection kernels shared by the top-K finalize (flat_select.cu) and the range finalize
-// (flat_range.cu): sorting, fp32 rescoring of one row, exclusion lists, in-place compaction.
+// Helpers shared by the top-K finalize (flat_select.cu) and the range finalize (flat_range.cu): sorting, exclusion
+// lists, the prologue and candidate lookup, in-place compaction, radix select, fp32 rescoring, and the launch rule.
+// Both kernels give a row the same fp32 score because both call rescore_rows.
 #pragma once
+#include <type_traits>
 #include "tt_common.cuh"
 #include "flat_internal.cuh"
 
@@ -26,28 +28,10 @@ __device__ __forceinline__ void bitonic_sort_desc(T* key, int P) {
   }
 }
 
-__device__ __forceinline__ int next_pow2(int n) {
+__host__ __device__ __forceinline__ int next_pow2(int n) {
   int p = 1;
   while (p < n) p <<= 1;
   return p;
-}
-
-// fp32 dot of a shared-memory query with a global row, warp-cooperative.
-__device__ __forceinline__ float warp_dot(const float* __restrict__ qs, const float* __restrict__ row, int D,
-                                          int lane, bool vec) {
-  float a = 0.f;
-  if (vec) {
-    const float4* r4 = reinterpret_cast<const float4*>(row);
-    const float4* q4 = reinterpret_cast<const float4*>(qs);
-    for (int c = lane; c < (D >> 2); c += 32) {
-      const float4 x = __ldg(r4 + c);
-      const float4 y = q4[c];
-      a = fmaf(x.x, y.x, a); a = fmaf(x.y, y.y, a); a = fmaf(x.z, y.z, a); a = fmaf(x.w, y.w, a);
-    }
-  } else {
-    for (int d = lane; d < D; d += 32) a = fmaf(__ldg(row + d), qs[d], a);
-  }
-  return warp_sum(a);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -77,6 +61,58 @@ __device__ __forceinline__ bool is_excluded(const unsigned int* ex, int P, unsig
   int lo = 0, hi = P;   // first position whose entry is <= row (the list is descending)
   while (lo < hi) { const int mid = (lo + hi) >> 1; if (ex[mid] > row) lo = mid + 1; else hi = mid; }
   return lo < P && ex[lo] == row;
+}
+
+// ------------------------------------------------------------------------------------------
+// Prologue of both finalize kernels (one CTA of NT threads per query q).  The scan left the query's candidates in
+// per-slice segments cand[q, sl, 0 .. seg_cnt[q, sl]), each holding at most seg_cap of them.  Lays them end to end:
+// s_off[sl] = where slice sl starts, s_off[nslices] = the number of candidates; *s_need = the largest count before
+// clamping (a segment overflowed iff it exceeds seg_cap).  Stages the query in qs[0, D) and, under EXCL, its exclusion
+// list in ex[0, EP) sorted descending, *s_any_ex = 1 if it names a row of this shard.  Ends with a barrier, so shared
+// state the caller's thread 0 sets before the call is visible to every thread after it.
+template <int NT, bool EXCL>
+__device__ __forceinline__ void stage_query(int q, const unsigned int* __restrict__ seg_cnt, int nslices, int seg_cap,
+                                            const float* __restrict__ qn, int D, const long long* __restrict__ excl, int E,
+                                            long long id_offset, long long N, int* s_off, unsigned int* s_need, float* qs,
+                                            unsigned int* ex, int EP, int* s_any_ex) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid == 0) { s_off[0] = 0; *s_need = 0u; *s_any_ex = 0; }
+  __syncthreads();
+  for (int sl = tid; sl < nslices; sl += NT) {
+    const unsigned int c = seg_cnt[(size_t)q * nslices + sl];
+    if (c) atomicMax(s_need, c);
+    s_off[sl + 1] = (int)min(c, (unsigned int)seg_cap);
+  }
+  for (int d = tid; d < D; d += NT) qs[d] = qn[(long long)q * D + d];
+  if constexpr (EXCL) {
+    if (stage_exclusions(excl, E, q, id_offset, N, ex, EP)) *s_any_ex = 1;
+  }
+  __syncthreads();
+  if constexpr (EXCL) {
+    if (*s_any_ex) bitonic_sort_desc(ex, EP);   // ends with a barrier
+  }
+  if (warp == 0) {
+    int carry = 0;
+    for (int base = 0; base < nslices; base += 32) {
+      const int sl = base + lane;
+      int v = (sl < nslices) ? s_off[sl + 1] : 0;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v += t; }
+      const int incl = carry + v;
+      if (sl < nslices) s_off[sl + 1] = incl;
+      carry = __shfl_sync(0xffffffffu, incl, 31);
+    }
+  }
+  __syncthreads();
+}
+
+// Candidate i of query q (bf16 score bits, row) in the list stage_query laid out: slice lo is the largest with
+// s_off[lo] <= i, found by binary search.
+__device__ __forceinline__ uint2 segment_entry(const uint2* __restrict__ cand, const int* s_off, int nslices, int seg_cap,
+                                               int q, int i) {
+  int lo = 0, hi = nslices;
+  while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (s_off[mid] <= i) lo = mid; else hi = mid; }
+  return cand[((size_t)q * nslices + lo) * seg_cap + (i - s_off[lo])];
 }
 
 // In-place, order-keeping compaction of key[0, n) to the keys `keep(key)` accepts; returns the new count.  Chunks of
@@ -150,17 +186,43 @@ __device__ __forceinline__ uint32_t radix_select_desc(int n, int kk, unsigned in
   return prefix;
 }
 
-// fp32 scores of U catalog rows against the shared-memory query qs, warp-cooperative, with the arithmetic of the
-// finalize kernel's rescoring (per row: float4 pieces lane, lane + 32, ..., fmaf in x, y, z, w order, then warp_sum;
-// scalar columns when !vec), so both kernels give a row the same fp32 score bit for bit.  Rows with ok[u] false
-// score 0.  Every lane returns the sums.
-template <int U>
+// The fp32 score of a row, as both finalize kernels compute it: fp32 scores of U catalog rows against the shared-memory
+// query qs, warp-cooperative.  Per row: float4 pieces lane, lane + 32, ..., fmaf in x, y, z, w order, then warp_sum;
+// scalar columns when !vec.  Rows with ok[u] false score 0.  Every lane returns the sums.
+// WIDE (latency-bound CTAs of a small batch): with D <= 512, every 16-byte piece of the U rows is requested before the
+// first one is used, one memory latency per call instead of one per 128 columns (the rows are scattered over the
+// table: DRAM or, after the prefetch, L2).  The summation order is the same, so the score is too.
+template <int U, bool WIDE = false>
 __device__ __forceinline__ void rescore_rows(const float* __restrict__ qs, const float* __restrict__ Xn, int D, bool vec,
                                              const uint32_t (&row)[U], const bool (&ok)[U], float (&sc)[U], int lane) {
   float a[U];
 #pragma unroll
   for (int u = 0; u < U; ++u) a[u] = 0.f;
-  if (vec) {
+  if (WIDE && vec && D <= 512) {
+    constexpr int NVX = 4;
+    const float4* q4 = reinterpret_cast<const float4*>(qs);
+    const int nvec = D >> 2;
+    float4 x[U][NVX];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const float4* rp = reinterpret_cast<const float4*>(Xn + (long long)row[u] * D);
+#pragma unroll
+      for (int v = 0; v < NVX; ++v) {
+        const int cc = v * 32 + lane;
+        x[u][v] = (ok[u] && cc < nvec) ? __ldg(rp + cc) : make_float4(0.f, 0.f, 0.f, 0.f);
+      }
+    }
+#pragma unroll
+    for (int v = 0; v < NVX; ++v) {
+      const int cc = v * 32 + lane;
+      const float4 y = (cc < nvec) ? q4[cc] : make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        a[u] = fmaf(x[u][v].x, y.x, a[u]); a[u] = fmaf(x[u][v].y, y.y, a[u]);
+        a[u] = fmaf(x[u][v].z, y.z, a[u]); a[u] = fmaf(x[u][v].w, y.w, a[u]);
+      }
+    }
+  } else if (vec) {
     const float4* q4 = reinterpret_cast<const float4*>(qs);
     for (int cc = lane; cc < (D >> 2); cc += 32) {
       const float4 y = q4[cc];
@@ -184,6 +246,31 @@ __device__ __forceinline__ void rescore_rows(const float* __restrict__ qs, const
   }
 #pragma unroll
   for (int u = 0; u < U; ++u) sc[u] = warp_sum(a[u]);
+}
+
+// ------------------------------------------------------------------------------------------
+// Launch rule of both finalize kernels, one CTA per query.  Large batches get one 256-thread CTA per query, several CTAs
+// per SM.  Small batches (fewer queries than SMs) get 1024-thread CTAs: the latency-bound phases of the single query
+// (gather or streaming, fp32 rescoring of scattered rows) get 4x the warps.  Measured on the top-K finalize
+// (1M x 384): nq = 1 wide 20 us vs 31 us; nq = 128 wide 57 us vs 23 us.
+constexpr int FIN_THREADS = 256;
+constexpr int FIN_THREADS_WIDE = 1024;
+constexpr int FIN_WIDE_MAX_NQ = 16;   // batches up to this many queries get the wide CTA
+
+// Calls launch(nt, excl) for the finalize instance of a batch of nq queries, with the CTA size nt and whether the
+// queries carry exclusion lists as std::integral_constant, so that they can be the kernel's template arguments.
+template <typename Launch>
+int launch_finalize_instance(int nq, bool with_excl, Launch&& launch) {
+  using Wide = std::integral_constant<int, FIN_THREADS_WIDE>;
+  using Narrow = std::integral_constant<int, FIN_THREADS>;
+  if (nq <= FIN_WIDE_MAX_NQ) return with_excl ? launch(Wide{}, std::true_type{}) : launch(Wide{}, std::false_type{});
+  return with_excl ? launch(Narrow{}, std::true_type{}) : launch(Narrow{}, std::false_type{});
+}
+
+// Dynamic shared memory of a finalize CTA: `keys` 8-byte keys, the query (D floats) and, for E > 0 exclusions, the
+// staged list of next_pow2(E) rows.
+inline size_t finalize_smem_bytes(int keys, int D, int E) {
+  return (size_t)keys * 8 + (size_t)D * 4 + 16 + (E > 0 ? (size_t)next_pow2(E) * 4 : 0);
 }
 
 }  // namespace tt
