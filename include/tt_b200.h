@@ -401,6 +401,26 @@ int tt_flat_shard_search_filtered(int nq, const float* Xn, const void* Xh, int64
 int tt_shard_merge(const void* gathered, size_t rank_stride, size_t off_scores, size_t off_ids,
                    size_t off_bound, size_t off_flags, int G, int nq, int K,
                    float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, void* stream);
+/* Range search over a catalog sharded over G devices.  Every rank runs tt_flat_range_search over its rows (ids = row +
+ * id_offset, exclusion lists of global ids) and packs {counts i64[nq] | scores f32[nq,L] | ids i64[nq,L] | flags i32[nq]}
+ * into one byte record; ONE all-gather gives `gathered` (G records, rank_stride bytes apart, fields at the given byte
+ * offsets; counts / ids 8-byte aligned, scores / flags 4-byte aligned, rank_stride a multiple of 8).  Where rank g
+ * certified query q (flag 1), its list holds min(counts_g[q], L) entries sorted by (score desc, id asc); the tail is not
+ * read.  Where it did not, its count and list may disagree (tt_flat_range_search may list fewer rows than its count):
+ * its list is not read at all, its count is still summed, and the merged query is uncertified.
+ * tt_range_merge writes
+ *   counts[q] = sum over g of counts_g[q]
+ *   scores / ids [nq, L]: the best min(counts[q], L) rows of the union, same order, tail (-inf, -1)
+ *   flags[q] = 1 if every rank's flag is 1, else -(OR of the ranks' reason bits)
+ *   n_uncertified: number of flags != 1 (zeroed on the stream first; nq = 0 only zeroes it).
+ * No global certificate is needed: each rank's count is exact and its list holds its best min(count, L) rows, so the
+ * global best L lie in the union of the lists.  A query is exact iff every rank certified it; a rank re-runs its own
+ * uncertified rows (tt_flat_range_search with a larger workspace, or tt_flat_range_search_exact) and the records of those
+ * rows are exchanged and merged again.  Ids must be below 2^32 (the merge key carries 32 bits of id).
+ * 1 <= G <= 64, 1 <= L <= TT_FLAT_RANGE_MAX_RESULTS. */
+int tt_range_merge(const void* gathered, size_t rank_stride, size_t off_counts, size_t off_scores, size_t off_ids,
+                   size_t off_flags, int G, int nq, int L,
+                   int64_t* counts, float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified, void* stream);
 
 /* All-gather of per-rank records over NVLink peer memory by our own kernels (the exchange of the sharded
  * search; NCCL stays available as the alternative).  The caller owns, on every rank, a receive buffer and

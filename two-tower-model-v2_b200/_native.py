@@ -102,6 +102,8 @@ SIGNATURES = {
     "tt_p2p_wait": (c_int, [c_void_p, c_int, c_int32, ctypes.c_double, c_void_p, c_void_p]),
     "tt_shard_merge": (c_int, [c_void_p, c_size_t, c_size_t, c_size_t, c_size_t, c_size_t, c_int, c_int, c_int,
                                c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "tt_range_merge": (c_int, [c_void_p, c_size_t, c_size_t, c_size_t, c_size_t, c_size_t, c_int, c_int, c_int,
+                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "tt_flat_search_exact_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int]),
     "tt_flat_search_exact": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int64,
                                      c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),

@@ -254,5 +254,25 @@ def shard_merge(gathered: torch.Tensor, off_scores: int, off_ids: int, off_bound
     return scores, ids, flags[:nq], nunc
 
 
-__all__ = ["shard_merge", "flat_build", "flat_search", "flat_search_exact", "pool_weighted", "pool_weighted_gather", "attention_logits", "pool_attention",
+def range_merge(gathered: torch.Tensor, layout, nq: int, L: int, nunc: torch.Tensor = None):
+    """[G, record bytes] all-gathered range records (sharded.range_record_layout) -> (counts [nq] i64, scores [nq, L],
+    ids [nq, L], flags [nq], n_uncertified [1]): the summed counts and the best min(count, L) rows of the union
+    (tt_range_merge)."""
+    G = gathered.shape[0]
+    dev = gathered.device
+    counts = torch.empty((nq,), device=dev, dtype=torch.int64)
+    scores = torch.empty((nq, L), device=dev, dtype=torch.float32)
+    ids = torch.empty((nq, L), device=dev, dtype=torch.int64)
+    flags = torch.empty((max(nq, 1),), device=dev, dtype=torch.int32)
+    if nunc is None:
+        nunc = torch.empty((1,), device=dev, dtype=torch.int32)
+    with torch.cuda.device(dev):
+        _native.check(_native.load().tt_range_merge(gathered.data_ptr(), gathered.stride(0), layout.off_counts,
+                                                    layout.off_scores, layout.off_ids, layout.off_flags, G, nq, L,
+                                                    counts.data_ptr(), scores.data_ptr(), ids.data_ptr(), flags.data_ptr(),
+                                                    nunc.data_ptr(), _stream()), "tt_range_merge")
+    return counts, scores, ids, flags[:nq], nunc
+
+
+__all__ = ["shard_merge", "range_merge", "flat_build", "flat_search", "flat_search_exact", "pool_weighted", "pool_weighted_gather", "attention_logits", "pool_attention",
            "pool_attention_gather", "pool_attention_fused", "pool_backward", "infonce_forward", "infonce_backward", "pool_partial_gather", "pool_partial_merge", "topk_merge", "_f32c", "_stream"]

@@ -22,7 +22,8 @@ import torch
 
 from .buyer_tower import BuyerTower
 from .config import DEFAULT_EVENT_WEIGHTS, get_event_weight
-from .vector_db import PendingSearch, VectorDatabase, require_masks
+from ._native import TT_FLAT_RANGE_MAX_RESULTS
+from .vector_db import PendingSearch, VectorDatabase, range_csr, require_masks
 
 
 class RetrievalPipeline:
@@ -79,12 +80,23 @@ class RetrievalPipeline:
             kw["exclude"] = indices.to(device=self.index.device, dtype=torch.int64).contiguous()
         return self.index.search_async(emb, k, **kw)
 
-    def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *, exclude_history: bool = False,
-                        require_all=0, require_any=0):
-        """-> (scores f32 [B,k'], row indices i64 [B,k']) numpy; one H2D of the padded history, one D2H.
-        exclude_history: leave out the buyer's last `max_interaction_history` interacted items; require_all /
-        require_any: label masks (see retrieve_device_async); a buyer with fewer than k' allowed items gets (-inf, -1)
-        at the tail."""
+    def retrieve_above_device_async(self, indices: torch.Tensor, weights: torch.Tensor, min_score,
+                                    max_results: int = TT_FLAT_RANGE_MAX_RESULTS, *, exclude_history: bool = False,
+                                    require_all=0, require_any=0) -> PendingSearch:
+        """Relevance floor instead of a fixed k: every item scoring strictly above `min_score` (a float, or one per
+        buyer), best first, at most `max_results` per buyer.  `.result()` -> (counts [B] i64, scores [B, L], rows [B, L]
+        i64, n_rerun_tensor, n_rerun_exact) as FlatIPIndex.range_search_async; counts[b] items qualified, the first
+        min(counts[b], L) are listed, the tail is (-inf, -1).  exclude_history, require_all, require_any as in
+        retrieve_device_async: excluded and disallowed items are neither listed nor counted."""
+        req = require_masks(require_all, require_any, int(indices.shape[0]))
+        emb = self.encode_device(indices, weights)
+        kw = {} if req is None else {"require": req}
+        if exclude_history:
+            kw["exclude"] = indices.to(device=self.index.device, dtype=torch.int64).contiguous()
+        return self.index.range_search_async(emb, min_score, max_results, **kw)
+
+    def _stage(self, batch: Sequence[Sequence[Dict[str, Any]]]):
+        """Padded history rows / weights of a batch, copied to the device through pinned buffers."""
         idx, w, _ = self.encode_histories(batch)
         key = idx.shape
         pins = self._pins.get(key)
@@ -96,7 +108,15 @@ class RetrievalPipeline:
         pins[0].copy_(torch.from_numpy(idx))
         pins[1].copy_(torch.from_numpy(w))
         dev = self.index.device
-        idx_dev, w_dev = pins[0].to(dev, non_blocking=True), pins[1].to(dev, non_blocking=True)
+        return pins[0].to(dev, non_blocking=True), pins[1].to(dev, non_blocking=True)
+
+    def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *, exclude_history: bool = False,
+                        require_all=0, require_any=0):
+        """-> (scores f32 [B,k'], row indices i64 [B,k']) numpy; one H2D of the padded history, one D2H.
+        exclude_history: leave out the buyer's last `max_interaction_history` interacted items; require_all /
+        require_any: label masks (see retrieve_device_async); a buyer with fewer than k' allowed items gets (-inf, -1)
+        at the tail."""
+        idx_dev, w_dev = self._stage(batch)
         pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=exclude_history,
                                              require_all=require_all, require_any=require_any)
         scores, ids, _ = pending.result()
@@ -120,6 +140,28 @@ class RetrievalPipeline:
         pids = self.db.product_ids
         n = len(pids)
         return [[(pids[i], s) for i, s in zip(ri, rs) if 0 <= i < n] for rs, ri in zip(scores.tolist(), ids.tolist())]
+
+    def retrieve_above_batch(self, batch: Sequence[Sequence[Dict[str, Any]]], min_score,
+                             max_results: int = TT_FLAT_RANGE_MAX_RESULTS, *, exclude_history: bool = False,
+                             require_all=0, require_any=0) -> List[List[Tuple[str, float]]]:
+        """Per buyer, every product scoring strictly above `min_score` (a float or one per buyer), best first, at most
+        `max_results`.  exclude_history, require_all, require_any as in retrieve_batch."""
+        idx_dev, w_dev = self._stage(batch)
+        counts, scores, ids, _, _ = self.retrieve_above_device_async(
+            idx_dev, w_dev, min_score, max_results, exclude_history=exclude_history, require_all=require_all,
+            require_any=require_any).result()
+        lims, s, r = range_csr(counts.cpu().numpy(), scores.cpu().numpy(), ids.cpu().numpy())
+        pids = self.db.product_ids
+        s, r = s.tolist(), r.tolist()
+        return [[(pids[i], v) for i, v in zip(r[lims[b]:lims[b + 1]], s[lims[b]:lims[b + 1]])] for b in range(len(batch))]
+
+    def retrieve_above(self, interactions: Sequence[Dict[str, Any]], min_score,
+                       max_results: int = TT_FLAT_RANGE_MAX_RESULTS, *, exclude_history: bool = False, require_all=0,
+                       require_any=0) -> List[Tuple[str, float]]:
+        """One request -> [(product_id, score)] of every product scoring strictly above `min_score`, best first, at most
+        `max_results` (see retrieve_above_batch)."""
+        return self.retrieve_above_batch([interactions], min_score, max_results, exclude_history=exclude_history,
+                                         require_all=require_all, require_any=require_any)[0]
 
 
 class ShardedRetrievalPipeline:
@@ -213,4 +255,34 @@ class ShardedRetrievalPipeline:
         def finish():
             s, i, n_bad = pending.result()
             return s.cpu().numpy(), i.cpu().numpy(), n_bad
+        return PendingSearch(finish)
+
+    def retrieve_above_device_async(self, indices: torch.Tensor, weights: torch.Tensor, min_score,
+                                    max_results: int = TT_FLAT_RANGE_MAX_RESULTS, *, exclude_history: bool = False,
+                                    require_all=0, require_any=0) -> PendingSearch:
+        """Relevance floor over the sharded catalog: owner-computes pooling (encode_device), then
+        ShardedFlatIPIndex.range_search_async.  `.result()` -> (counts [B] i64, scores [B, L], ids [B, L] GLOBAL rows,
+        n_rerun), the same on every rank.  exclude_history / require_all / require_any as in retrieve_device_async."""
+        req = require_masks(require_all, require_any, int(indices.shape[0]))
+        emb = self.encode_device(indices, weights)
+        kw = {} if req is None else {"require": req}
+        if exclude_history:
+            kw["exclude"] = indices.to(device=self.table.device, dtype=torch.int64).contiguous()
+        return self.sharded.range_search_async(emb, min_score, max_results, **kw)
+
+    def retrieve_above_host_async(self, idx_host: torch.Tensor, w_host: torch.Tensor, min_score,
+                                  max_results: int = TT_FLAT_RANGE_MAX_RESULTS, *, exclude_history: bool = False,
+                                  require_all=0, require_any=0) -> PendingSearch:
+        """Pinned host tensors in (the WHOLE batch, the same on every rank) -> `.result()` = faiss's (lims, D, I) numpy
+        layout of retrieve_above_device_async's result (I: global rows) and n_rerun."""
+        dev = self.table.device
+        idx_dev, w_dev = idx_host.to(dev, non_blocking=True), w_host.to(dev, non_blocking=True)
+        pending = self.retrieve_above_device_async(idx_dev, w_dev, min_score, max_results,
+                                                   exclude_history=exclude_history, require_all=require_all,
+                                                   require_any=require_any)
+
+        def finish():
+            c, s, i, n_bad = pending.result()
+            lims, D, I = range_csr(c.cpu().numpy(), s.cpu().numpy(), i.cpu().numpy())
+            return lims, D, I, n_bad
         return PendingSearch(finish)

@@ -11,6 +11,10 @@ global top-K on every rank together with a *global* exactness certificate: the m
 clear, on every shard, the bound of the rows that shard did not rescore in fp32.  Queries that fail it
 (rare) are re-run through the always-exact fp32 path on every shard and merged again.
 
+Range search (`range_search_async`) uses the same shape with { counts i64[nq] | scores f32[nq,L] | ids i64[nq,L] |
+flags i32[nq] } records and tt_range_merge: each shard's count and list are exact on their own, so the merge needs no
+global certificate; a query some shard did not certify is completed by that shard and merged again.
+
 The local search and the merge are injectable so that the pack / exchange / fallback logic is testable
 on CPU with the gloo backend (tests/test_sharded_gloo.py).
 """
@@ -67,6 +71,55 @@ def record_views(buf: torch.Tensor, lay: RecordLayout, nq: int, k: int):
 def _merge_cuda(gathered: torch.Tensor, lay: RecordLayout, nq: int, k: int, nunc: Optional[torch.Tensor] = None):
     from . import ops
     return ops.shard_merge(gathered, lay.off_scores, lay.off_ids, lay.off_bound, lay.off_flags, nq, k, nunc)
+
+
+class RangeRecordLayout(NamedTuple):
+    """Byte offsets of one rank's range-search record (every field 16-byte aligned)."""
+    off_counts: int
+    off_scores: int
+    off_ids: int
+    off_flags: int
+    nbytes: int
+
+
+def range_record_layout(nq: int, L: int) -> RangeRecordLayout:
+    """{ counts i64[nq] | scores f32[nq, L] | ids i64[nq, L] | flags i32[nq] } (tt_range_merge)."""
+    def up(x):
+        return (x + 15) // 16 * 16
+    o_scores = up(nq * 8)
+    o_ids = up(o_scores + nq * L * 4)
+    o_flags = up(o_ids + nq * L * 8)
+    return RangeRecordLayout(0, o_scores, o_ids, o_flags, up(o_flags + nq * 4))
+
+
+def range_record_views(buf: torch.Tensor, lay: RangeRecordLayout, nq: int, L: int):
+    """Typed views (counts, scores, ids, flags) into a uint8 range record (or a [G, nbytes] stack of records)."""
+    lead = buf.shape[:-1]
+
+    def field(off, n, dtype, shape):
+        size = torch.empty((), dtype=dtype).element_size()
+        return buf[..., off:off + n * size].view(dtype).view(*lead, *shape)
+    return (field(lay.off_counts, nq, torch.int64, (nq,)), field(lay.off_scores, nq * L, torch.float32, (nq, L)),
+            field(lay.off_ids, nq * L, torch.int64, (nq, L)), field(lay.off_flags, nq, torch.int32, (nq,)))
+
+
+# Bytes of gathered range records one exchange may take (G records padded to L entries per query: 6.4 GB at nq 4096,
+# L 16384, G 8); a larger batch is exchanged and merged in chunks of queries.
+RANGE_EXCHANGE_BUDGET = 1 << 30
+
+
+def range_chunk_rows(nq: int, L: int, world: int, budget: int = RANGE_EXCHANGE_BUDGET) -> int:
+    """Queries per range exchange: the most whose gathered records (world x record bytes) fit `budget`, at least 1 and
+    at most nq.  A function of replicated values only, so every rank issues the same collectives."""
+    rows = max(1, budget // (world * (L * 12 + 12)))
+    while rows > 1 and world * range_record_layout(rows, L).nbytes > budget:
+        rows -= 1
+    return max(1, min(nq, rows))
+
+
+def _range_merge_cuda(gathered: torch.Tensor, lay: RangeRecordLayout, nq: int, L: int):
+    from . import ops
+    return ops.range_merge(gathered, lay, nq, L)
 
 
 class _RawCudaBuffer:
@@ -241,11 +294,15 @@ class ShardedFlatIPIndex:
     [nq,k] record views (see FlatIPIndex).  Label filters also need `id_offset` (its first global row), `labels` and
     `set_labels(words, rows=None)`; the local calls then get `require=` (a LabelMasks) next to `exclude=`.
     `merge(gathered[G,nbytes] uint8, layout, nq, k) -> (scores, ids, flags, n_uncertified)`.
+    Range search also needs `d`, `_radii`, `range_shard_into`, `range_rerun`, `post_flag` and `read_flag` of the local
+    index (see FlatIPIndex) and `range_merge(gathered, range layout, nq, L) -> (counts, scores, ids, flags,
+    n_uncertified [1])`.
     """
 
     MAX_P2P_SHAPES = 4
 
-    def __init__(self, local_index, n_total: int, group=None, merge: Optional[Callable] = None, exchange: str = "auto"):
+    def __init__(self, local_index, n_total: int, group=None, merge: Optional[Callable] = None, exchange: str = "auto",
+                 range_merge: Optional[Callable] = None):
         if n_total >= 1 << 32:
             raise ValueError("sharded catalogs are limited to 2^32 - 1 rows (merge keys carry 32-bit ids)")
         self.local = local_index
@@ -253,6 +310,7 @@ class ShardedFlatIPIndex:
         self.n_total = int(n_total)
         self.group = group
         self._merge = merge if merge is not None else _merge_cuda
+        self._range_merge = range_merge if range_merge is not None else _range_merge_cuda
         self._bufs = {}
         self._p2p = {}
         # "p2p": our push/wait kernels over NVLink peer memory; "nccl": torch.distributed all-gather.
@@ -688,3 +746,136 @@ class ShardedFlatIPIndex:
             ev.synchronize()
             return hs.numpy().copy(), hi.numpy().copy(), n_bad
         return PendingSearch(finish)
+
+    # -- range search -------------------------------------------------------------------------------------------
+    def _range_args(self, q: torch.Tensor, radius, max_results, exclude, require):
+        """Validates a sharded range search on this rank before any collective (every argument is replicated, so a bad
+        one raises on every rank instead of leaving the others waiting) -> (q f32, radii f32 [nq], L, exclude or None,
+        LabelMasks or None)."""
+        from ._native import TT_FLAT_MAX_EXCLUDE
+        from .vector_db import range_max_results
+        d = self.local.d
+        if not isinstance(q, torch.Tensor) or q.dim() != 2 or q.shape[1] != d:
+            raise ValueError(f"expected queries [nq, {d}], got {tuple(getattr(q, 'shape', ()))}")
+        nq = q.shape[0]
+        L = range_max_results(max_results)
+        rad = self.local._radii(radius, nq)
+        req = self._requires(require, nq, q.device)
+        if exclude is not None:
+            if not (isinstance(exclude, torch.Tensor) and exclude.dtype == torch.int64 and exclude.dim() == 2
+                    and exclude.shape[0] == nq):
+                raise ValueError(f"exclude must be an int64 tensor [nq={nq}, E], got "
+                                 f"{getattr(exclude, 'dtype', type(exclude))} {tuple(getattr(exclude, 'shape', ()))}")
+            if exclude.shape[1] > TT_FLAT_MAX_EXCLUDE:
+                raise ValueError(f"at most {TT_FLAT_MAX_EXCLUDE} exclusions per query, got {exclude.shape[1]}")
+            exclude = exclude.to(q.device).contiguous() if exclude.shape[1] else None
+        return q.to(torch.float32).contiguous(), rad, L, exclude, req
+
+    def range_search_async(self, q: torch.Tensor, radius, max_results: int = 16384, *,
+                           exclude: Optional[torch.Tensor] = None, require=None):
+        """Range search over the sharded catalog (collective: every rank calls it with the same arguments): every row
+        whose fp32 score is strictly greater than `radius` (a float, or a numpy / device [nq] array), its exact count and
+        the best min(count, L) of them, L = max_results <= 16384.  Returns a PendingSearch; `.result()` -> (counts [nq]
+        i64, scores [nq, L] f32, ids [nq, L] i64 GLOBAL rows, n_rerun), the same device tensors on every rank, every
+        query exact; n_rerun counts the queries some rank had to complete after the first pass.
+
+        First pass, with no host synchronisation: this shard's tt_flat_range_search into its record, one all-gather of
+        the records and tt_range_merge (a batch whose gathered records exceed RANGE_EXCHANGE_BUDGET goes in chunks of
+        queries).  Each shard's count is exact and its list holds its best min(count, L) rows, so the merged result is
+        exact wherever every shard certified its part.  `.result()` reads the merged flag; for the queries some shard did
+        not certify, each rank completes its OWN uncertified rows (FlatIPIndex.range_rerun), keeps its certified rows as
+        they are, and one more exchange and merge of just those queries replaces them.
+        `exclude` (i64 [nq, E], GLOBAL ids, -1 padding) and `require` ([nq, 2] or [2] {all, any} label masks, see
+        set_labels) as in search_async: excluded and disallowed rows are neither returned nor counted."""
+        from .vector_db import LabelMasks, PendingSearch
+        q, rad, L, exclude, require = self._range_args(q, radius, max_results, exclude, require)
+        world = dist.get_world_size(self.group) if dist.is_initialized() else 1
+        nq, dev = q.shape[0], q.device
+        if nq == 0:
+            empty = (torch.zeros((0,), dtype=torch.int64, device=dev), torch.zeros((0, L), dtype=torch.float32, device=dev),
+                     torch.zeros((0, L), dtype=torch.int64, device=dev), 0)
+            return PendingSearch(lambda: empty)
+        self.flush()          # never interleave with the pipelined top-K schedule
+        self._validate(world, dev)
+
+        def part(a, b):
+            """Slices of the per-query arguments for queries [a, b)."""
+            return (q[a:b], rad[a:b], None if exclude is None else exclude[a:b],
+                    None if require is None else require.words[a:b])
+
+        chunk = range_chunk_rows(nq, L, world)
+        firsts, merged = [], []
+        for a in range(0, nq, chunk):
+            b = min(nq, a + chunk)
+            lay = range_record_layout(b - a, L)
+            rec = torch.empty(lay.nbytes, dtype=torch.uint8, device=dev)        # owned by this call until .result()
+            views = range_record_views(rec, lay, b - a, L)
+            qc, rc, ec, wc = part(a, b)
+            need = self.local.range_shard_into(qc, rc, L, *views,
+                                               **self._kw(ec, None if wc is None else LabelMasks(wc)))
+            gathered = torch.empty((world, lay.nbytes), dtype=torch.uint8, device=dev)
+            self._exchange(rec, gathered, world)
+            merged.append(self._range_merge(gathered, lay, b - a, L))
+            firsts.append((a, b, views, need))
+        if len(merged) == 1:
+            counts, scores, ids, flags, nunc = merged[0]
+        else:
+            counts, scores, ids, flags = (torch.cat([m[j] for m in merged]) for j in range(4))
+            nunc = merged[0][4].clone()
+            for m in merged[1:]:
+                nunc += m[4]
+        token = self.local.post_flag(nunc)
+
+        def finish():
+            n_bad = self.local.read_flag(token)
+            if not n_bad:
+                return counts, scores, ids, 0
+            bad = torch.nonzero(flags != 1).flatten().cpu().numpy()       # the same rows on every rank
+            for a, b, (c_l, s_l, i_l, f_l), need in firsts:
+                rows = bad[(bad >= a) & (bad < b)] - a
+                if rows.size == 0:
+                    continue
+                qc, rc, ec, wc = part(a, b)
+                self.local.range_rerun(qc, rc, L, ec, wc, c_l, s_l, i_l, f_l, need, rows=rows)
+                sel = torch.from_numpy(rows).to(dev)
+                lay2 = range_record_layout(rows.size, L)
+                rec2 = torch.empty(lay2.nbytes, dtype=torch.uint8, device=dev)
+                c2, s2, i2, f2 = range_record_views(rec2, lay2, rows.size, L)
+                c2.copy_(c_l[sel])
+                s2.copy_(s_l[sel])
+                i2.copy_(i_l[sel])
+                f2.copy_(f_l[sel])          # 1 for every row range_rerun completed
+                gathered2 = torch.empty((world, lay2.nbytes), dtype=torch.uint8, device=dev)
+                self._exchange(rec2, gathered2, world)
+                mc, ms, mi, mf, _ = self._range_merge(gathered2, lay2, rows.size, L)
+                if bool((mf != 1).any()):
+                    raise RuntimeError("sharded range search: queries still uncertified after the re-run")
+                gsel = sel + a
+                counts[gsel], scores[gsel], ids[gsel] = mc, ms, mi
+            return counts, scores, ids, int(n_bad)
+        return PendingSearch(finish)
+
+    def range_search_device(self, q: torch.Tensor, radius, max_results: int = 16384, *,
+                            exclude: Optional[torch.Tensor] = None, require=None):
+        """range_search_async(...).result(): (counts, scores, ids, n_rerun), the same on every rank."""
+        return self.range_search_async(q, radius, max_results, exclude=exclude, require=require).result()
+
+    def range_search(self, q, radius, max_results: int = 16384, *, exclude=None, require=None):
+        """Host-to-host range search over the sharded catalog, the shape of faiss `index.range_search(q, radius)`: q f32
+        [nq, d] (un-normalised), the same on every rank -> (lims i64 [nq + 1], D f32 [total], I i64 [total] GLOBAL rows),
+        identical on every rank.  `exclude`: numpy int64 [nq, E] global ids; `require`: label masks (see search_async)."""
+        import numpy as np
+        from .vector_db import range_csr
+        dev, d = self.local.device, self.local.d
+        q = np.ascontiguousarray(q, dtype=np.float32)
+        if q.ndim != 2 or q.shape[1] != d:
+            raise ValueError(f"expected queries [nq, {d}], got {q.shape}")
+        kw = {}
+        if exclude is not None:
+            exclude = np.ascontiguousarray(exclude, dtype=np.int64)
+            if exclude.ndim != 2 or exclude.shape[0] != q.shape[0]:
+                raise ValueError(f"expected exclusions [nq={q.shape[0]}, E], got {exclude.shape}")
+            kw["exclude"] = torch.from_numpy(exclude).to(dev)
+        counts, scores, ids, _ = self.range_search_device(torch.from_numpy(q).to(dev), radius, max_results,
+                                                          require=require, **kw)
+        return range_csr(counts.cpu().numpy(), scores.cpu().numpy(), ids.cpu().numpy())

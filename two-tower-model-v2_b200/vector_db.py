@@ -740,12 +740,16 @@ class FlatIPIndex:
             b //= 2
         return b
 
-    def _range_launch(self, q, rad, L: int, excl, req, budget: int, cache: bool = True):
+    def _range_launch(self, q, rad, L: int, excl, req, budget: int, cache: bool = True, out=None):
+        """`out`: the caller's contiguous (counts [nq], scores [nq, L], ids [nq, L], flags [nq]) to write into (nq >= 1)."""
         nq = q.shape[0]
-        counts = torch.empty((nq,), device=self.device, dtype=torch.int64)
-        scores = torch.empty((nq, L), device=self.device, dtype=torch.float32)
-        ids = torch.empty((nq, L), device=self.device, dtype=torch.int64)
-        flags = torch.empty((max(nq, 1),), device=self.device, dtype=torch.int32)
+        if out is not None:
+            counts, scores, ids, flags = out
+        else:
+            counts = torch.empty((nq,), device=self.device, dtype=torch.int64)
+            scores = torch.empty((nq, L), device=self.device, dtype=torch.float32)
+            ids = torch.empty((nq, L), device=self.device, dtype=torch.int64)
+            flags = torch.empty((max(nq, 1),), device=self.device, dtype=torch.int32)
         need = torch.empty((max(nq, 1),), device=self.device, dtype=torch.int32)
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
         ws = self._range_workspace(max(nq, 1), budget, cache)
@@ -804,36 +808,65 @@ class FlatIPIndex:
         def finish():
             if not self._ring.read(*token):
                 return counts, scores, ids, 0, 0
-            fl, nd = flags.cpu().numpy(), need.cpu().numpy()
-            over = np.flatnonzero((fl != 1) & ((-fl) & 1 == 1))
-            exact = [np.flatnonzero((fl != 1) & ((-fl) & 1 == 0))]
-            lib = _native.load()
-            first_slices = _plan_slices(self.ntotal, self.d, max(nq, 1))
-
-            def ws_bytes(n, need_max):
-                return int(lib.tt_flat_range_workspace_bytes(self.ntotal, self.d, n,
-                                                             self._rerun_budget(n, need_max, first_slices)))
-            n_tensor = 0
-            for g in range_rerun_groups(over, nd, ws_bytes, self.RANGE_WS_BUDGET):
-                need_max = int(nd[g].max())
-                if g.size == 1 and ws_bytes(1, need_max) > self.RANGE_WS_BUDGET:
-                    exact.append(g)
-                    continue
-                sel = torch.from_numpy(g).to(self.device)
-                c2, s2, i2, f2, _, _ = self._range_launch(
-                    q[sel].contiguous(), rad[sel].contiguous(), L, None if excl is None else excl[sel].contiguous(),
-                    None if req is None else req[sel].contiguous(), self._rerun_budget(g.size, need_max, first_slices),
-                    cache=False)
-                ok = f2 == 1
-                counts[sel[ok]], scores[sel[ok]], ids[sel[ok]] = c2[ok], s2[ok], i2[ok]
-                exact.append(g[~ok.cpu().numpy()])
-                n_tensor += g.size
-            rows = np.concatenate(exact)
-            if rows.size:
-                self._range_exact(q, rad, L, excl, req, counts, scores, ids,
-                                  torch.from_numpy(rows.astype(np.int32)).to(self.device))
-            return counts, scores, ids, n_tensor, int(rows.size)
+            n_tensor, n_exact = self.range_rerun(q, rad, L, excl, req, counts, scores, ids, flags, need)
+            return counts, scores, ids, n_tensor, n_exact
         return PendingSearch(finish)
+
+    def range_rerun(self, q, rad, L: int, excl, req, counts, scores, ids, flags, need, rows=None):
+        """Completes a first range pass in place: the uncertified queries among `rows` (numpy query rows; None = all) are
+        re-run through the tensor-core path with segments sized from `need`, in groups whose workspace fits
+        RANGE_WS_BUDGET; a query that alone does not fit, and every other uncertified query, through the exact fp32 path.
+        The completed rows' flags are set to 1.  q, rad, excl, req are the validated first-pass arguments (see _range_args) -> (n_rerun_tensor, n_rerun_exact)."""
+        nq = q.shape[0]
+        fl, nd = flags.cpu().numpy(), need.cpu().numpy()
+        bad = fl != 1
+        if rows is not None:
+            sel_rows = np.zeros(nq, bool)
+            sel_rows[np.asarray(rows, np.int64)] = True
+            bad &= sel_rows
+        over = np.flatnonzero(bad & ((-fl) & 1 == 1))
+        exact = [np.flatnonzero(bad & ((-fl) & 1 == 0))]
+        lib = _native.load()
+        first_slices = _plan_slices(self.ntotal, self.d, max(nq, 1))
+
+        def ws_bytes(n, need_max):
+            return int(lib.tt_flat_range_workspace_bytes(self.ntotal, self.d, n,
+                                                         self._rerun_budget(n, need_max, first_slices)))
+        n_tensor = 0
+        for g in range_rerun_groups(over, nd, ws_bytes, self.RANGE_WS_BUDGET):
+            need_max = int(nd[g].max())
+            if g.size == 1 and ws_bytes(1, need_max) > self.RANGE_WS_BUDGET:
+                exact.append(g)
+                continue
+            sel = torch.from_numpy(g).to(self.device)
+            c2, s2, i2, f2, _, _ = self._range_launch(
+                q[sel].contiguous(), rad[sel].contiguous(), L, None if excl is None else excl[sel].contiguous(),
+                None if req is None else req[sel].contiguous(), self._rerun_budget(g.size, need_max, first_slices),
+                cache=False)
+            ok = f2 == 1
+            counts[sel[ok]], scores[sel[ok]], ids[sel[ok]] = c2[ok], s2[ok], i2[ok]
+            exact.append(g[~ok.cpu().numpy()])
+            n_tensor += g.size
+        rows = np.concatenate(exact)
+        if rows.size:
+            self._range_exact(q, rad, L, excl, req, counts, scores, ids,
+                              torch.from_numpy(rows.astype(np.int32)).to(self.device))
+        done = np.flatnonzero(bad)
+        if done.size:
+            flags[torch.from_numpy(done).to(self.device)] = 1       # every completed row is now exact
+        return n_tensor, int(rows.size)
+
+    def range_shard_into(self, q: torch.Tensor, rad: torch.Tensor, L: int, counts, scores, ids, flags, *,
+                         exclude: Optional[torch.Tensor] = None, require=None) -> torch.Tensor:
+        """First pass of ShardedFlatIPIndex.range_search_async over this shard's rows, written into the caller's record
+        views (counts [nq], scores / ids [nq, L], flags [nq], contiguous; nq >= 1) -> need [nq].  `rad`: validated f32
+        [nq] radii on this device (no host read here); `exclude`: GLOBAL ids; `require`: label masks (a LabelMasks
+        costs no host read).  Ids are row + id_offset."""
+        req = self._requires(require, q.shape[0])
+        q = ops._f32c(q, "queries")
+        excl = self._exclusions(exclude, q.shape[0])
+        return self._range_launch(q, rad, L, excl, req, self._range_budget(q.shape[0], L),
+                                  out=(counts, scores, ids, flags))[4]
 
     def range_search(self, q: np.ndarray, radius, max_results: int = _native.TT_FLAT_RANGE_MAX_RESULTS, *,
                      exclude: Optional[np.ndarray] = None, require=None):
