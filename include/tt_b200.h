@@ -257,6 +257,48 @@ int tt_flat_search_exact_filtered(const float* q, int nq, const int32_t* qsel, i
                                   const int64_t* excl, int E,
                                   void* workspace, size_t workspace_bytes, void* stream);
 
+/* Grouped search: the exact top-K with at most max_per_group rows per group (a brand, a seller), so that one group's
+ * near-duplicates cannot fill the answer.
+ *   groups  i32 [N]       < 0 = ungrouped (no cap), else a group id in [0, n_groups); an id >= n_groups is treated as
+ *                         ungrouped (never used as an index)
+ *   max_per_group         1 <= m <= TT_FLAT_MAX_PER_GROUP, one cap for the whole call
+ *   labels, require       label filter as in tt_flat_search_filtered: both NULL (no filter) or both non-NULL
+ *   excl, E               exclusion lists as in tt_flat_search_excl (E = 0 without a list)
+ * For query q let A be its allowed, not excluded rows in (fp32 score desc, id asc) order.  Walk A and TAKE a row if it is
+ * ungrouped or fewer than m rows of its group were taken before it; stop after K takes.  scores / ids are the taken rows
+ * in walk order with a (-inf, -1) tail when fewer than K rows can be taken: the top-K of the rows that rank among the
+ * first m of their own group within A.  Excluded and disallowed rows never use up a group's quota.
+ * The scan, its plan (K_plan as in tt_flat_search_excl) and the certificate are those of tt_flat_search; the finalize
+ * walks the candidates instead of selecting the K best.  flags / n_uncertified as in tt_flat_search, read over the rows
+ * the walk may take: bit 2 = fewer than K rows could be taken while some allowed rows were not rescored (when every
+ * allowed row was rescored, a short answer is certified).  An uncertified query is re-run through
+ * tt_flat_search_exact_grouped with the same cap, masks and list.
+ * workspace: tt_flat_search_grouped_workspace_bytes(N, D, nq, K, E, n_groups): tt_flat_search_excl_workspace_bytes on
+ * the tensor-core path, tt_flat_search_exact_grouped_workspace_bytes where the planner routes the batch to the exact
+ * path (D > 1024, or K a large fraction of N).
+ * tt_flat_search_exact_grouped: tt_flat_search_exact_filtered's arguments (labels / require may be NULL) plus the cap.
+ * After the exclusion and filter sentinels it runs m passes over each query's N scores that find every group's m-th
+ * best row; the rows of a group below it are dropped like excluded rows.  That cost, m passes over the catalog, is why
+ * the cap is at most 64.  Its workspace, tt_flat_search_exact_grouped_workspace_bytes, is the exact path's plus
+ * 8 * n_groups * 16 bytes. */
+#define TT_FLAT_MAX_PER_GROUP 64
+size_t tt_flat_search_grouped_workspace_bytes(int64_t N, int D, int nq, int K, int E, int32_t n_groups);
+int tt_flat_search_grouped(const float* q, int nq,
+                           const float* Xn, const void* Xh, const float* stats, int64_t N, int D,
+                           int K, int64_t id_offset,
+                           float* scores, int64_t* ids, int32_t* flags, int32_t* n_uncertified,
+                           const int32_t* groups, int32_t n_groups, int max_per_group,
+                           const uint32_t* labels, const uint32_t* require,
+                           const int64_t* excl, int E,
+                           void* workspace, size_t workspace_bytes, void* stream);
+size_t tt_flat_search_exact_grouped_workspace_bytes(int64_t N, int D, int nsel, int K, int32_t n_groups);
+int tt_flat_search_exact_grouped(const float* q, int nq, const int32_t* qsel, int nsel,
+                                 const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                                 float* scores, int64_t* ids, const uint32_t* labels, const uint32_t* require,
+                                 const int64_t* excl, int E,
+                                 const int32_t* groups, int32_t n_groups, int max_per_group,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+
 /* Range search: every row whose fp32 score is STRICTLY greater than a per-query radius (faiss's inner-product
  * range_search), how many there are, and the best L of them.
  *   radius  f32 [nq]      finite; queries are renormalised as in tt_flat_search

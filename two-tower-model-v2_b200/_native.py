@@ -18,6 +18,7 @@ TT_FLAT_MAX_K = 2048
 TT_SHARD_TOPR = 32
 TT_FLAT_MAX_EXCLUDE = 1024
 TT_FLAT_RANGE_MAX_RESULTS = 16384
+TT_FLAT_MAX_PER_GROUP = 64
 ABI_VERSION = 1
 
 
@@ -78,6 +79,14 @@ SIGNATURES = {
     "tt_flat_shard_search_filtered": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_int64, c_int, c_int, c_int64,
                                               c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                               c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_search_grouped_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int, c_int, c_int32]),
+    "tt_flat_search_grouped": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_int64,
+                                       c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int, c_void_p,
+                                       c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "tt_flat_search_exact_grouped_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int, c_int32]),
+    "tt_flat_search_exact_grouped": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int64, c_int, c_int, c_int64,
+                                             c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int32,
+                                             c_int, c_void_p, c_size_t, c_void_p]),
     "tt_flat_range_workspace_bytes": (c_size_t, [c_int64, c_int, c_int, c_int64]),
     "tt_flat_range_search": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_int, c_int64,
                                      c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,

@@ -99,7 +99,8 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_excl_wor
 static int flat_search_impl(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,
                             int64_t N, int D, int K, int64_t id_offset, float* scores, int64_t* ids,
                             int32_t* flags, int32_t* n_uncertified, float* bound, const int64_t* excl, int E,
-                            void* workspace, size_t workspace_bytes, void* stream, const LabelArgs& lab = LabelArgs{}) {
+                            void* workspace, size_t workspace_bytes, void* stream, const LabelArgs& lab = LabelArgs{},
+                            const GroupArgs& grp = GroupArgs{}) {
   TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
   TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   TT_CHECK_ARG(q && Xn && Xh && stats && scores && ids && flags && n_uncertified, "null pointer");
@@ -124,6 +125,10 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
       fill_int_kernel<<<(nq + 255) / 256, 256, 0, st>>>(reinterpret_cast<int*>(bound), nq, (int)0xff800000);
       TT_CHECK_LAUNCH();
     }
+    if (grp.groups)
+      return tt_flat_search_exact_grouped(q, nq, nullptr, nq, Xn, N, D, K, id_offset, scores, ids, lab.labels, lab.require,
+                                          excl, E, grp.groups, grp.n_groups, grp.max_per_group, workspace, workspace_bytes,
+                                          stream);
     if (lab.labels)
       return tt_flat_search_exact_filtered(q, nq, nullptr, nq, Xn, N, D, K, id_offset, scores, ids, lab.labels, lab.require,
                                            excl, E, workspace, workspace_bytes, stream);
@@ -144,6 +149,10 @@ static int flat_search_impl(const float* q, int nq, const float* Xn, const void*
 
   if (int e = launch_prep_queries(q, nq, pl.nq_pad, D, pl.Dp, stats, qn, qh, eps, n_uncertified, st)) return e;
   if (int e = launch_scan(pl, qh, Xh, N, nq, thr, cnt, cand, sample, st, lab)) return e;
+  if (grp.groups)
+    return launch_group_finalize(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, cnt, cand, scores,
+                                 reinterpret_cast<long long*>(ids), flags, n_uncertified, grp, st,
+                                 reinterpret_cast<const long long*>(excl), E);
   return launch_finalize(pl, qn, Xn, N, D, nq, K, id_offset, thr, eps, cnt, cand, scores,
                          reinterpret_cast<long long*>(ids), flags, n_uncertified, bound, st,
                          reinterpret_cast<const long long*>(excl), E);
@@ -186,6 +195,41 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_filtered(co
   TT_CHECK_ARG(bad == nullptr, bad);
   return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
                           excl, E, workspace, workspace_bytes, stream, lab);
+}
+
+extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_grouped_workspace_bytes(int64_t N, int D, int nq, int K, int E,
+                                                                                      int32_t n_groups) {
+  if (E < 0 || E > TT_FLAT_MAX_EXCLUDE || N < 1 || D < 1 || nq < 1 || K < 1 || n_groups < 0) return 0;
+  const ScanPlan pl = make_scan_plan(N, D, nq, plan_k(N, K, E));
+  if (pl.route_exact || !pl.supported) return exact_workspace_bytes(N, K, n_groups);
+  return search_ws_layout(pl, D, nq).total;
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_grouped(const float* q, int nq, const float* Xn, const void* Xh,
+                                                                            const float* stats, int64_t N, int D, int K,
+                                                                            int64_t id_offset, float* scores, int64_t* ids,
+                                                                            int32_t* flags, int32_t* n_uncertified,
+                                                                            const int32_t* groups, int32_t n_groups,
+                                                                            int max_per_group, const uint32_t* labels,
+                                                                            const uint32_t* require, const int64_t* excl,
+                                                                            int E, void* workspace, size_t workspace_bytes,
+                                                                            void* stream) {
+  TT_CHECK_ARG(groups != nullptr, "null groups");
+  TT_CHECK_ARG(n_groups >= 0, "n_groups < 0");
+  TT_CHECK_ARG(max_per_group >= 1 && max_per_group <= TT_FLAT_MAX_PER_GROUP,
+               "need 1 <= max_per_group <= TT_FLAT_MAX_PER_GROUP (64)");
+  TT_CHECK_ARG((labels == nullptr) == (require == nullptr), "labels and require must be both NULL or both non-NULL");
+  LabelArgs lab;
+  if (labels) {
+    const char* bad = label_args(labels, require, &lab);
+    TT_CHECK_ARG(bad == nullptr, bad);
+  }
+  GroupArgs grp;
+  grp.groups = groups;
+  grp.n_groups = n_groups;
+  grp.max_per_group = max_per_group;
+  return flat_search_impl(q, nq, Xn, Xh, stats, N, D, K, id_offset, scores, ids, flags, n_uncertified, nullptr,
+                          excl, E, workspace, workspace_bytes, stream, lab, grp);
 }
 
 extern "C" __attribute__((visibility("default"))) int tt_flat_search_shard(const float* q, int nq, const float* Xn, const void* Xh, const float* stats,

@@ -63,6 +63,26 @@ int launch_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long l
                     const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
                     float* bound_out, cudaStream_t st, const long long* excl = nullptr, int E = 0);
 
+// Group cap of a grouped search (tt_flat_search_grouped): groups i32 [N], at most max_per_group rows per group id in
+// [0, n_groups); any other id is ungrouped.
+struct GroupArgs {
+  const int32_t* groups = nullptr;
+  int n_groups = 0;
+  int max_per_group = 0;
+};
+
+// The grouped finalize (flat_group.cu): flat_finalize_kernel's inputs, the group walk in place of the top-K selection
+int launch_group_finalize(const ScanPlan& pl, const float* qn, const float* Xn, long long N, int D, int nq, int K,
+                          long long id_offset, const float* thr, const float* eps, const unsigned int* seg_cnt,
+                          const void* cand, float* scores, long long* ids, int* flags, int* n_uncertified,
+                          const GroupArgs& grp, cudaStream_t st, const long long* excl = nullptr, int E = 0);
+
+// The group cap on the exact path (flat_group.cu): the scores of grouped rows outside their group's best
+// max_per_group in scores_ws [nslot, N] become sentinel_bits.  group_ws: exact_group_ws_bytes(n_groups) bytes.
+size_t exact_group_ws_bytes(int n_groups);
+int launch_exact_group_cap(float* scores_ws, long long N, int nslot, const GroupArgs& grp, void* group_ws,
+                           unsigned int sentinel_bits, cudaStream_t st);
+
 // p[0, n) = v (api.cu): the exact-path routes set every flag to 1 with it, and every shard bound to the bits of -inf
 __global__ void fill_int_kernel(int* p, int n, int v);
 
@@ -74,7 +94,10 @@ ScanPlan make_range_plan(long long N, int D, int nq, long long cand_budget);
 constexpr int EX_QB = 8;   // queries scored per pass over the fp32 table
 int launch_exact_group(const float* q, const int32_t* qsel, int slot0, int nslot, const float* Xn, long long N, int D, int K,
                        long long id_offset, float* scores, int64_t* ids, bool out_by_query, const int64_t* excl, int E,
-                       const uint32_t* labels, const uint32_t* require, void* workspace, cudaStream_t st);
+                       const uint32_t* labels, const uint32_t* require, void* workspace, cudaStream_t st,
+                       const GroupArgs& grp = GroupArgs{});
+// Workspace of the exact path for K results, and for a group cap over n_groups groups (0 = none)
+size_t exact_workspace_bytes(long long N, int K, int n_groups);
 
 // shared TMA descriptor helper (flat_scan.cu) and the tensor-core attention-logits launcher (attn_logits_tc.cu)
 int make_tmap_f32(void* tensor_map /* CUtensorMap* */, const void* base, long long rows, int cols, int box_rows, int box_cols);

@@ -540,12 +540,14 @@ namespace tt {
 // One group of nslot <= EX_QB query slots of the exact path; slot s serves query row qi = qsel[slot0 + s] (slot0 + s
 // without qsel).  fp32 scores of every row go to the first EX_QB * N floats of `workspace` (rows the query excludes or
 // does not allow hold EXCL_SCORE_BITS), then the exact top-K of each slot is written to row qi of scores / ids [*, K]
-// (out_by_query), or to row s.  workspace: exact_ws_layout(N, K) bytes.
+// (out_by_query), or to row s.  With grp.groups, the grouped rows outside their group's best grp.max_per_group get the
+// same sentinel before the select (launch_exact_group_cap).  workspace: exact_workspace_bytes(N, K, n_groups) bytes.
 int launch_exact_group(const float* q, const int32_t* qsel, int slot0, int nslot, const float* Xn, long long N, int D, int K,
                        long long id_offset, float* scores, int64_t* ids, bool out_by_query, const int64_t* excl, int E,
-                       const uint32_t* labels, const uint32_t* require, void* workspace, cudaStream_t st) {
+                       const uint32_t* labels, const uint32_t* require, void* workspace, cudaStream_t st,
+                       const GroupArgs& grp) {
   size_t o_state, o_hist, o_keys;
-  (void)exact_ws_layout(N, K, &o_state, &o_hist, &o_keys);
+  const size_t o_groups = exact_ws_layout(N, K, &o_state, &o_hist, &o_keys);
   unsigned char* ws = reinterpret_cast<unsigned char*>(workspace);
   float* scores_ws = reinterpret_cast<float*>(ws);
   SelState* state = reinterpret_cast<SelState*>(ws + o_state);
@@ -573,6 +575,9 @@ int launch_exact_group(const float* q, const int32_t* qsel, int slot0, int nslot
     exact_filter_kernel<<<dim3((unsigned)gs, nslot), 256, 0, st>>>(labels, require, qsel, slot0, N, scores_ws);
     TT_CHECK_LAUNCH();
   }
+  if (grp.groups) {
+    if (int e = launch_exact_group_cap(scores_ws, N, nslot, grp, ws + o_groups, EXCL_SCORE_BITS, st)) return e;
+  }
   exact_init_kernel<<<(nslot * 256 + 255) / 256, 256, 0, st>>>(state, hist, nslot, K);
   TT_CHECK_LAUNCH();
   for (int shift = 56; shift >= 0; shift -= 8) {
@@ -585,9 +590,14 @@ int launch_exact_group(const float* q, const int32_t* qsel, int slot0, int nslot
   TT_CHECK_LAUNCH();
   exact_sort_kernel<<<nslot, 256, (size_t)P * 8, st>>>(keys, out_by_query ? qsel : nullptr, out_by_query ? slot0 : 0, K,
                                                        id_offset, scores, reinterpret_cast<long long*>(ids),
-                                                       E > 0 || labels != nullptr);
+                                                       E > 0 || labels != nullptr || grp.groups != nullptr);
   TT_CHECK_LAUNCH();
   return TT_OK;
+}
+
+size_t exact_workspace_bytes(long long N, int K, int n_groups) {
+  size_t a, b, c;
+  return exact_ws_layout(N, K, &a, &b, &c) + (n_groups > 0 ? exact_group_ws_bytes(n_groups) : 0);
 }
 }  // namespace tt
 
@@ -600,21 +610,21 @@ extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_exact_wo
 static int flat_search_exact_impl(const float* q, int nq, const int32_t* qsel, int nsel, const float* Xn, int64_t N,
                                   int D, int K, int64_t id_offset, float* scores, int64_t* ids, const int64_t* excl,
                                   int E, void* workspace, size_t workspace_bytes, void* stream,
-                                  const uint32_t* labels = nullptr, const uint32_t* require = nullptr) {
+                                  const uint32_t* labels = nullptr, const uint32_t* require = nullptr,
+                                  const GroupArgs& grp = GroupArgs{}) {
   TT_CHECK_ARG(q && Xn && scores && ids && workspace, "null pointer");
   TT_CHECK_ARG(N >= 1 && N < (1LL << 32) && D >= 1, "need 1 <= N < 2^32, D >= 1");
   TT_CHECK_ARG(K >= 1 && K <= N && K <= TT_FLAT_MAX_K, "need 1 <= K <= min(N, TT_FLAT_MAX_K)");
   TT_CHECK_ARG(nq >= 0 && nsel >= 0 && (qsel != nullptr || nsel == nq), "qsel == NULL requires nsel == nq");
   TT_CHECK_ARG((size_t)EX_QB * D * sizeof(float) <= 160 * 1024, "D too large");
   if (nsel == 0) return TT_OK;
-  size_t o_state, o_hist, o_keys;
-  const size_t need = exact_ws_layout(N, K, &o_state, &o_hist, &o_keys);
+  const size_t need = exact_workspace_bytes(N, K, grp.groups ? grp.n_groups : 0);
   if (workspace_bytes < need) { set_error("tt_flat_search_exact: workspace too small"); return TT_ERR_WORKSPACE; }
   cudaStream_t st = (cudaStream_t)stream;
   for (int slot0 = 0; slot0 < nsel; slot0 += EX_QB) {
     const int nslot = (nsel - slot0 < EX_QB) ? (nsel - slot0) : EX_QB;
     if (int e = launch_exact_group(q, qsel, slot0, nslot, Xn, N, D, K, id_offset, scores, ids, true, excl, E, labels, require,
-                                   workspace, st)) return e;
+                                   workspace, st, grp)) return e;
   }
   return TT_OK;
 }
@@ -647,4 +657,31 @@ extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact_filte
   TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
   return flat_search_exact_impl(q, nq, qsel, nsel, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
                                 workspace_bytes, stream, labels, require);
+}
+
+extern "C" __attribute__((visibility("default"))) size_t tt_flat_search_exact_grouped_workspace_bytes(int64_t N, int D, int nsel, int K,
+                                                                                            int32_t n_groups) {
+  (void)D; (void)nsel;
+  if (N < 1 || K < 1 || n_groups < 0) return 0;
+  return exact_workspace_bytes(N, K, n_groups);
+}
+
+extern "C" __attribute__((visibility("default"))) int tt_flat_search_exact_grouped(const float* q, int nq, const int32_t* qsel, int nsel,
+                                                  const float* Xn, int64_t N, int D, int K, int64_t id_offset,
+                                                  float* scores, int64_t* ids, const uint32_t* labels, const uint32_t* require,
+                                                  const int64_t* excl, int E, const int32_t* groups, int32_t n_groups,
+                                                  int max_per_group, void* workspace, size_t workspace_bytes, void* stream) {
+  TT_CHECK_ARG(groups != nullptr, "null groups");
+  TT_CHECK_ARG(n_groups >= 0, "n_groups < 0");
+  TT_CHECK_ARG(max_per_group >= 1 && max_per_group <= TT_FLAT_MAX_PER_GROUP,
+               "need 1 <= max_per_group <= TT_FLAT_MAX_PER_GROUP (64)");
+  TT_CHECK_ARG((labels == nullptr) == (require == nullptr), "labels and require must be both NULL or both non-NULL");
+  TT_CHECK_ARG(E >= 0 && E <= TT_FLAT_MAX_EXCLUDE, "need 0 <= E <= TT_FLAT_MAX_EXCLUDE (1024) exclusions per query");
+  TT_CHECK_ARG(excl != nullptr || E == 0, "null exclusion list with E > 0");
+  GroupArgs grp;
+  grp.groups = groups;
+  grp.n_groups = n_groups;
+  grp.max_per_group = max_per_group;
+  return flat_search_exact_impl(q, nq, qsel, nsel, Xn, N, D, K, id_offset, scores, ids, excl, E, workspace,
+                                workspace_bytes, stream, labels, require, grp);
 }

@@ -66,18 +66,22 @@ class RetrievalPipeline:
         return self.tower.forward_gather(self.table, indices, weights, self.item_logits)
 
     def retrieve_device_async(self, indices: torch.Tensor, weights: torch.Tensor, k: int, *,
-                              exclude_history: bool = False, require_all=0, require_any=0) -> PendingSearch:
+                              exclude_history: bool = False, require_all=0, require_any=0,
+                              max_per_group: Optional[int] = None) -> PendingSearch:
         """exclude_history: the pooled history rows `indices` (-1 padded; the last `max_interaction_history`
         interactions when they come from encode_histories) are also the exclusion list of the search, so no buyer
         is shown the items they have just viewed, carted or bought.  No extra host-to-device copy.
         require_all / require_any: label masks (scalars or one per buyer, host values): only items whose label word
-        (VectorDatabase.set_labels) has every bit of require_all and, unless require_any is 0, one bit of require_any."""
+        (VectorDatabase.set_labels) has every bit of require_all and, unless require_any is 0, one bit of require_any.
+        max_per_group: at most that many items of one group (VectorDatabase.set_groups: a brand, a seller) per buyer."""
         k = min(k, self.index.ntotal)                                                  # vector_db.py:159
         req = require_masks(require_all, require_any, int(indices.shape[0]))
         emb = self.encode_device(indices, weights)
         kw = {} if req is None else {"require": req}
         if exclude_history:
             kw["exclude"] = indices.to(device=self.index.device, dtype=torch.int64).contiguous()
+        if max_per_group is not None:
+            kw["max_per_group"] = max_per_group
         return self.index.search_async(emb, k, **kw)
 
     def retrieve_above_device_async(self, indices: torch.Tensor, weights: torch.Tensor, min_score,
@@ -111,32 +115,36 @@ class RetrievalPipeline:
         return pins[0].to(dev, non_blocking=True), pins[1].to(dev, non_blocking=True)
 
     def retrieve_arrays(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *, exclude_history: bool = False,
-                        require_all=0, require_any=0):
+                        require_all=0, require_any=0, max_per_group: Optional[int] = None):
         """-> (scores f32 [B,k'], row indices i64 [B,k']) numpy; one H2D of the padded history, one D2H.
         exclude_history: leave out the buyer's last `max_interaction_history` interacted items; require_all /
         require_any: label masks (see retrieve_device_async); a buyer with fewer than k' allowed items gets (-inf, -1)
-        at the tail."""
+        at the tail; max_per_group: group cap (see retrieve_device_async)."""
         idx_dev, w_dev = self._stage(batch)
         pending = self.retrieve_device_async(idx_dev, w_dev, k, exclude_history=exclude_history,
-                                             require_all=require_all, require_any=require_any)
+                                             require_all=require_all, require_any=require_any,
+                                             max_per_group=max_per_group)
         scores, ids, _ = pending.result()
         return scores.cpu().numpy(), ids.cpu().numpy()
 
     def retrieve(self, interactions: Sequence[Dict[str, Any]], k: int = 10, *,
-                 exclude_history: bool = False, require_all=0, require_any=0) -> List[Tuple[str, float]]:
+                 exclude_history: bool = False, require_all=0, require_any=0,
+                 max_per_group: Optional[int] = None) -> List[Tuple[str, float]]:
         """One request, the shape of server.py:241-244 -> [(product_id, score)] in descending score.
         exclude_history: never return the items of the buyer's last `max_interaction_history` interactions.
-        require_all / require_any: label masks (see retrieve_device_async)."""
+        require_all / require_any: label masks; max_per_group: group cap (see retrieve_device_async)."""
         scores, ids = self.retrieve_arrays([interactions], k, exclude_history=exclude_history, require_all=require_all,
-                                           require_any=require_any)
+                                           require_any=require_any, max_per_group=max_per_group)
         pids = self.db.product_ids
         return [(pids[i], float(s)) for i, s in zip(ids[0].tolist(), scores[0].tolist()) if 0 <= i < len(pids)]
 
     def retrieve_batch(self, batch: Sequence[Sequence[Dict[str, Any]]], k: int = 10, *,
-                       exclude_history: bool = False, require_all=0, require_any=0) -> List[List[Tuple[str, float]]]:
-        """exclude_history: as in retrieve, per buyer; require_all / require_any: scalars or one value per buyer."""
+                       exclude_history: bool = False, require_all=0, require_any=0,
+                       max_per_group: Optional[int] = None) -> List[List[Tuple[str, float]]]:
+        """exclude_history: as in retrieve, per buyer; require_all / require_any: scalars or one value per buyer;
+        max_per_group: group cap (see retrieve_device_async)."""
         scores, ids = self.retrieve_arrays(batch, k, exclude_history=exclude_history, require_all=require_all,
-                                           require_any=require_any)
+                                           require_any=require_any, max_per_group=max_per_group)
         pids = self.db.product_ids
         n = len(pids)
         return [[(pids[i], s) for i, s in zip(ri, rs) if 0 <= i < n] for rs, ri in zip(scores.tolist(), ids.tolist())]

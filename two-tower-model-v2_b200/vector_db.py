@@ -292,6 +292,10 @@ class FlatIPIndex:
         self.id_offset = 0
         self.labels: Optional[torch.Tensor] = None        # int32 [N] (u32 label words) once set_labels was called
         self._labels_store: Optional[torch.Tensor] = None
+        self.groups: Optional[torch.Tensor] = None        # int32 [N] dense group ids (-1 = ungrouped) once set_groups ran
+        self.n_groups = 0
+        self._group_keys_store: Optional[torch.Tensor] = None   # int64 [capacity] raw keys as given to set_groups
+        self._groups_store: Optional[torch.Tensor] = None
         self._ws: Dict[Tuple[int, int], torch.Tensor] = {}
         self._exact_ws: Optional[torch.Tensor] = None
         self._ring: Optional[_FlagRing] = None
@@ -324,6 +328,16 @@ class FlatIPIndex:
                 self._labels_store = lab
             self._labels_store[old:n].zero_()
             self.labels = self._labels_store[:n]
+        if self._groups_store is not None:             # so do groups; new rows are ungrouped
+            if self._groups_store.shape[0] < self._xn_store.shape[0]:
+                keys = torch.full((self._xn_store.shape[0],), -1, device=self.device, dtype=torch.int64)
+                keys[:old].copy_(self._group_keys_store[:old])
+                dense = torch.full((self._xn_store.shape[0],), -1, device=self.device, dtype=torch.int32)
+                dense[:old].copy_(self._groups_store[:old])
+                self._group_keys_store, self._groups_store = keys, dense
+            self._group_keys_store[old:n].fill_(-1)
+            self._groups_store[old:n].fill_(-1)
+            self.groups = self._groups_store[:n]
         self._ws.clear()
         self._exact_ws = None
 
@@ -434,6 +448,59 @@ class FlatIPIndex:
             else:
                 self.labels.index_copy_(0, rows.to(self.device, torch.int64), w.to(self.device))
 
+    # -- groups --------------------------------------------------------------------------------
+    def set_groups(self, keys, rows=None) -> None:
+        """Sets the group key (a brand, a seller) of every row (`keys` [ntotal]), or of the listed `rows` only (`keys`
+        then has one value per listed row): int64 values, numpy or CUDA.  A negative key means ungrouped.  Keys may be
+        sparse (64-bit seller ids): the index renumbers the non-negative keys of all rows densely on every call.  A
+        search with `max_per_group=m` returns at most m rows of one group.  Rows added later are ungrouped.  Groups are
+        serving state: save / load do not store them."""
+        if self.ntotal == 0:
+            raise ValueError("empty index")
+        k = keys if isinstance(keys, torch.Tensor) else torch.from_numpy(np.asarray(keys))
+        if k.dtype not in (torch.int64, torch.int32, torch.int16, torch.int8, torch.uint8):
+            raise ValueError(f"group keys must be integers, got {k.dtype}")
+        if rows is None:
+            if tuple(k.shape) != (self.ntotal,):
+                raise ValueError(f"expected one group key per row ({self.ntotal}), got shape {tuple(k.shape)}")
+        else:
+            r = rows if isinstance(rows, torch.Tensor) else torch.from_numpy(np.asarray(rows))
+            if r.dim() != 1 or r.dtype not in (torch.int64, torch.int32) or tuple(k.shape) != (r.shape[0],):
+                raise ValueError(f"rows must be a 1-D integer array with one entry per group key, got rows "
+                                 f"{r.dtype} {tuple(r.shape)} and keys {tuple(k.shape)}")
+            if r.numel() and (int(r.min()) < 0 or int(r.max()) >= self.ntotal):
+                raise ValueError(f"rows must be in [0, {self.ntotal})")
+        k = k.to(self.device, torch.int64)
+        with torch.cuda.device(self.device):
+            if self._group_keys_store is None:
+                cap = self._xn_store.shape[0]
+                self._group_keys_store = torch.full((cap,), -1, device=self.device, dtype=torch.int64)
+                self._groups_store = torch.full((cap,), -1, device=self.device, dtype=torch.int32)
+            raw = self._group_keys_store[:self.ntotal]
+            if rows is None:
+                raw.copy_(k)
+            else:
+                raw.index_copy_(0, r.to(self.device, torch.int64), k)
+            grouped = raw >= 0
+            uniq, inv = torch.unique(raw[grouped], return_inverse=True)
+            dense = self._groups_store[:self.ntotal]
+            dense.fill_(-1)
+            dense[grouped] = inv.to(torch.int32)
+            self.groups = dense
+            self.n_groups = int(uniq.numel())
+
+    def _group_cap(self, max_per_group) -> Optional[int]:
+        """Validates a per-group cap -> the int, or None (no cap: the plain search runs)."""
+        if max_per_group is None:
+            return None
+        if isinstance(max_per_group, (bool, np.bool_)) or not isinstance(max_per_group, (int, np.integer)):
+            raise ValueError(f"max_per_group must be an int, got {type(max_per_group).__name__}")
+        if not 1 <= int(max_per_group) <= _native.TT_FLAT_MAX_PER_GROUP:
+            raise ValueError(f"max_per_group must be in [1, {_native.TT_FLAT_MAX_PER_GROUP}], got {max_per_group}")
+        if self.groups is None:
+            raise ValueError("a group cap needs group keys: call set_groups() first")
+        return int(max_per_group)
+
     def _requires(self, require, nq: int) -> Optional[torch.Tensor]:
         """Validates per-query label masks (CUDA or numpy [nq, 2] = {all, any}, or [2] for every query) -> int32 [nq, 2]
         on this device, or None when every query's masks are (0, 0): the unfiltered search runs."""
@@ -491,7 +558,20 @@ class FlatIPIndex:
             self._ws[key] = ws
         return ws
 
-    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
+    def _group_workspace(self, nq: int, k: int, n_excl: int) -> torch.Tensor:
+        key = (nq, k, "group", n_excl, self.n_groups)
+        ws = self._ws.get(key)
+        if ws is None:
+            nbytes = int(_native.load().tt_flat_search_grouped_workspace_bytes(self.ntotal, self.d, nq, k, n_excl,
+                                                                               self.n_groups))
+            ws = torch.empty(max(nbytes, 256), device=self.device, dtype=torch.uint8)
+            if len(self._ws) > 8:
+                self._ws.clear()
+            self._ws[key] = ws
+        return ws
+
+    def search_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None,
+                      max_per_group: Optional[int] = None):
         """Asynchronous search of CUDA f32 queries [nq,D] on the current stream.
 
         Returns (scores [nq,k] f32, ids [nq,k] i64, flags [nq] i32, n_uncertified [1] i32) device
@@ -501,6 +581,8 @@ class FlatIPIndex:
         not list in exclude[i]; with fewer than k allowed rows the tail is (-inf, -1).
         `require` (CUDA or numpy [nq, 2] = {all, any} u32 masks, or [2] for every query): only rows whose label word
         has every bit of `all` and, unless any == 0, one bit of `any` (see set_labels); composes with `exclude`.
+        `max_per_group` (int in [1, 64], needs set_groups): at most that many rows of one group, taken best first; the
+        rows a group cannot take make room for the next best rows (see tt_flat_search_grouped).
         """
         if self.ntotal == 0:
             raise ValueError("empty index")
@@ -509,6 +591,7 @@ class FlatIPIndex:
         if not 1 <= k <= min(self.ntotal, _native.TT_FLAT_MAX_K):
             raise ValueError(f"k must be in [1, min(ntotal, {_native.TT_FLAT_MAX_K})], got {k}")
         req = self._requires(require, q.shape[0])
+        cap = self._group_cap(max_per_group)
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
         excl = self._exclusions(exclude, nq)
@@ -518,7 +601,16 @@ class FlatIPIndex:
         nunc = torch.empty((1,), device=self.device, dtype=torch.int32)
         lib = _native.load()
         with torch.cuda.device(self.device):
-            if req is not None:
+            if cap is not None:
+                E = 0 if excl is None else excl.shape[1]
+                ws = self._group_workspace(max(nq, 1), k, E)
+                _native.check(lib.tt_flat_search_grouped(
+                    q.data_ptr(), nq, self.xn.data_ptr(), self.xh.data_ptr(), self.stats.data_ptr(), self.ntotal, self.d,
+                    k, self.id_offset, scores.data_ptr(), ids.data_ptr(), flags.data_ptr(), nunc.data_ptr(),
+                    self.groups.data_ptr(), self.n_groups, cap, 0 if req is None else self.labels.data_ptr(),
+                    0 if req is None else req.data_ptr(), 0 if excl is None else excl.data_ptr(), E, ws.data_ptr(),
+                    ws.numel(), ops._stream()), "tt_flat_search_grouped")
+            elif req is not None:
                 E = 0 if excl is None else excl.shape[1]
                 ws = self._workspace(max(nq, 1), k, E)
                 _native.check(lib.tt_flat_search_filtered(
@@ -543,10 +635,12 @@ class FlatIPIndex:
 
     def search_exact_device(self, q: torch.Tensor, k: int, scores: Optional[torch.Tensor] = None,
                             ids: Optional[torch.Tensor] = None, qsel: Optional[torch.Tensor] = None, *,
-                            exclude: Optional[torch.Tensor] = None, require=None):
+                            exclude: Optional[torch.Tensor] = None, require=None, max_per_group: Optional[int] = None):
         """Always-exact fp32 path; with `qsel` (i32 query rows) only those rows of scores/ids are rewritten.
-        `exclude` [nq, E] and `require` [nq, 2] are indexed by query row (qsel[i]), as in search_device."""
+        `exclude` [nq, E] and `require` [nq, 2] are indexed by query row (qsel[i]), as in search_device;
+        `max_per_group` as in search_device."""
         req = self._requires(require, q.shape[0])
+        cap = self._group_cap(max_per_group)
         q = ops._f32c(q, "queries")
         nq = q.shape[0]
         excl = self._exclusions(exclude, nq)
@@ -555,11 +649,20 @@ class FlatIPIndex:
             ids = torch.empty((nq, k), device=self.device, dtype=torch.int64)
         nsel = nq if qsel is None else int(qsel.numel())
         lib = _native.load()
-        need = int(lib.tt_flat_search_exact_workspace_bytes(self.ntotal, self.d, nsel, k))
+        need = int(lib.tt_flat_search_exact_workspace_bytes(self.ntotal, self.d, nsel, k) if cap is None else
+                   lib.tt_flat_search_exact_grouped_workspace_bytes(self.ntotal, self.d, nsel, k, self.n_groups))
         if self._exact_ws is None or self._exact_ws.numel() < need:
             self._exact_ws = torch.empty(need, device=self.device, dtype=torch.uint8)
         with torch.cuda.device(self.device):
-            if req is not None:
+            if cap is not None:
+                _native.check(lib.tt_flat_search_exact_grouped(
+                    q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
+                    self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(),
+                    0 if req is None else self.labels.data_ptr(), 0 if req is None else req.data_ptr(),
+                    0 if excl is None else excl.data_ptr(), 0 if excl is None else excl.shape[1],
+                    self.groups.data_ptr(), self.n_groups, cap, self._exact_ws.data_ptr(), self._exact_ws.numel(),
+                    ops._stream()), "tt_flat_search_exact_grouped")
+            elif req is not None:
                 _native.check(lib.tt_flat_search_exact_filtered(
                     q.data_ptr(), nq, 0 if qsel is None else qsel.data_ptr(), nsel, self.xn.data_ptr(), self.ntotal,
                     self.d, k, self.id_offset, scores.data_ptr(), ids.data_ptr(), self.labels.data_ptr(), req.data_ptr(),
@@ -649,14 +752,17 @@ class FlatIPIndex:
         return out
 
     def search_async(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None,
-                     require=None) -> PendingSearch:
+                     require=None, max_per_group: Optional[int] = None) -> PendingSearch:
         """Enqueues a search and returns at once; `.result()` checks the certificate later, so a caller can
         keep the next batch's kernels queued behind this one (no idle GPU between batches).  `exclude`, `require`:
         see search_device; uncertified queries are re-run exactly with the same lists and masks.  (Masks in a CUDA
-        tensor cost one device-to-host read to tell a filter from (0, 0); numpy masks cost none.)"""
+        tensor cost one device-to-host read to tell a filter from (0, 0); numpy masks cost none.)  `max_per_group`: see
+        search_device; the re-runs keep the cap."""
         kw = {} if exclude is None else {"exclude": exclude}
         if require is not None:
             kw["require"] = require
+        if max_per_group is not None:
+            kw["max_per_group"] = max_per_group
         scores, ids, flags, nunc = self.search_device(q, k, **kw)
         if self._ring is None:
             self._ring = _FlagRing()
@@ -670,9 +776,10 @@ class FlatIPIndex:
             return scores, ids, n_bad
         return PendingSearch(finish)
 
-    def search_checked_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None):
+    def search_checked_device(self, q: torch.Tensor, k: int, *, exclude: Optional[torch.Tensor] = None, require=None,
+                              max_per_group: Optional[int] = None):
         """search_device + re-run of uncertified queries through the exact path (one host sync)."""
-        return self.search_async(q, k, exclude=exclude, require=require).result()
+        return self.search_async(q, k, exclude=exclude, require=require, max_per_group=max_per_group).result()
 
     # -- range search (tt_flat_range_search) -----------------------------------------------------
     # Bytes of workspace one range call takes at most: the first pass sizes its candidate budget to fit, and the
@@ -971,28 +1078,33 @@ class FlatIPIndex:
                     ops._stream()), "tt_flat_shard_search_excl")
 
     def search_host_async(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None,
-                          require=None) -> PendingSearch:
+                          require=None, max_per_group: Optional[int] = None) -> PendingSearch:
         """Host-to-host search, asynchronous: stages q through pinned memory, enqueues H2D + search + D2H and
         returns; `.result()` -> (scores, ids, n_rerun) numpy arrays.  Up to 3 calls may be in flight.
-        `exclude`: numpy int64 [nq, E]; `require`: numpy [nq, 2] or [2] label masks (see search_device)."""
-        return host_search_async(self, self.search_async, self.device, self.d, q, k, exclude=exclude, require=require)
+        `exclude`: numpy int64 [nq, E]; `require`: numpy [nq, 2] or [2] label masks; `max_per_group`: group cap (see
+        search_device)."""
+        return host_search_async(self, self.search_async, self.device, self.d, q, k, exclude=exclude, require=require,
+                                 max_per_group=max_per_group)
 
     def search(self, q: np.ndarray, k: int, *, exclude: Optional[np.ndarray] = None,
-               require=None) -> Tuple[np.ndarray, np.ndarray]:
+               require=None, max_per_group: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
         """Host-to-host search, the shape of faiss `index.search(q, k)`: q f32 [nq,d] (un-normalised:
         the device op applies q/(||q||+1e-8)) -> (scores f32 [nq,k], ids i64 [nq,k]).  `exclude`: numpy int64
         [nq, E] ids to leave out per query (-1 = padding); `require`: label masks {all, any} per query ([nq, 2] or
-        [2]); short results end in (-inf, -1)."""
-        scores, ids, _ = self.search_host_async(q, k, exclude=exclude, require=require).result()
+        [2]); `max_per_group`: at most that many rows per group (see set_groups); short results end in (-inf, -1)."""
+        scores, ids, _ = self.search_host_async(q, k, exclude=exclude, require=require,
+                                                max_per_group=max_per_group).result()
         return scores, ids
 
 
 def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int, depth: int = 3, *,
-                      exclude: Optional[np.ndarray] = None, require=None) -> PendingSearch:
+                      exclude: Optional[np.ndarray] = None, require=None,
+                      max_per_group: Optional[int] = None) -> PendingSearch:
     """Shared host round trip of FlatIPIndex / ShardedFlatIPIndex: pinned staging buffers in a ring of `depth`
     sets per (nq, k) so that consecutive batches overlap their copies with the previous batch's kernels.
     `exclude` (numpy int64 [nq, E]) is copied to the device with the queries and passed on as `exclude=`; `require`
-    (label masks, FlatIPIndex only) is passed on as `require=`."""
+    (label masks, FlatIPIndex only) is passed on as `require=`, and `max_per_group` (FlatIPIndex only) as
+    `max_per_group=`."""
     q = np.ascontiguousarray(q, dtype=np.float32)
     if q.ndim != 2 or q.shape[1] != d:
         raise ValueError(f"expected queries [nq, {d}], got {q.shape}")
@@ -1028,6 +1140,8 @@ def host_search_async(owner, search_async, device, d: int, q: np.ndarray, k: int
         kw = {} if exclude is None else {"exclude": torch.from_numpy(exclude).to(device)}
         if require is not None:
             kw["require"] = require
+        if max_per_group is not None:
+            kw["max_per_group"] = max_per_group
         pending = search_async(dq, k, **kw)
 
     def finish():
@@ -1125,18 +1239,43 @@ class VectorDatabase:
             raise ValueError(f"{len(unknown)} unknown product ids, e.g. {unknown[:3]}")
         self.index.set_labels(labels, rows=np.array([self.id_to_index[p] for p in product_ids], np.int64))
 
+    def set_groups(self, groups, product_ids: Optional[List[str]] = None) -> None:
+        """Sets each product's group for `max_per_group` (a brand name, a seller id: any hashable value; None =
+        ungrouped): one per index row in index order, or one per listed product id.  Equal values are one group.  An
+        unknown product id raises ValueError and changes nothing.  Groups are serving state: save_index / load_index do
+        not store them."""
+        if self.index is None:
+            raise ValueError("Index not built. Call build_index() or load_index() first.")
+        groups = list(groups)
+        rows = None
+        if product_ids is not None:
+            product_ids = list(product_ids)
+            if len(product_ids) != len(groups):
+                raise ValueError(f"expected one group per product id ({len(product_ids)}), got {len(groups)}")
+            unknown = [p for p in product_ids if p not in self.id_to_index]
+            if unknown:
+                raise ValueError(f"{len(unknown)} unknown product ids, e.g. {unknown[:3]}")
+            rows = np.array([self.id_to_index[p] for p in product_ids], np.int64)
+        codes = self.__dict__.setdefault("_group_codes", {})
+        keys = np.array([-1 if g is None else codes.setdefault(g, len(codes)) for g in groups], np.int64)
+        self.index.set_groups(keys, rows=rows)
+
     # -- search --------------------------------------------------------------------------------
     def search_batch(self, query_embeddings: np.ndarray, k: int = 10, *,
-                     exclude_rows: Optional[np.ndarray] = None, require=None) -> Tuple[np.ndarray, np.ndarray]:
+                     exclude_rows: Optional[np.ndarray] = None, require=None,
+                     max_per_group: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
         """Array-returning retrieval: (scores f32 [nq,k'], row indices i64 [nq,k']) with k' = min(k, ntotal).
         `exclude_rows` int64 [nq, E] (-1 = padding): row indices query i must not return; `require` [nq, 2] or [2]:
-        {all, any} label masks (see FlatIPIndex.search_device); with fewer than k' allowed rows the tail is (-inf, -1)."""
+        {all, any} label masks (see FlatIPIndex.search_device); `max_per_group`: at most that many rows per group (see
+        set_groups); with fewer than k' rows to return the tail is (-inf, -1)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         k = min(k, self.index.ntotal)   # vector_db.py:159
         kw = {} if exclude_rows is None else {"exclude": exclude_rows}
         if require is not None:
             kw["require"] = require
+        if max_per_group is not None:
+            kw["max_per_group"] = max_per_group
         return self.index.search(np.asarray(query_embeddings), k, **kw)
 
     def _exclude_rows(self, lists, nq: int) -> Optional[np.ndarray]:
@@ -1152,11 +1291,13 @@ class VectorDatabase:
         return out
 
     def retrieve(self, query_embedding: np.ndarray, k: int = 10, *,
-                 exclude: Optional[List[str]] = None, require_all=0, require_any=0) -> List[Tuple[str, float]]:
+                 exclude: Optional[List[str]] = None, require_all=0, require_any=0,
+                 max_per_group: Optional[int] = None) -> List[Tuple[str, float]]:
         """vector_db.py:130-169 — descending score; only query row 0 is returned, as in the reference.
         `exclude`: product ids that must not be returned (e.g. the buyer's own history); unknown ids are ignored.
         `require_all` / `require_any`: label masks (scalars, or one per query row): only products whose label word has
-        every bit of require_all and, unless require_any is 0, one bit of require_any (see set_labels)."""
+        every bit of require_all and, unless require_any is 0, one bit of require_any (see set_labels).
+        `max_per_group`: at most that many products of one group (see set_groups)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         query_embedding = np.asarray(query_embedding)
@@ -1169,6 +1310,8 @@ class VectorDatabase:
             kw["require"] = req
         if exclude is not None:
             kw["exclude_rows"] = self._exclude_rows([exclude] * nq, nq)
+        if max_per_group is not None:
+            kw["max_per_group"] = max_per_group
         scores, indices = self.search_batch(query_embedding, k, **kw)
         results = []
         for idx, score in zip(indices[0], scores[0]):
@@ -1178,9 +1321,10 @@ class VectorDatabase:
 
     def retrieve_batch(self, query_embeddings: np.ndarray, k: int = 10, *,
                        exclude: Optional[List[List[str]]] = None, require_all=0,
-                       require_any=0) -> List[List[Tuple[str, float]]]:
+                       require_any=0, max_per_group: Optional[int] = None) -> List[List[Tuple[str, float]]]:
         """vector_db.py:171-209.  `exclude`: one list of product ids per query that it must not return.
-        `require_all` / `require_any`: label masks, scalars or one per query (see retrieve)."""
+        `require_all` / `require_any`: label masks, scalars or one per query (see retrieve); `max_per_group`: at most
+        that many products of one group per query (see set_groups)."""
         if self.index is None:
             raise ValueError("Index not built. Call build_index() or load_index() first.")
         nq = np.asarray(query_embeddings).shape[0]
@@ -1192,6 +1336,8 @@ class VectorDatabase:
             if len(exclude) != nq:
                 raise ValueError(f"exclude needs one list per query ({nq}), got {len(exclude)}")
             kw["exclude_rows"] = self._exclude_rows(exclude, nq)
+        if max_per_group is not None:
+            kw["max_per_group"] = max_per_group
         scores, indices = self.search_batch(query_embeddings, k, **kw)
         pids = self.product_ids
         n = len(pids)
